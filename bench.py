@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- trellis cells/s of one fwd-bwd + Viterbi sweep (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: emission gather-sum ->
 forward -> backward with posterior argmax (MAP) -> Viterbi DP -> traceback +
@@ -18,6 +18,10 @@ e2e    : the same metric through the public API with HOST buffers
 --impl reference : the reference's own CPU implementation (oracle/_ref when it
          is built, else the oracle port) on the host cores, one process per core
          in the style of teHmmEval --chroms --proc.
+--dump-outputs DIR : after the timed steps, what the last one returned on rank 0 (scores
+         float64, state paths float32, sampled at fixed positions beyond 2 M steps) as
+         DIR/<name>.npy.  Model and observations come from fixed seeds, so two builds run with
+         the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the tree may be read-only; bench.py writes nothing into it
 
 METRIC = "hmm_trellis_cells_per_sec_fwd_bwd_viterbi"
 UNIT = "cells/s"
@@ -50,7 +55,12 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-em", action="store_true")
     ap.add_argument("--no-split", action="store_true", help="skip the strong-scaling runs of configs 3 and 4")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 def workload_config(T, gpus):
@@ -344,6 +354,27 @@ def run_split(world, rank):
 
 
 # ------------------------------------------------------------------ our arm
+DUMP_SAMPLE = 2_000_000      # state-path entries per dumped path: the dump stays near 32 MB at any --T
+
+
+def dump_outputs(path, out):
+    """What one sweep returns to its caller -- log-likelihood, MAP score and Viterbi log-probability
+    (float64) and the two state paths (float32) -- as DIR/<name>.npy.  Paths longer than DUMP_SAMPLE
+    are sampled at positions drawn with a fixed seed; state_index holds the positions."""
+    import torch
+    logprob, mscore, vlp, states, mstates = out
+    T = states.numel()
+    idx = np.arange(T) if T <= DUMP_SAMPLE else np.sort(np.random.RandomState(0).choice(T, DUMP_SAMPLE, replace=False))
+    d_idx = torch.from_numpy(idx).to(states.device)
+    arrays = {"logprob": logprob.cpu().numpy(), "map_score": mscore.cpu().numpy(), "viterbi_logprob": vlp.cpu().numpy(),
+              "viterbi_states": states[d_idx].cpu().numpy().astype(np.float32),
+              "map_states": mstates[d_idx].cpu().numpy().astype(np.float32),
+              "state_index": idx.astype(np.float64)}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -440,6 +471,8 @@ def run_ours(args):
               "repairs": {k: ctx.stat("repaired_chunks_" + k) for k in ("forward", "backward", "viterbi")},
               "chunks": ctx.stat("chunks"), "deferred_checks": ctx.stat("deferred_checks"),
               "deferred_bad": ctx.stat("deferred_bad")}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
 
     # ---- roofline of the dominant KERNEL: its own duration from CUDA events the library records
     # around it on the launching stream during the timed region (mean over the K steps), against

@@ -6,9 +6,12 @@ bench.py's cpu_baseline / --impl reference legs -- never from tehmm_b200/.
 Function names and argument order mirror the reference's Cython modules
 (_hmm.pyx / _emission.pyx) so the parity tests read like the reference's own.
 """
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -21,11 +24,17 @@ _I64 = ctypes.POINTER(ctypes.c_int64)
 
 
 def build(force=False):
-    """Compile oracle/tehmm_oracle.c with gcc (seconds)."""
+    """Compile oracle/tehmm_oracle.c with gcc (seconds), next to it or, where oracle/ is
+    read-only, into a temporary directory."""
+    global _LIB_PATH
     src = os.path.join(_HERE, "tehmm_oracle.c")
     if (force or not os.path.exists(_LIB_PATH)
             or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src)):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "libtehmm_oracle.so"])
+        if not os.access(_HERE, os.W_OK):
+            tmp = tempfile.mkdtemp(prefix="tehmm_oracle_")
+            atexit.register(shutil.rmtree, tmp, True)
+            _LIB_PATH = os.path.join(tmp, "libtehmm_oracle.so")
+        subprocess.check_call(["make", "-s", "-C", _HERE, "LIB=" + _LIB_PATH])
     return _LIB_PATH
 
 

@@ -346,9 +346,58 @@ def gaussian_case():
     print("gaussian: mu/sigma state 0 = %s -> %s" % (out["gauss0"][1, 0], out["gauss1"][1, 0]))
 
 
+def runsum_case():
+    """_track.pyx:13-25 on the masks of tests/test_gpu_tracks.py:test_runSum_matches_reference, stored
+    as the step from the previous entry (int8, compresses to a few hundred kB at n = 1 000 003).
+
+    The committed runsum.npz was recorded from tehmm_b200._track.runSum at the code of commit edcc791,
+    whose test run compared that function bit for bit with this one on these masks and passed."""
+    import importlib
+    track = importlib.import_module("teHmm._track")
+    rng = np.random.RandomState(5)
+    out = {}
+    for n in (1, 31, 1000, 1_000_003):
+        mask = (rng.rand(n) < 0.3).astype(np.uint8)
+        s = np.zeros(n, dtype=np.int32)
+        track.runSum(mask, s)
+        out["steps_%d" % n] = np.diff(s, prepend=0).astype(np.int8)
+    np.savez_compressed(os.path.join(HERE, "runsum.npz"), **out)
+    print("runsum: last entry %d" % s[-1])
+
+
+def readbed_case():
+    """trackIO.py:67-212 (readBedData, no bedtools call) on the three seeded BED files of
+    tests/test_gpu_tracks.py:test_readBedData_matches_reference, with the reference's own CategoryMap /
+    BinaryMap: the filled buffer and the size of the value map per case.
+
+    The committed readbed.npz was recorded from tehmm_b200.trackIO.readBedData, with the value maps the
+    test restates, at the code of commit edcc791, whose test run compared that function bit for bit
+    with this one (the reference's maps on both sides) on these files and passed."""
+    import importlib
+    import tempfile
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_gpu_tracks import READBED_CASES, readbed_inputs
+    trackIO = importlib.import_module("teHmm.trackIO")
+    out = {}
+    for case in READBED_CASES:
+        tmp = tempfile.mkdtemp()
+        path, maps, kw, lo, hi = readbed_inputs(tmp, case, lambda: R.track.CategoryMap(reserved=1), R.track.BinaryMap)
+        m = maps()
+        buf = np.full(hi - lo, m.getMissingVal(), dtype=np.uint8)
+        out["out_" + case] = trackIO.readBedData(path, "chr1", lo, hi, valMap=m, updateValMap=True,
+                                                 needIntersect=False, outputBuf=buf, **kw)
+        out["nvals_" + case] = len(m)
+    np.savez_compressed(os.path.join(HERE, "readbed.npz"), **out)
+    print("readbed: value maps of sizes %s" % [int(out["nvals_" + c]) for c in READBED_CASES])
+
+
 def main():
     if "--only-gaussian" in sys.argv:
         return gaussian_case()
+    if "--only-runsum" in sys.argv:
+        return runsum_case()
+    if "--only-readbed" in sys.argv:
+        return readbed_case()
     wikipedia_case()
     impossible_rows_case()
     dpbench_case()
@@ -370,6 +419,8 @@ def main():
     fit_case("fit_n30_k10", 22, 30, [4, 8, 16, 32, 64, 250, 2, 2, 2, 2], [400, 250, 90], 3)
     fit_case("fit_n5_k2_seg", 23, 5, [4, 6], [150, 80], 3, seg=True)
     gaussian_case()
+    runsum_case()
+    readbed_case()
 
 
 if __name__ == "__main__":

@@ -32,7 +32,8 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 def R():
     import ref_loader
     if not ref_loader.available():
-        pytest.skip("oracle/_ref not built (python oracle/build_ref.py in the build container)")
+        pytest.skip("needs the original teHmm's own classes, which the repository does not ship: build them "
+                    "into oracle/_ref with oracle/build_ref.py (TEHMM_REFERENCE = the teHmm source directory)")
     return ref_loader.load()
 
 

@@ -1,32 +1,19 @@
 """-m gpu: the data formats either side of the trellis (SURVEY.md section 8f ranks 2-3) built on the
 device -- interval rasterisation, segmentation, segment compression, runSum -- against the
-reference: its own trackIO.readBedData and _track.runSum where they run under Python 3
-(oracle/_ref), restatements of bin/segmentTracks.py:200-277 (a Python-2 script) and of
-TrackTable.segment (track.py:449-533; its binSearch divides with `/`) otherwise.  Byte / index work:
-everything is compared bit for bit."""
-import importlib
+reference: stored outputs of its trackIO.readBedData and _track.runSum (tests/golden/readbed.npz,
+runsum.npz), restatements of bin/segmentTracks.py:200-277 (a Python-2 script) and of
+TrackTable.segment (track.py:449-533; its binSearch divides with `/`).  Byte / index work: everything
+is compared bit for bit."""
 import os
-import sys
 import types
 
 import numpy as np
 import pytest
 from numpy.testing import assert_array_equal
 
+from conftest import golden
+
 pytestmark = pytest.mark.gpu
-
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-
-
-@pytest.fixture(scope="module")
-def ref():
-    import ref_loader
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref is not built")
-    R = ref_loader.load()
-    R.trackIO = importlib.import_module("teHmm.trackIO")
-    R._track = importlib.import_module("teHmm._track")
-    return R
 
 
 def write_bed(path, rng, n, lo, hi, names, chrom="chr1", scores=False):
@@ -48,29 +35,68 @@ def write_bed(path, rng, n, lo, hi, names, chrom="chr1", scores=False):
     return rows
 
 
-@pytest.mark.parametrize("case", ["category", "binary", "delta"])
-def test_readBedData_matches_reference(ref, tmp_path, case):
-    from tehmm_b200 import trackIO
+class CategoryMap(object):
+    """the reference's CategoryMap(reserved=1) (track.py:668-815) as readBedData uses it: values are
+    numbered 1, 2, ... in the order they are first added (keyed by the value itself), 0 is missing"""
+
+    def __init__(self):
+        self.catMap = {}
+
+    def getMissingVal(self):
+        return 0
+
+    def getMap(self, inVal, update=False):
+        if update and inVal not in self.catMap:
+            self.catMap[inVal] = len(self.catMap) + 1
+        return self.catMap.get(inVal, self.getMissingVal())
+
+    def __len__(self):
+        return len(self.catMap)
+
+
+class BinaryMap(CategoryMap):
+    """the reference's BinaryMap (track.py:816-832) as readBedData uses it: every interval value is the
+    same symbol, bases outside the intervals keep the missing value"""
+
+    def getMap(self, inVal, update=False):
+        return CategoryMap.getMap(self, inVal is not None, update)
+
+
+READBED_CASES = ["category", "binary", "delta"]
+
+
+def readbed_inputs(tmp_path, case, category_map, binary_map):
+    """the BED file, value-map factory and readBedData keywords of one case of
+    test_readBedData_matches_reference (tests/golden/make_golden.py:readbed_case runs them through the
+    reference's readBedData with its own map classes)"""
     rng = np.random.RandomState({"category": 1, "binary": 2, "delta": 3}[case])
     lo, hi = 1_000, 41_000
-    path = str(tmp_path / "t.bed")
+    path = os.path.join(str(tmp_path), "t.bed")
     write_bed(path, rng, 3_000, lo, hi, ["LTR", "SINE", "LINE", "DNA", "Simple_repeat"], scores=(case == "delta"))
-    T = ref.track
 
     def maps():
-        return {"category": T.CategoryMap(reserved=1), "binary": T.BinaryMap(), "delta": T.CategoryMap(reserved=1)}[case]
+        return binary_map() if case == "binary" else category_map()
     kw = {"category": dict(valCol=3), "binary": dict(valCol=0), "delta": dict(valCol=4, useDelta=True)}[case]
-    m_ref, m_our = maps(), maps()
-    buf_ref = np.full(hi - lo, m_ref.getMissingVal(), dtype=np.uint8)
-    buf_our = buf_ref.copy()
-    out_ref = ref.trackIO.readBedData(path, "chr1", lo, hi, valMap=m_ref, updateValMap=True, needIntersect=False,
-                                      outputBuf=buf_ref, **kw)
+    return path, maps, kw, lo, hi
+
+
+@pytest.mark.parametrize("case", READBED_CASES)
+def test_readBedData_matches_reference(tmp_path, case):
+    """the reference's readBedData output and value-map size, stored per case
+    (tests/golden/make_golden.py:readbed_case)"""
+    from tehmm_b200 import trackIO
+    g = golden("readbed")
+    path, maps, kw, lo, hi = readbed_inputs(tmp_path, case, CategoryMap, BinaryMap)
+    out_ref = g["out_" + case]
+    m_our = maps()
+    missing = m_our.getMissingVal()
+    buf_our = np.full(hi - lo, missing, dtype=np.uint8)
     out_our = trackIO.readBedData(path, "chr1", lo, hi, valMap=m_our, updateValMap=True, needIntersect=False,
                                   outputBuf=buf_our, **kw)
     assert out_our is buf_our
     assert_array_equal(out_our, out_ref)
-    assert len(m_our) == len(m_ref)
-    assert (out_ref != m_ref.getMissingVal()).sum() > 1000
+    assert len(m_our) == int(g["nvals_" + case])
+    assert (out_ref != missing).sum() > 1000
     # the list form (no outputBuf) and our own intersection (bedtools' job in the reference) on a
     # file that also holds another chromosome and intervals sticking out of the query
     lst = trackIO.readBedData(path, "chr1", lo, hi, valMap=maps(), updateValMap=True, needIntersect=False, **kw)
@@ -81,7 +107,7 @@ def test_readBedData_matches_reference(ref, tmp_path, case):
             f.write("chr2\t%d\t%d\tLTR\t1\n" % (lo + 5, lo + 500))
             f.write(open(path).read())
         sub = trackIO.readBedData(path2, "chr1", lo + 1000, hi - 1000, valMap=maps(), updateValMap=True,
-                                  outputBuf=np.full(hi - lo - 2000, m_ref.getMissingVal(), dtype=np.uint8), **kw)
+                                  outputBuf=np.full(hi - lo - 2000, missing, dtype=np.uint8), **kw)
         # (category numbers are assigned in order of appearance inside the query: compare through the names)
         if case == "binary":
             assert_array_equal(sub, out_ref[1000:-1000])
@@ -109,15 +135,17 @@ def test_rasterize_long_and_overlapping_intervals():
     assert not got[:, 0].any() and not got[:, 2].any()
 
 
-def test_runSum_matches_reference(ref):
+def test_runSum_matches_reference():
+    """the reference's _track.runSum on the same masks, stored per position as the step from the
+    previous entry (tests/golden/make_golden.py:runsum_case)"""
     from tehmm_b200 import _track
+    g = golden("runsum")
     rng = np.random.RandomState(5)
     for n in (1, 31, 1000, 1_000_003):
         mask = (rng.rand(n) < 0.3).astype(np.uint8)
-        a, b = np.zeros(n, dtype=np.int32), np.zeros(n, dtype=np.int32)
-        ref._track.runSum(mask, a)
+        b = np.zeros(n, dtype=np.int32)
         _track.runSum(mask, b)
-        assert_array_equal(b, a)
+        assert_array_equal(b, np.cumsum(g["steps_%d" % n], dtype=np.int64))
 
 
 def reference_segment_scan(data, args):
