@@ -156,6 +156,24 @@ int tehmm_strict_update_counts(tehmm_ctx *ctx, const void *obs, int obs_bytes,
                                int64_t T, int K, int64_t start, int64_t end, int state,
                                double *stats /*K*N*S in-out*/, int N, int S,
                                const double *ratios);
+/* Supervised counts of every labelled interval in one device pass.  d_obs is a
+ * DEVICE (total, K) matrix in the layout of tehmm_set_batch's d_obs (the
+ * concatenated tables); no model or batch needs to be set.  Interval i covers
+ * the global rows [h_row_start[i], h_row_end[i]) with state h_state[i]; the
+ * weight of row r is d_ratios[r] (DEVICE, total entries) or 1.0 when d_ratios
+ * is NULL.  h_stats (HOST, K*N*S, in-out) ends bit for bit as after one
+ * tehmm_strict_update_counts per interval in the given order: every bin is
+ * init + w_1 + w_2 + ... in sequential float64 adds, interval order, positions
+ * ascending.  Intervals may overlap (counted again) and come in any order;
+ * empty ones are no-ops.  With unit weights and integer initial values the
+ * counts are integer histograms (order-free, exact); otherwise every bin is
+ * summed as one ordered chain.  The kernel launches do not depend on n.
+ * TEHMM_EINVAL, with h_stats untouched, for a row outside [0, total), a state
+ * outside [0, N), obs_bytes not 1, 2 or 4, or a counted symbol >= S.         */
+int tehmm_supervised_counts(tehmm_ctx *ctx, const void *d_obs, int obs_bytes, int64_t total, int K,
+                            int64_t n, const int64_t *h_row_start, const int64_t *h_row_end,
+                            const int32_t *h_state, const double *d_ratios /* total, or NULL */,
+                            double *h_stats /* K*N*S, in-out */, int N, int S);
 
 /* ----------------------------------------------------------------- L1 batched
  * Model: HOST pointers (small).  log_start (N), log_trans (N,N), table (K,N,S)

@@ -46,6 +46,7 @@ SIGNATURES = {
     "tehmm_strict_log_sum_lneta": (_c_int, [_c_void, _c_i64, _c_int, _c_void, _c_void, _c_void, _c_void, _c_dbl, _c_void, _c_void]),
     "tehmm_strict_accumulate_stats": (_c_int, [_c_void, _c_void, _c_int, _c_i64, _c_int, _c_void, _c_int, _c_int, _c_void, _c_void]),
     "tehmm_strict_update_counts": (_c_int, [_c_void, _c_void, _c_int, _c_i64, _c_int, _c_i64, _c_i64, _c_int, _c_void, _c_int, _c_int, _c_void]),
+    "tehmm_supervised_counts": (_c_int, [_c_void, _c_void, _c_int, _c_i64, _c_int, _c_i64, _c_void, _c_void, _c_void, _c_void, _c_void, _c_int, _c_int]),
     "tehmm_set_model": (_c_int, [_c_void, _c_int, _c_int, _c_int, _c_void, _c_void, _c_void, _c_dbl, _c_void]),
     "tehmm_set_batch": (_c_int, [_c_void, _c_void, _c_int, _c_i64, _c_void]),
     "tehmm_batch_total": (_c_i64, [_c_void]),

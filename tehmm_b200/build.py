@@ -15,11 +15,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libtehmm_b200.so")
-UNITS = ["api", "strict", "emission", "forward", "backward", "viterbi", "stats", "tile", "host", "umma", "fallback", "tracks", "ratios"]
+UNITS = ["api", "strict", "emission", "forward", "backward", "viterbi", "stats", "tile", "host", "umma", "fallback", "tracks", "ratios", "supervised"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",
           "-Xptxas", "-v"]
-EXTRA = {"strict": ["-fmad=false"]}
+EXTRA = {"strict": ["-fmad=false"], "supervised": ["-fmad=false"]}
 
 
 def _nvcc():

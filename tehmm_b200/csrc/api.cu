@@ -17,6 +17,8 @@ void tehmm_launch_strict_viterbi(cudaStream_t, int64_t, int, const double *, con
 void tehmm_launch_strict_lneta(cudaStream_t, int64_t, int, const double *, const double *, const double *, const double *, double, const double *, double *);
 void tehmm_launch_strict_accumulate(cudaStream_t, const void *, int, int64_t, int, double *, int, int, const double *, const double *);
 void tehmm_launch_strict_counts(cudaStream_t, const void *, int, int, int64_t, int64_t, int, double *, int, int, const double *);
+int tehmm_launch_sup_hist(cudaStream_t, const void *, int, int, int, int, int64_t, int64_t, const int64_t *, const int64_t *, const int64_t *, unsigned long long *, double *, int *);
+int tehmm_launch_sup_chain(cudaStream_t, const void *, int, int, int, int, const int64_t *, const int64_t *, const int64_t *, const int64_t *, const double *, double *, int *);
 size_t tehmm_emission_table_budget(int K);
 int tehmm_launch_emission(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const double *, void *, void *, double *, double *, int *, int, cudaError_t *, int64_t, int64_t);
 bool tehmm_emission_rows_ok(const TehmmModelDev &, int, const double *);
@@ -484,6 +486,75 @@ int tehmm_strict_update_counts(tehmm_ctx *c, const void *obs, int obs_bytes, int
     CU(cudaGetLastError());
     D2H(stats, dst_.p, sb);
     CU(cudaStreamSynchronize(st));
+    return TEHMM_OK;
+}
+
+int tehmm_supervised_counts(tehmm_ctx *c, const void *d_obs, int obs_bytes, int64_t total, int K, int64_t n,
+                            const int64_t *h_row_start, const int64_t *h_row_end, const int32_t *h_state,
+                            const double *d_ratios, double *h_stats, int N, int S)
+{
+    STRICT_PROLOGUE();
+    if (!d_obs || !h_stats || total < 0 || n < 0 || K <= 0 || N <= 0 || S <= 0) return fail(TEHMM_EINVAL, "bad argument");
+    if (n > 0 && (!h_row_start || !h_row_end || !h_state)) return fail(TEHMM_EINVAL, "NULL interval arrays");
+    if (check_obs_bytes(obs_bytes)) return TEHMM_EINVAL;
+    // group the non-empty intervals by state, interval order kept within a state (counting sort)
+    std::vector<int64_t> sbeg(N + 2, 0);
+    int64_t rows = 0;
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t a = h_row_start[i], b = h_row_end[i];
+        if (a < 0 || a > total || b > total)
+            return fail(TEHMM_EINVAL, "interval %lld: rows [%lld,%lld) outside [0,%lld)", (long long)i, (long long)a, (long long)b, (long long)total);
+        if (h_state[i] < 0 || h_state[i] >= N)
+            return fail(TEHMM_EINVAL, "interval %lld: state %d outside [0,%d)", (long long)i, h_state[i], N);
+        if (b > a) { sbeg[h_state[i] + 2] += 1; rows += b - a; }
+    }
+    if (rows == 0) return TEHMM_OK;
+    for (int s = 0; s < N; ++s) sbeg[s + 2] += sbeg[s + 1];
+    const int64_t m = sbeg[N + 1];
+    // blob: istart[m] | pfx[m + 1] | sbeg[N + 1] | sflat[N + 1]
+    std::vector<int64_t> blob(2 * m + 1 + 2 * (N + 1));
+    int64_t *istart = blob.data(), *pfx = istart + m, *hs = pfx + m + 1, *hf = hs + N + 1;
+    std::vector<int64_t> len(m);
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t a = h_row_start[i], b = h_row_end[i];
+        if (b <= a) continue;
+        const int64_t j = sbeg[h_state[i] + 1]++;
+        istart[j] = a;
+        len[j] = b - a;
+    }
+    pfx[0] = 0;
+    for (int64_t j = 0; j < m; ++j) pfx[j + 1] = pfx[j] + len[j];
+    for (int s = 0; s <= N; ++s) { hs[s] = sbeg[s]; hf[s] = pfx[sbeg[s]]; }
+    // integer regime: unit weights and initial values that stay exact integers after every count is added
+    const size_t bins = (size_t)K * N * S;
+    bool integral = d_ratios == nullptr;
+    for (size_t i = 0; integral && i < bins; ++i) {
+        const double v = h_stats[i];
+        integral = v == floor(v) && fabs(v) + (double)rows <= 9007199254740992.0;
+    }
+    DevBuf dblob, dstats, dcounts, dflag;
+    CU(dblob.alloc(blob.size() * 8)); CU(dstats.alloc(bins * 8)); CU(dflag.alloc(sizeof(int)));
+    H2D(dblob.p, blob.data(), blob.size() * 8);
+    H2D(dstats.p, h_stats, bins * 8);
+    CU(cudaMemsetAsync(dflag.p, 0, sizeof(int), st));
+    const int64_t *d_istart = dblob.as<int64_t>(), *d_pfx = d_istart + m, *d_sbeg = d_pfx + m + 1, *d_sflat = d_sbeg + N + 1;
+    if (integral) {
+        CU(dcounts.alloc(bins * 8));
+        CU(cudaMemsetAsync(dcounts.p, 0, bins * 8, st));
+        c->launches += tehmm_launch_sup_hist(st, d_obs, obs_bytes, K, N, S, m, rows, d_istart, d_pfx, d_sflat,
+                                             dcounts.as<unsigned long long>(), dstats.as<double>(), dflag.as<int>());
+    } else {
+        c->launches += tehmm_launch_sup_chain(st, d_obs, obs_bytes, K, N, S, d_istart, d_pfx, d_sbeg, d_sflat,
+                                              d_ratios, dstats.as<double>(), dflag.as<int>());
+    }
+    CU(cudaGetLastError());
+    int h_flag = 0;
+    std::vector<double> out(bins);
+    D2H(&h_flag, dflag.p, sizeof(int));
+    D2H(out.data(), dstats.p, bins * 8);
+    CU(cudaStreamSynchronize(st));
+    if (h_flag) return fail(TEHMM_EINVAL, "an observation in a counted row is >= S=%d (or negative)", S);
+    memcpy(h_stats, out.data(), bins * 8);
     return TEHMM_OK;
 }
 

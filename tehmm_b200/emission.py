@@ -12,7 +12,7 @@ import itertools
 import numpy as np
 from numpy.testing import assert_array_almost_equal
 
-from ._emission import canFast, fastAccumulateStats, fastAllLogProbs, fastUpdateCounts
+from ._emission import canFast, fastAccumulateStats, fastAllLogProbs
 from .common import EPSILON, NEGINF, assert_almost_equal_fast, logger, myLog, normalize
 from .track import is_track_table
 
@@ -195,29 +195,27 @@ class IndependentMultinomialEmissionModel(object):
     # ------------------------------------------------------------ supervised
     def supervisedTrain(self, trackData, bedIntervals):
         """Count emissions per labelled interval, then maximize (emission.py:293-331).
-        Both trackData and bedIntervals must be sorted."""
+        Both trackData and bedIntervals must be sorted.  The rows every interval counts are found
+        on the host (supervised.interval_triples: the reference's table scan, lastHit quirk
+        included), the tables they fall in go to the device once, and one
+        Engine.supervised_counts call counts them all, bit-identical to one fastUpdateCounts per
+        interval."""
+        from .engine import get_engine
+        from .supervised import interval_triples
         tables = trackData.getTrackTableList()
         assert len(tables) > 0
         assert len(bedIntervals) > 0
         obsStats = self.initStats()
-        lastTable, lastRatios = None, None
-        lastHit = 0
-        lastOverlapEnd = -1
-        for interval in bedIntervals:
-            hit = False
-            for tableIdx in range(lastHit, len(tables)):
-                table = tables[tableIdx]
-                overlap = table.getOverlapInTableCoords(interval, lastOverlapEnd)
-                if overlap is not None:
-                    lastHit = tableIdx
-                    hit = True
-                    lastOverlapEnd = max(0, overlap[2] - 1)
-                    if table is not lastTable:
-                        lastRatios = self.getSegmentRatios(table)
-                        lastTable = table
-                    fastUpdateCounts(overlap, table, obsStats, lastRatios)
-                elif hit is True:
-                    break
+        tix, lo, hi, state = interval_triples(tables, bedIntervals)
+        if len(tix) > 0:
+            # the per-interval path refuses these too (tehmm_strict_update_counts)
+            assert state.min() >= 0 and state.max() < self.numStates, "interval state outside [0, %d)" % self.numStates
+            used = np.unique(tix)
+            eng = get_engine()
+            offsets = eng.upload_batch([tables[t] for t in used])
+            d_ratios = eng.upload_ratios([self.getSegmentRatios(tables[t]) for t in used])
+            base = offsets[np.searchsorted(used, tix)]
+            eng.supervised_counts(base + lo, base + hi, state, obsStats, d_ratios)
         self.maximize(obsStats, trackData.getTrackList())
         self.validate()
 

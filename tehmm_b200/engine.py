@@ -214,6 +214,7 @@ class Engine(object):
                                             _lib.ptr(offsets)))
         self.total = int(offsets[-1])
         self.nseq = len(arrays)
+        self.obs_bytes = dt.itemsize
         self.h2d_bytes = host.nbytes
         return offsets
 
@@ -295,6 +296,7 @@ class Engine(object):
                                             _lib.ptr(offsets)))
         self.total = int(offsets[-1])
         self.nseq = len(offsets) - 1
+        self.obs_bytes = int(obs_bytes)
         return offsets
 
     def upload_ratios(self, ratios_list):
@@ -309,6 +311,45 @@ class Engine(object):
                 assert r.shape[0] == offsets[i + 1] - offsets[i]
                 host[offsets[i]:offsets[i + 1]] = r
         return self.torch.from_numpy(host).to(self.device)
+
+    def supervised_counts(self, row_start, row_end, state, obs_stats, d_ratios=None):
+        """Supervised emission counts of labelled intervals over the current batch (upload_batch or
+        use_device_batch) in one device pass (tehmm_supervised_counts).  Interval i covers the
+        batch's global rows [row_start[i], row_end[i]) with state[i]; d_ratios (device tensor or host
+        array of `total` weights, or None for 1.0) is the concatenation upload_ratios builds.
+        obs_stats (K, N, S) float64 is updated in place, bit-identical to one
+        _emission.fastUpdateCounts per interval in the given order.  Raises TehmmError, leaving
+        obs_stats as it was, for rows outside the batch, states outside [0, N) or a counted symbol >= S."""
+        torch = self.torch
+        d_obs = self._keep.get("obs")
+        if d_obs is None:
+            raise _lib.TehmmError("supervised_counts: no device batch (upload_batch or use_device_batch first)")
+        assert isinstance(obs_stats, np.ndarray) and obs_stats.dtype == np.float64 and obs_stats.ndim == 3
+        assert obs_stats.flags.c_contiguous, "obs_stats must be C-contiguous (it is updated in place)"
+        K, N, S = obs_stats.shape
+        rs = np.ascontiguousarray(row_start, dtype=np.int64).reshape(-1)
+        re = np.ascontiguousarray(row_end, dtype=np.int64).reshape(-1)
+        st64 = np.asarray(state, dtype=np.int64).reshape(-1)
+        assert rs.shape == re.shape == st64.shape, "row_start, row_end and state must have the same length"
+        if rs.size and (st64.min() < 0 or st64.max() >= N):
+            bad = int(np.flatnonzero((st64 < 0) | (st64 >= N))[0])
+            raise _lib.TehmmError("supervised_counts: interval %d has state %d outside [0, %d)" % (bad, int(st64[bad]), N))
+        st = np.ascontiguousarray(st64, dtype=np.int32)
+        nbytes = d_obs.numel() * d_obs.element_size()
+        if nbytes != self.total * K * self.obs_bytes:
+            raise _lib.TehmmError("supervised_counts: the batch is not a (%d, %d) matrix of %d-byte symbols"
+                                  % (self.total, K, self.obs_bytes))
+        if d_ratios is not None:
+            if not torch.is_tensor(d_ratios):
+                d_ratios = torch.from_numpy(_lib.f64(d_ratios)).to(self.device)
+            assert d_ratios.dtype == torch.float64 and d_ratios.numel() == self.total and d_ratios.is_contiguous()
+        self._bind_stream()
+        rc = self.lib.tehmm_supervised_counts(self.ctx.handle, self._p(d_obs), int(self.obs_bytes), int(self.total), K,
+                                              int(rs.size), _lib.ptr(rs), _lib.ptr(re), _lib.ptr(st), self._p(d_ratios),
+                                              _lib.ptr(obs_stats), N, S)
+        if rc != _lib.TEHMM_OK:
+            raise _lib.TehmmError("libtehmm_b200 error %d: %s" % (rc, self.lib.tehmm_last_error().decode("utf-8", "replace")))
+        return obs_stats
 
     def scratch(self, prec):
         n = int(self.lib.tehmm_scratch_bytes(self.ctx.handle, prec))

@@ -457,19 +457,36 @@ class MultitrackHmm(BaseHMM):
         N = self.emissionModel.getNumStates()
         transitionCount = self.fudge + np.zeros((N, N), np.float64)
         freqCount = self.fudge + np.zeros((N,), np.float64)
-        prev = None
-        for interval in bedIntervals:
-            state = int(interval[3])
-            assert state < N
-            transitionCount[state, state] += interval[2] - interval[1] - 1
-            freqCount[state] += interval[2] - interval[1]
-            if prev is not None and prev[0] == interval[0]:
-                if interval[1] < prev[2]:
-                    raise RuntimeError("Overlapping or out of order training intervals detected: "
-                                       "%s and %s." % (str(prev), str(interval)))
-                elif interval[1] == prev[2]:
-                    transitionCount[prev[3], state] += 1
-            prev = interval
+        # the reference's loop (hmm.py:174-210), vectorised: np.add.at applies the adds one by one in
+        # index order, so every float64 sum is taken in the loop's order
+        intervals = list(bedIntervals)
+        n = len(intervals)
+        if n > 0:
+            state = np.array([int(iv[3]) for iv in intervals], dtype=np.int64)
+            start = np.array([iv[1] for iv in intervals])
+            end = np.array([iv[2] for iv in intervals])
+            chrom = np.empty(n, dtype=object)
+            chrom[:] = [iv[0] for iv in intervals]
+            same = np.zeros(n, dtype=bool)
+            same[1:] = chrom[1:] == chrom[:-1]
+            overlap = np.zeros(n, dtype=bool)
+            overlap[1:] = same[1:] & (start[1:] < end[:-1])
+            bad_state = np.flatnonzero(~(state < N))
+            first_overlap = np.flatnonzero(overlap)
+            if len(first_overlap) and (len(bad_state) == 0 or first_overlap[0] < bad_state[0]):
+                i = int(first_overlap[0])
+                raise RuntimeError("Overlapping or out of order training intervals detected: "
+                                   "%s and %s." % (str(intervals[i - 1]), str(intervals[i])))
+            assert len(bad_state) == 0
+            # per interval: (state, state) += length - 1, then (previous state, state) += 1 when adjacent
+            adjacent = np.zeros(n, dtype=bool)
+            adjacent[1:] = same[1:] & (start[1:] == end[:-1])
+            rows = np.stack([state, np.roll(state, 1)], axis=1)
+            cols = np.stack([state, state], axis=1)
+            vals = np.stack([end - start - 1, np.ones(n, dtype=np.int64)], axis=1)
+            keep = np.stack([np.ones(n, dtype=bool), adjacent], axis=1)
+            np.add.at(transitionCount, (rows[keep], cols[keep]), vals[keep])
+            np.add.at(freqCount, state, end - start)
         for row in range(N):
             transitionCount[row] /= np.sum(transitionCount[row])
         self.transmat_ = np.copy(transitionCount)
