@@ -275,7 +275,7 @@ int tehmm_run_viterbi(tehmm_ctx *ctx, int prec, const void *d_elog, const double
  * the reference returns, _hmm.pyx:210), h_logprob float64[nseq] out (Viterbi:
  * path log-probability; MAP: forward log-likelihood), h_score float64[nseq] out
  * (MAP: sum of the posterior maxima, basehmm.py:357; may be NULL for Viterbi).
- * No segment ratios.  The library owns everything in between: a grow-only
+ * No segment ratios (tehmm_decode_host_ratios below takes them).  The library owns everything in between: a grow-only
  * device arena, pinned staging rings and a thread pool (TEHMM_HOST_THREADS,
  * default min(16, cores)) that stages pageable input and widens the uint8
  * states that crossed PCIe.  Blocks until the outputs are complete.          */
@@ -295,6 +295,23 @@ int tehmm_decode_host_both(tehmm_ctx *ctx, const void *const *h_obs_ptrs, int64_
                            int64_t nseq, const int64_t *h_offsets, int prec,
                            int64_t *h_viterbi_states, double *h_viterbi_logprob,
                            int64_t *h_map_states, double *h_map_score, double *h_forward_logprob);
+/* The same two calls for segmented tables (segmentTracks.py, teHmmEval.py --segment): h_ratio_ptrs =
+ * nseq host float64 arrays of T_i segment ratios (segment length / effective segment length, pageable
+ * or pinned), an entry NULL for a sequence without ratios (segRatios=None); h_ratio_ptrs NULL = no
+ * sequence has ratios.  As the reference's decode: the emission never sees the ratios (basehmm.py:327);
+ * the Viterbi DP, its traceback and the float64 log-probability of the path do (hmm.py:674), each
+ * sequence with its own -- a sequence without ratios gets the plain recursion, not the one at ratio 1
+ * (_hmm.pyx:234-237 treats from-state 0 differently whenever ratios are given); the MAP path and the
+ * forward log-likelihood ignore them (basehmm.py:261-264: not read).  The ratios travel through the
+ * same staging ring as the observations.  A ratio that is not finite and > 0 gives TEHMM_EINVAL before
+ * any output is written.  At most 64 states.                                                         */
+int tehmm_decode_host_ratios(tehmm_ctx *ctx, const void *const *h_obs_ptrs, int64_t nptr, int obs_bytes,
+                             int64_t nseq, const int64_t *h_offsets, const double *const *h_ratio_ptrs,
+                             int algorithm, int prec, int64_t *h_states, double *h_logprob, double *h_score);
+int tehmm_decode_host_both_ratios(tehmm_ctx *ctx, const void *const *h_obs_ptrs, int64_t nptr, int obs_bytes,
+                                  int64_t nseq, const int64_t *h_offsets, const double *const *h_ratio_ptrs,
+                                  int prec, int64_t *h_viterbi_states, double *h_viterbi_logprob,
+                                  int64_t *h_map_states, double *h_map_score, double *h_forward_logprob);
 /* bytes the last tehmm_decode_host moved over PCIe: which = 0 host->device, 1 device->host */
 int64_t tehmm_decode_host_bytes(tehmm_ctx *ctx, int which);
 /* wall-clock milliseconds of the phases of the last tehmm_decode_host call made with the

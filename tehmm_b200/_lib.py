@@ -77,6 +77,8 @@ SIGNATURES = {
     "tehmm_bed_close": (None, [_c_void]),
     "tehmm_decode_host": (_c_int, [_c_void, _c_void, _c_i64, _c_int, _c_i64, _c_void, _c_int, _c_int, _c_void, _c_void, _c_void]),
     "tehmm_decode_host_both": (_c_int, [_c_void, _c_void, _c_i64, _c_int, _c_i64, _c_void, _c_int, _c_void, _c_void, _c_void, _c_void, _c_void]),
+    "tehmm_decode_host_ratios": (_c_int, [_c_void, _c_void, _c_i64, _c_int, _c_i64, _c_void, _c_void, _c_int, _c_int, _c_void, _c_void, _c_void]),
+    "tehmm_decode_host_both_ratios": (_c_int, [_c_void, _c_void, _c_i64, _c_int, _c_i64, _c_void, _c_void, _c_int, _c_void, _c_void, _c_void, _c_void, _c_void]),
     "tehmm_decode_host_bytes": (_c_i64, [_c_void, _c_int]),
     "tehmm_host_pool_selftest": (_c_i64, [_c_int, _c_i64]),
     "tehmm_decode_host_phase_ms": (ctypes.c_double, [_c_void, _c_int]),

@@ -276,10 +276,15 @@ void tehmm_hostpipe_release(tehmm_ctx *c)
 extern "C" {
 
 // algorithm TEHMM_DECODE_BOTH: h_states = the Viterbi path, h_logprob = its log-probability, h_states_map = the
-// MAP path, h_score = its score, h_fwd_logprob = the forward log-likelihood
+// MAP path, h_score = its score, h_fwd_logprob = the forward log-likelihood.
+// h_ratio_ptrs (may be NULL): nseq host arrays of segment ratios, NULL for a sequence without them.  Only the
+// Viterbi DP, its traceback and re-score see them (hmm.py:674); the emission and the MAP path do not
+// (basehmm.py:261-264, 327).  On the device a sequence without ratios gets -1.0, which the Viterbi kernels
+// read as "no ratio terms" (csrc/viterbi.cu).
 static int decode_host_impl(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t nptr, int obs_bytes, int64_t nseq,
-                            const int64_t *h_offsets, int algorithm, int prec, int64_t *h_states,
-                            double *h_logprob, double *h_score, int64_t *h_states_map, double *h_fwd_logprob)
+                            const int64_t *h_offsets, const double *const *h_ratio_ptrs, int algorithm, int prec,
+                            int64_t *h_states, double *h_logprob, double *h_score, int64_t *h_states_map,
+                            double *h_fwd_logprob)
 {
     if (!c || !h_obs_ptrs || !h_offsets || !h_states || !h_logprob) return herr(TEHMM_EINVAL, "NULL argument");
     if (nptr != 1 && nptr != nseq) return herr(TEHMM_EINVAL, "nptr must be 1 (one contiguous matrix) or nseq (one matrix per sequence)");
@@ -300,12 +305,16 @@ static int decode_host_impl(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t
     Trace tr(st, p->phase_ms);
     const int64_t total = h_offsets[nseq];
     if (total <= 0) return herr(TEHMM_EINVAL, "empty batch");
+    // segment ratios are staged only when some sequence has them and a Viterbi path is wanted
+    bool use_ratios = false;
+    if (h_ratio_ptrs && algorithm != TEHMM_DECODE_MAP)
+        for (int64_t i = 0; i < nseq && !use_ratios; ++i) use_ratios = h_ratio_ptrs[i] && h_offsets[i + 1] > h_offsets[i];
     const int LD = tehmm_lattice_stride(c);
     const size_t ts = prec == TEHMM_F32 ? 4 : 8;
     const size_t obs_bytes_total = (size_t)total * K * obs_bytes;
     const size_t lat = (size_t)total * LD * ts;
 
-    // ---- arena layout: obs | states | logprob, score | rowmax | lattice A | lattice B | scratch
+    // ---- arena layout: obs | states | logprob, score | rowmax | lattice A | lattice B | [int64 states] | [ratios] | scratch
     size_t o = 0;
     const size_t o_obs = o; o = up256(o + obs_bytes_total);
     const size_t o_states = o; o = up256(o + (size_t)total);
@@ -331,6 +340,7 @@ static int decode_host_impl(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t
         if (pinned_out) gpu_widen = w != nullptr && !strcmp(w, "gpu");
     }
     const size_t o_s64 = o; if (gpu_widen) o = up256(o + (size_t)total * 8);
+    const size_t o_rat = o; if (use_ratios) o = up256(o + (size_t)total * 8);
     const size_t o_scratch = o;
     // the scratch size depends on the partition: describe the batch first, with the obs pointer
     // the arena will have (the arena may have to grow before anything is enqueued)
@@ -429,7 +439,73 @@ static int decode_host_impl(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t
         HCU(cudaStreamWaitEvent(st, p->slice_ev[slot], 0));
         if (piecewise) HOK(tehmm_run_emission_rows(c, prec, nullptr, em_log, em_lin, (double *)(A + o_rowmax), r0, r1, UINT64_MAX));
     }
-    p->h2d_bytes = (int64_t)obs_bytes_total;
+    // The segment ratios follow the observations through the same ring and copy stream (the Viterbi DP is the
+    // first stage that needs them): the worker threads gather each slice from the per-sequence arrays, fill -1.0
+    // for a sequence without ratios, and check every value on the way.
+    const double *d_rat = use_ratios ? (const double *)(A + o_rat) : nullptr;
+    if (use_ratios) {
+        const int64_t rat_rows = (int64_t)(SLICE / sizeof(double));
+        for (int64_t r0 = 0; r0 < total; r0 += rat_rows, ++slot) {
+            const int64_t r1 = std::min(total, r0 + rat_rows);
+            const int r = (int)(slot % NRING);
+            if (!p->ring[r]) {
+                HCU(cudaMallocHost((void **)&p->ring[r], SLICE));
+                HCU(cudaEventCreateWithFlags(&p->ring_ev[r], cudaEventDisableTiming));
+            }
+            if (p->ring_used[r]) HCU(cudaEventSynchronize(p->ring_ev[r]));
+            double *dst = (double *)p->ring[r];
+            const int64_t per = ((r1 - r0 + nth - 1) / nth + 7) & ~(int64_t)7;
+            std::atomic<int64_t> bad_row(INT64_MAX);
+            p->pool->parallel_for(nth, [&](int t) {
+                int64_t a = r0 + (int64_t)t * per;
+                const int64_t e = std::min(r1, a + per);
+                if (a >= e) return;
+                int64_t i = std::upper_bound(h_offsets, h_offsets + nseq + 1, a) - h_offsets - 1;
+                while (a < e) {
+                    while (h_offsets[i + 1] <= a) ++i;                 // (empty sequences)
+                    const int64_t n = std::min(e, h_offsets[i + 1]) - a;
+                    double *d = dst + (a - r0);
+                    const double *src = h_ratio_ptrs[i];
+                    if (!src) {
+                        std::fill(d, d + n, -1.0);
+                    } else {
+                        src += a - h_offsets[i];
+                        bool ok = true;
+                        for (int64_t k = 0; k < n; ++k) {
+                            const double v = src[k];
+                            ok &= v > 0.0 && v != INFINITY;            // NaN fails the first test
+                            d[k] = v;
+                        }
+                        if (!ok) {
+                            int64_t k = 0;
+                            while (src[k] > 0.0 && src[k] != INFINITY) ++k;
+                            int64_t cur = bad_row.load();
+                            while (a + k < cur && !bad_row.compare_exchange_weak(cur, a + k)) {}
+                        }
+                    }
+                    a += n;
+                }
+            });
+            if (bad_row.load() != INT64_MAX) {
+                const int64_t row = bad_row.load();
+                const int64_t i = std::upper_bound(h_offsets, h_offsets + nseq + 1, row) - h_offsets - 1;
+                return herr(TEHMM_EINVAL, "segment ratio %g of sequence %lld, step %lld: ratios must be finite and > 0",
+                            h_ratio_ptrs[i][row - h_offsets[i]], (long long)i, (long long)(row - h_offsets[i]));
+            }
+            HCU(cudaMemcpyAsync(A + o_rat + (size_t)r0 * 8, dst, (size_t)(r1 - r0) * 8, cudaMemcpyHostToDevice, p->copy_stream));
+            HCU(cudaEventRecord(p->ring_ev[r], p->copy_stream));
+            p->ring_used[r] = true;
+        }
+        // one event behind the last ratio slice (the ratio slices themselves record only their ring events)
+        while (p->slice_ev.size() <= (size_t)slot) {
+            cudaEvent_t ev;
+            HCU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+            p->slice_ev.push_back(ev);
+        }
+        HCU(cudaEventRecord(p->slice_ev[slot], p->copy_stream));
+        HCU(cudaStreamWaitEvent(st, p->slice_ev[slot], 0));
+    }
+    p->h2d_bytes = (int64_t)obs_bytes_total + (use_ratios ? total * 8 : 0);
     tr.mark("h2d+emission", true);
 
     // Two attempts at most.  The first runs the stages with deferred verification (option "defer":
@@ -453,7 +529,7 @@ static int decode_host_impl(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t
             HOK(tehmm_run_backward(c, prec, TEHMM_BWD_MAP | TEHMM_BWD_RENORM_EPS, A + o_lc, A + o_lb, nullptr, nullptr,
                                    d_states2, d_sc, nullptr, A + o_scratch));
         } else if (viterbi) {
-            HOK(tehmm_run_viterbi(c, prec, A + o_la, (const double *)(A + o_rowmax), nullptr, nullptr, A + o_lb, d_states, nullptr, d_lp, A + o_scratch));
+            HOK(tehmm_run_viterbi(c, prec, A + o_la, (const double *)(A + o_rowmax), nullptr, d_rat, A + o_lb, d_states, nullptr, d_lp, A + o_scratch));
         } else {
             HOK(tehmm_run_forward(c, prec, A + o_la, (double *)(A + o_rowmax), nullptr, A + o_lb, d_lp, A + o_scratch));
             HOK(tehmm_run_backward(c, prec, TEHMM_BWD_MAP | TEHMM_BWD_RENORM_EPS, A + o_la, A + o_lb, nullptr, nullptr,
@@ -530,7 +606,7 @@ static int decode_host_impl(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t
             HCU(cudaEventRecord(p->both_ev, st));
             HCU(cudaStreamWaitEvent(p->copy_stream, p->both_ev, 0));
             HOK(queue_copies(d_states2, 1, p->copy_stream));
-            HOK(tehmm_run_viterbi(c, prec, A + o_la, (const double *)(A + o_rowmax), nullptr, nullptr, A + o_lb, d_states, nullptr, d_lp, A + o_scratch));
+            HOK(tehmm_run_viterbi(c, prec, A + o_la, (const double *)(A + o_rowmax), nullptr, d_rat, A + o_lb, d_states, nullptr, d_lp, A + o_scratch));
             HCU(cudaMemcpyAsync(pin_lp, d_lp, (size_t)nseq * 32, cudaMemcpyDeviceToHost, st));
             HOK(queue_copies(d_states, 0, st));
             widen_slices(h_states_map, 1);
@@ -564,15 +640,32 @@ int tehmm_decode_host(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t nptr,
                       double *h_logprob, double *h_score)
 {
     if (algorithm == TEHMM_DECODE_BOTH) return herr(TEHMM_EINVAL, "TEHMM_DECODE_BOTH goes through tehmm_decode_host_both");
-    return decode_host_impl(c, h_obs_ptrs, nptr, obs_bytes, nseq, h_offsets, algorithm, prec, h_states, h_logprob, h_score, nullptr, nullptr);
+    return decode_host_impl(c, h_obs_ptrs, nptr, obs_bytes, nseq, h_offsets, nullptr, algorithm, prec, h_states, h_logprob, h_score, nullptr, nullptr);
+}
+
+int tehmm_decode_host_ratios(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t nptr, int obs_bytes, int64_t nseq,
+                             const int64_t *h_offsets, const double *const *h_ratio_ptrs, int algorithm, int prec,
+                             int64_t *h_states, double *h_logprob, double *h_score)
+{
+    if (algorithm == TEHMM_DECODE_BOTH) return herr(TEHMM_EINVAL, "TEHMM_DECODE_BOTH goes through tehmm_decode_host_both_ratios");
+    return decode_host_impl(c, h_obs_ptrs, nptr, obs_bytes, nseq, h_offsets, h_ratio_ptrs, algorithm, prec, h_states, h_logprob, h_score, nullptr, nullptr);
 }
 
 int tehmm_decode_host_both(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t nptr, int obs_bytes, int64_t nseq,
                            const int64_t *h_offsets, int prec, int64_t *h_viterbi_states, double *h_viterbi_logprob,
                            int64_t *h_map_states, double *h_map_score, double *h_forward_logprob)
 {
-    return decode_host_impl(c, h_obs_ptrs, nptr, obs_bytes, nseq, h_offsets, TEHMM_DECODE_BOTH, prec, h_viterbi_states,
+    return decode_host_impl(c, h_obs_ptrs, nptr, obs_bytes, nseq, h_offsets, nullptr, TEHMM_DECODE_BOTH, prec, h_viterbi_states,
                             h_viterbi_logprob, h_map_score, h_map_states, h_forward_logprob);
+}
+
+int tehmm_decode_host_both_ratios(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t nptr, int obs_bytes, int64_t nseq,
+                                  const int64_t *h_offsets, const double *const *h_ratio_ptrs, int prec,
+                                  int64_t *h_viterbi_states, double *h_viterbi_logprob, int64_t *h_map_states,
+                                  double *h_map_score, double *h_forward_logprob)
+{
+    return decode_host_impl(c, h_obs_ptrs, nptr, obs_bytes, nseq, h_offsets, h_ratio_ptrs, TEHMM_DECODE_BOTH, prec,
+                            h_viterbi_states, h_viterbi_logprob, h_map_score, h_map_states, h_forward_logprob);
 }
 
 

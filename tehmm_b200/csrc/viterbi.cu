@@ -25,6 +25,12 @@
 // The returned log-probability is a float64 re-score of the returned path
 // against the float64 tables, so it does not carry fp32 DP rounding.
 //
+// Segment ratios (RATIO kernels): a NEGATIVE ratio marks a step of a sequence
+// that has no ratios (segRatios=None).  Such a step gets the plain recursion:
+// the reference's from-state-0 term (_hmm.pyx:234-237) is applied only where
+// ratios are present, so it would be wrong to fill 1.0 for such a sequence in
+// a batch that mixes the two (tehmm_decode_host_ratios).  Real ratios are > 0.
+//
 // Algorithmic HBM bytes per step (fp32): DP 4N read (e) + 4N written (delta);
 // traceback 4N read + 1 written; re-score K + 1 read.
 #include "scan.cuh"
@@ -117,14 +123,15 @@ viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
                 // _hmm.pyx:234-237 vs 243-244: from-state 0 always gets A_jj*r (minus A_00
                 // when j==0); the other from-states get A_jj*(r-1), and only if r>1.
                 const T r = (T)rr[row];
+                const bool seg = r >= (T)0;        // negative: a sequence without ratios
                 const T x0 = ds[buf][0];
 #pragma unroll
                 for (int s = 0; s < NS; ++s) {
                     const T common = r > (T)1 ? dg[s] * (r - (T)1) : (T)0;
                     // (a zero-probability self transition would give inf-inf here; the
                     //  reference's finite -1e100 sentinel has no fp32 twin, see DESIGN.md)
-                    T extra0 = dg[s] > NEG ? dg[s] * r - common : (T)0;
-                    if (lane + 32 * s == 0 && a00 > NEG) extra0 -= a00;
+                    T extra0 = seg && dg[s] > NEG ? dg[s] * r - common : (T)0;
+                    if (seg && lane + 32 * s == 0 && a00 > NEG) extra0 -= a00;
                     T rest = NEG;      // max over from-states >= 1
                     T c0 = NEG;
 #pragma unroll
@@ -298,10 +305,11 @@ viterbi_lean_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
                 float f0 = lo2(c0), f1 = lo2(c1);          // candidates of from-state 16h
                 if (RATIO) {
                     // (a zero-probability self transition would give inf - inf in the reference's terms; guarded to 0
-                    //  like viterbi_kernel, DESIGN.md section 6)
-                    float x0 = dg0 > -INFINITY ? (r > 1.f ? dg0 : dg0 * r) : 0.f;
-                    float x1 = dg1 > -INFINITY ? (r > 1.f ? dg1 : dg1 * r) : 0.f;
-                    if (a2 == 0 && a00 > -INFINITY) x0 -= a00;
+                    //  like viterbi_kernel, DESIGN.md section 6; r < 0: a sequence without ratios, no correction)
+                    const bool seg = r >= 0.f;
+                    float x0 = seg && dg0 > -INFINITY ? (r > 1.f ? dg0 : dg0 * r) : 0.f;
+                    float x1 = seg && dg1 > -INFINITY ? (r > 1.f ? dg1 : dg1 * r) : 0.f;
+                    if (seg && a2 == 0 && a00 > -INFINITY) x0 -= a00;
                     if (h == 0) { f0 += x0; f1 += x1; }
                     if (r > 1.f) et += dgl * (r - 1.f);      // -inf for a state without self transition: it cannot hold a long segment
                 }
@@ -401,7 +409,7 @@ viterbi_lean_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
 }
 
 // ---------------------------------------------------------------------------
-// fp32 DP for 33..64 states (lattice rows of 64 floats, no segment ratios): TWO warps per chunk (round 2).
+// fp32 DP for 33..64 states (lattice rows of 64 floats): TWO warps per chunk (round 2).
 //
 // viterbi_kernel<float, 2> gives a lane two whole columns of log A: 128 registers, so one CTA of 8-12 warps per
 // SM whatever the launch bounds, 16 broadcast LDS.128 per step, and (ncu, profiles/r02_notes_wide.md) 46 % issue
@@ -414,14 +422,19 @@ viterbi_lean_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
 // is known to everybody behind the barrier, so the next step subtracts it (max_i(x_i - M + a) = max_i(x_i + a) - M)
 // and the owner stores delta_t = v_t - M_t one step late.  Same chunk protocol as viterbi_kernel (start_vec /
 // end_vec normalised, maximum 0).
+// RATIO: segment ratios as in viterbi_lean_kernel.  The common term [r_t > 1] logA_jj (r_t - 1) is folded into the
+// lane's e; the from-state-0 correction goes to the first candidate of the lanes of group h = 0, which hold
+// from-state 0 for their four to-states.
 #define VW_PAIRS 8
 #ifndef VW_ENABLED
 #define VW_ENABLED 1
 #endif
+template <bool RATIO>
 __global__ void __launch_bounds__(VW_PAIRS * 64, 1)
 viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ elog,
                     float *__restrict__ lattice, float *__restrict__ start_vec,
-                    float *__restrict__ end_vec, const int *__restrict__ bad, int mode)
+                    float *__restrict__ end_vec, const int *__restrict__ bad, int mode,
+                    const double *__restrict__ ratios)
 {
     __shared__ __align__(16) float ds_all[VW_PAIRS][2][72];      // 64 values, the two warps' maxima at [64], [65]
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, pair = warp >> 1, w = warp & 1;
@@ -445,6 +458,18 @@ viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
     const uint32_t BUF = 72u * 4u;
     const int bar_id = 1 + pair;
     const bool h0 = (h & 1) != 0, h1 = (h & 2) != 0;
+    // RATIO: diagonal of log A for this lane's state (common term) and, on the lanes of group h = 0, for its four
+    // to-states (from-0 correction x0_k = logA_kk min(r, 1) - [k = 0] logA_00, i.e. (r > 1 ? logA_kk : logA_kk r) as
+    // viterbi_lean_kernel writes it; 0 on the other lanes, and for a -inf diagonal, DESIGN.md section 6)
+    const float dgl = RATIO ? (float)m.cut_trans[(int64_t)j * 64 + j] : 0.f;
+    float dgk[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const int jk = 32 * w + a4 + k;
+        const float d = RATIO ? (float)m.cut_trans[(int64_t)jk * 64 + jk] : 0.f;
+        dgk[k] = h == 0 && d > -INFINITY ? d : 0.f;
+    }
+    const float a00 = RATIO && h == 0 && w == 0 && a4 == 0 && m.cut_trans[0] > -INFINITY ? (float)m.cut_trans[0] : 0.f;
 
     for (int64_t ci = (int64_t)blockIdx.x * VW_PAIRS + pair; ci < b.nchunks; ci += (int64_t)gridDim.x * VW_PAIRS) {
         if (mode == 1 && !bad[ci]) continue;                       // the same decision in both warps of the pair
@@ -457,6 +482,7 @@ viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
         }
         const float *ep = elog + tw * 64 + j;
         float *lp = lattice + tw * 64 + j;
+        const double *rp = RATIO ? ratios + tw : nullptr;             // advances with ep
         const int row0 = (int)(ch.t0 - tw), row1 = (int)(ch.t1 - tw);
         int row = 0, cur = 0;
         float vv;                                                  // this lane's published value of row - 1
@@ -475,7 +501,7 @@ viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
             return fmaxf(m0, m1);
         };
         // one step: row `row` from the row published in `cur`; stores the row before it if it is an output row
-        auto step = [&](float et) {
+        auto step = [&](float et, float r) {
             const uint32_t rd = ds_base + (uint32_t)cur * BUF + 16u * (uint32_t)h;
             u64 x[8];
 #pragma unroll
@@ -484,11 +510,20 @@ viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
             const float M = row_max(cur);
             if (row - 1 >= row0) lp[(int64_t)(row - 1) * 64] = fmaxf(vv - M, -INFINITY);      // all -inf: NaN -> -inf
             float p[4];
+            // r < 0: a sequence without ratios, no correction (min(max(r, 0), 1) = 0)
+            const float rc = RATIO ? __saturatef(r) : 0.f, a0 = RATIO && r >= 0.f ? a00 : 0.f;
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
                 const u64 c0 = fadd2(x[0], A2[k][0]);
-                p[k] = fmaxf(lo2(c0), hi2(c0));
+                float f = lo2(c0);                                 // from-state 4h: from-state 0 in group h = 0
+                if (RATIO) {
+                    float x0 = dgk[k] * rc;
+                    if (k == 0) x0 -= a0;
+                    f += x0;
+                }
+                p[k] = fmaxf(f, hi2(c0));
             }
+            if (RATIO && r > 1.f) et += dgl * (r - 1.f);           // -inf for a state without self transition
 #pragma unroll
             for (int q = 1; q < 8; ++q) {
 #pragma unroll
@@ -516,6 +551,11 @@ viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
             row = 0;
         } else if (from_start) {
             vv = ls + (own ? *ep : -INFINITY);                     // _hmm.pyx:214-220
+            if (RATIO) {                                           // _hmm.pyx:222-225
+                const float r0 = (float)rp[0];
+                if (r0 > 1.f) vv += dgl * (r0 - 1.f);
+                rp += 1;
+            }
             publish(vv, cur);
             ep += 64;
             row = 1;
@@ -526,31 +566,33 @@ viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
         }
         // (a virtual row -1 published by the first and the third branch is never stored: -1 < row0)
         if (mode == 0 && row0 > 0) {
-            while (row < row0) { step(*ep); ep += 64; }
+            while (row < row0) { step(*ep, RATIO ? (float)*rp : 1.f); ep += 64; if (RATIO) rp += 1; }
             const float M = row_max(cur);
             start_vec[ci * 64 + j] = fmaxf(vv - M, -INFINITY);
         }
-        float en[VIT_U];
+        float en[VIT_U], rn[VIT_U];
         if (row + VIT_U <= row1) {
 #pragma unroll
-            for (int u = 0; u < VIT_U; ++u) en[u] = ep[u * 64];
+            for (int u = 0; u < VIT_U; ++u) { en[u] = ep[u * 64]; rn[u] = RATIO ? (float)rp[u] : 1.f; }
         }
         while (row + 2 * VIT_U <= row1) {
-            float ec[VIT_U];
+            float ec[VIT_U], rc[VIT_U];
 #pragma unroll
-            for (int u = 0; u < VIT_U; ++u) ec[u] = en[u];
+            for (int u = 0; u < VIT_U; ++u) { ec[u] = en[u]; rc[u] = rn[u]; }
             ep += VIT_U * 64;
+            if (RATIO) rp += VIT_U;
 #pragma unroll
-            for (int u = 0; u < VIT_U; ++u) en[u] = ep[u * 64];
+            for (int u = 0; u < VIT_U; ++u) { en[u] = ep[u * 64]; rn[u] = RATIO ? (float)rp[u] : 1.f; }
 #pragma unroll
-            for (int u = 0; u < VIT_U; ++u) step(ec[u]);
+            for (int u = 0; u < VIT_U; ++u) step(ec[u], rc[u]);
         }
         if (row + VIT_U <= row1) {
 #pragma unroll
-            for (int u = 0; u < VIT_U; ++u) step(en[u]);
+            for (int u = 0; u < VIT_U; ++u) step(en[u], rn[u]);
             ep += VIT_U * 64;
+            if (RATIO) rp += VIT_U;
         }
-        while (row < row1) { step(*ep); ep += 64; }
+        while (row < row1) { step(*ep, RATIO ? (float)*rp : 1.f); ep += 64; if (RATIO) rp += 1; }
         {
             const float M = row_max(cur);
             const float dlast = fmaxf(vv - M, -INFINITY);
@@ -650,8 +692,8 @@ vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lat
             for (int s = 0; s < NS; ++s) cand[s] = dprev[s] + AT[st * NP + lane + 32 * s];
             if (RATIO) {
                 // only the from-state-0 candidate differs between from-states (see viterbi_kernel)
-                if (lane == 0) {
-                    const T r = (T)rr[row];
+                const T r = (T)rr[row];
+                if (lane == 0 && r >= (T)0) {           // negative: a sequence without ratios
                     const T dgs = AT[st * NP + st];
                     const T common = r > (T)1 ? dgs * (r - (T)1) : (T)0;
                     T extra0 = dgs > NEG ? dgs * r - common : (T)0;
@@ -847,9 +889,10 @@ vit_traceback4_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict_
                              : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w) : "r"(at_lane + (uint32_t)st * (uint32_t)(NP * 4)));
                 if (RATIO) {
                     // candidate of from-state 0 (lane u = 0, first element): + logA_ss r - [r > 1] logA_ss (r - 1), - logA_00 for s = 0
+                    // (r < 0: a sequence without ratios, no correction)
                     const float dgs = AT[st * NP + st];
-                    float extra0 = dgs > -INFINITY ? (r > 1.f ? dgs : dgs * r) : 0.f;
-                    if (st == 0 && a00 > -INFINITY) extra0 -= a00;
+                    float extra0 = r >= 0.f && dgs > -INFINITY ? (r > 1.f ? dgs : dgs * r) : 0.f;
+                    if (r >= 0.f && st == 0 && a00 > -INFINITY) extra0 -= a00;
                     if (u == 0) a.x += extra0;
                 }
                 const int sn = tb4_argmax<NS>(dv.x + a.x, dv.y + a.y, dv.z + a.z, dv.w + a.w, u, segshift, lane0);
@@ -920,7 +963,7 @@ __global__ void vit_rescore_kernel(TehmmModelDev m, TehmmBatchDev b, const OBS *
         } else {
             const int i = states[t - 1];
             term = m.log_trans[(int64_t)i * N + j] + e;
-            if (ratios_dp) {
+            if (ratios_dp && ratios_dp[t] >= 0.) {      // negative: a sequence without ratios
                 const double r = ratios_dp[t];
                 if (i == 0) {
                     term += ajj * r;
@@ -984,9 +1027,13 @@ cudaError_t tehmm_launch_viterbi(cudaStream_t st, const TehmmModelDev &m, const 
             return cudaGetLastError();
         }
         if (m.NS == 1) return launch_vit<float, 1>(st, m, b, (const float *)elog, ratios, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, grid);
-        if (m.LD == 64 && !ratios && VW_ENABLED) {
+        if (m.LD == 64 && VW_ENABLED) {
             const int64_t need = (b.nchunks + VW_PAIRS - 1) / VW_PAIRS;
-            viterbi_wide_kernel<<<(int)(need < grid ? need : grid), VW_PAIRS * 64, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode);
+            const int g = (int)(need < grid ? need : grid);
+            if (ratios)
+                viterbi_wide_kernel<true><<<g, VW_PAIRS * 64, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, ratios);
+            else
+                viterbi_wide_kernel<false><<<g, VW_PAIRS * 64, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, nullptr);
             return cudaGetLastError();
         }
         return launch_vit<float, 2>(st, m, b, (const float *)elog, ratios, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, grid);

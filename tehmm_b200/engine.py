@@ -218,14 +218,9 @@ class Engine(object):
         self.h2d_bytes = host.nbytes
         return offsets
 
-    def decode_host(self, obs_list, algorithm, precision=None):
-        """The whole decode call with host buffers on both sides, in the library
-        (tehmm_decode_host: pinned staging + worker threads in, uint8 states over PCIe and
-        widened to the reference's int64 out).  No segment ratios.
-        Returns (logprob float64[nseq], score float64[nseq] (MAP only), [int64 states])."""
-        self._bind_stream()
-        self.batch_token = None
-        prec, _ = self._prec(precision)
+    @staticmethod
+    def _host_arrays(obs_list):
+        """observation matrices of a host-buffer call: (arrays, dtype, offsets int64[nseq+1], void* table)"""
         arrays = [as_obs_array(o) for o in obs_list]
         assert len(arrays) > 0
         K = arrays[0].shape[1]
@@ -238,45 +233,79 @@ class Engine(object):
         offsets = np.zeros(len(arrays) + 1, dtype=np.int64)
         np.cumsum([a.shape[0] for a in arrays], out=offsets[1:])
         ptrs = (ctypes.c_void_p * len(arrays))(*[a.ctypes.data for a in arrays])   # no concatenation
+        return arrays, dt, offsets, ptrs
+
+    @staticmethod
+    def _host_ratios(ratios, offsets):
+        """per-sequence segment ratios -> (float64 arrays kept alive, double* table), or (None, None) when no
+        sequence has any; the library checks the values (finite, > 0)"""
+        if ratios is None or all(r is None for r in ratios):
+            return None, None
+        n = len(offsets) - 1
+        assert len(ratios) == n, "one entry of ratios per sequence"
+        keep = [None if r is None else np.ascontiguousarray(r, dtype=np.float64).reshape(-1) for r in ratios]
+        for i, r in enumerate(keep):
+            assert r is None or r.shape[0] == offsets[i + 1] - offsets[i], \
+                "sequence %d: %d segment ratios for %d observations" % (i, r.shape[0], offsets[i + 1] - offsets[i])
+        return keep, (ctypes.c_void_p * n)(*[None if r is None else r.ctypes.data for r in keep])
+
+    def decode_host(self, obs_list, algorithm, precision=None, ratios=None):
+        """The whole decode call with host buffers on both sides, in the library
+        (tehmm_decode_host: pinned staging + worker threads in, uint8 states over PCIe and
+        widened to the reference's int64 out).  ratios: None, or per sequence an array of
+        segment ratios or None (tehmm_decode_host_ratios); the Viterbi DP takes them, the
+        emission and MAP decoding do not, as in the reference's decode.
+        Returns (logprob float64[nseq], score float64[nseq] (MAP only), [int64 states])."""
+        self._bind_stream()
+        self.batch_token = None
+        prec, _ = self._prec(precision)
+        arrays, dt, offsets, ptrs = self._host_arrays(obs_list)
+        keep, rptrs = self._host_ratios(ratios, offsets)
+        n = len(arrays)
         total = int(offsets[-1])
         states = _result_pool.empty_int64(total)
-        logprob = np.empty(len(arrays), dtype=np.float64)
-        score = np.empty(len(arrays), dtype=np.float64)
-        _lib.check(self.lib.tehmm_decode_host(self.ctx.handle, ptrs, len(arrays), dt.itemsize, len(arrays),
-                                              _lib.ptr(offsets), int(algorithm), prec, _lib.ptr(states),
-                                              _lib.ptr(logprob), _lib.ptr(score)))
+        logprob = np.empty(n, dtype=np.float64)
+        score = np.empty(n, dtype=np.float64)
+        if rptrs is None:
+            _lib.check(self.lib.tehmm_decode_host(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets),
+                                                  int(algorithm), prec, _lib.ptr(states), _lib.ptr(logprob),
+                                                  _lib.ptr(score)))
+        else:
+            _lib.check(self.lib.tehmm_decode_host_ratios(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets),
+                                                         rptrs, int(algorithm), prec, _lib.ptr(states),
+                                                         _lib.ptr(logprob), _lib.ptr(score)))
+        del keep
         self._keep.pop("obs", None)            # the batch now points into the library's arena
         self._keep["offsets"] = offsets
-        self.total, self.nseq = total, len(arrays)
+        self.total, self.nseq = total, n
         self.h2d_bytes = int(self.lib.tehmm_decode_host_bytes(self.ctx.handle, 0))
         self.d2h_bytes = int(self.lib.tehmm_decode_host_bytes(self.ctx.handle, 1))
-        return logprob, score, [states[offsets[i]:offsets[i + 1]] for i in range(len(arrays))]
+        return logprob, score, [states[offsets[i]:offsets[i + 1]] for i in range(n)]
 
-    def decode_host_both(self, obs_list, precision=None):
+    def decode_host_both(self, obs_list, precision=None, ratios=None):
         """Viterbi AND posterior (MAP) decoding of the same observations in one call
-        (tehmm_decode_host_both): one upload, one emission pass.  Returns
+        (tehmm_decode_host_both): one upload, one emission pass.  ratios as for decode_host:
+        the Viterbi path takes them, the MAP path and the forward log-likelihood do not.  Returns
         (viterbi logprob[nseq], [viterbi states], map score[nseq], [map states], forward logprob[nseq])."""
         self._bind_stream()
         self.batch_token = None
         prec, _ = self._prec(precision)
-        arrays = [as_obs_array(o) for o in obs_list]
-        assert len(arrays) > 0
-        K = arrays[0].shape[1]
-        for a in arrays:
-            assert a.shape[1] == K, "all sequences must have the same number of tracks"
-        dt = arrays[0].dtype
-        if any(a.dtype != dt for a in arrays):
-            dt = np.dtype(np.int32)
-            arrays = [a.astype(np.int32) for a in arrays]
+        arrays, dt, offsets, ptrs = self._host_arrays(obs_list)
+        keep, rptrs = self._host_ratios(ratios, offsets)
         n = len(arrays)
-        offsets = np.zeros(n + 1, dtype=np.int64)
-        np.cumsum([a.shape[0] for a in arrays], out=offsets[1:])
-        ptrs = (ctypes.c_void_p * n)(*[a.ctypes.data for a in arrays])
         total = int(offsets[-1])
         vst, mst = _result_pool.empty_int64(total), _result_pool.empty_int64(total)
         vlp, msc, flp = (np.empty(n, dtype=np.float64) for _ in range(3))
-        _lib.check(self.lib.tehmm_decode_host_both(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets), prec,
-                                                   _lib.ptr(vst), _lib.ptr(vlp), _lib.ptr(mst), _lib.ptr(msc), _lib.ptr(flp)))
+        if rptrs is None:
+            _lib.check(self.lib.tehmm_decode_host_both(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets), prec,
+                                                       _lib.ptr(vst), _lib.ptr(vlp), _lib.ptr(mst), _lib.ptr(msc),
+                                                       _lib.ptr(flp)))
+        else:
+            _lib.check(self.lib.tehmm_decode_host_both_ratios(self.ctx.handle, ptrs, n, dt.itemsize, n,
+                                                              _lib.ptr(offsets), rptrs, prec, _lib.ptr(vst),
+                                                              _lib.ptr(vlp), _lib.ptr(mst), _lib.ptr(msc),
+                                                              _lib.ptr(flp)))
+        del keep
         self._keep.pop("obs", None)
         self._keep["offsets"] = offsets
         self.total, self.nseq = total, n
@@ -300,7 +329,12 @@ class Engine(object):
         return offsets
 
     def upload_ratios(self, ratios_list):
-        """list of per-sequence float64 arrays (or None) -> device tensor or None."""
+        """list of per-sequence float64 arrays (or None) -> device tensor or None.
+        A sequence without ratios gets 1.0: right for the forward / backward passes and the E-step,
+        where the ratio terms vanish at 1.0, but not for the Viterbi DP of a batch that mixes
+        sequences with and without ratios (the reference's from-state-0 term applies whenever
+        ratios are given, _hmm.pyx:234-237).  Engine.viterbi keeps this; decode_host(ratios=...)
+        decodes such batches as the reference does."""
         if ratios_list is None or all(r is None for r in ratios_list):
             return None
         offsets = self._keep["offsets"]

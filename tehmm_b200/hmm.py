@@ -320,39 +320,26 @@ class MultitrackHmm(BaseHMM):
         if self._wide():
             return [self._wide_decode(o, algorithm) for o in obs_list]
         eng = self._engine()
-        ratios_dp = [self._seg_ratios(o) for o in obs_list] if algorithm == "viterbi" else None
-        if algorithm in ("viterbi", "map") and (ratios_dp is None or all(r is None for r in ratios_dp)):
-            # host buffers in and out, everything in between inside the library
-            lps, scores, states = eng.decode_host(
-                obs_list, _lib.DECODE_VITERBI if algorithm == "viterbi" else _lib.DECODE_MAP)
-            if algorithm == "viterbi":
-                return [(float(lp), st) for lp, st in zip(lps, states)]
-            for lp in lps:
-                self._note_forward_logprob(float(lp))
-            return [(float(sc), st) for sc, st in zip(scores, states)]
-        eng.upload_batch(obs_list)
+        # host buffers in and out, everything in between inside the library
         if algorithm == "viterbi":
             # basehmm.py:327: emission from np.asarray(obs) (no ratios);
             # hmm.py:674: the DP does see the table's segment ratios
-            lps, states = eng.viterbi(ratios_em=None, ratios_dp=ratios_dp)
+            lps, _, states = eng.decode_host(obs_list, _lib.DECODE_VITERBI,
+                                             ratios=[self._seg_ratios(o) for o in obs_list])
             return [(float(lp), st) for lp, st in zip(lps, states)]
-        out = eng.posteriors(renorm_eps=True, want_post=False, want_map=True)
-        res = []
-        for lp, sc, st in zip(out["logprob"], out["map_score"], out["map_states"]):
+        lps, scores, states = eng.decode_host(obs_list, _lib.DECODE_MAP)
+        for lp in lps:
             self._note_forward_logprob(float(lp))
-            res.append((float(sc), st))
-        return res
+        return [(float(sc), st) for sc, st in zip(scores, states)]
 
     def decode_both_batch(self, obs_list):
         """Viterbi path AND posterior (MAP) decoding of every sequence in ONE pass over the data: what
         decode_batch(obs, "viterbi") followed by decode_batch(obs, "map") return (bit-identical), as
         [(viterbi logprob, viterbi states, map score, map states)], for the price of one upload and one
         emission pass (teHmmEval.py asks for both of the same tracks, teHmmEval.py:127-160; the
-        reference computes its frame once per call).  Sequences with segment ratios, and models of
-        more than 64 states, take the two calls."""
-        wide = self._wide()
-        ratios = None if wide else [self._seg_ratios(o) for o in obs_list]
-        if wide or any(r is not None for r in ratios):
+        reference computes its frame once per call).  Segment ratios go to the Viterbi path only, as
+        in decode_batch.  Models of more than 64 states take the two calls."""
+        if self._wide():
             saved = self._algorithm
             try:
                 self._algorithm = "viterbi"
@@ -362,7 +349,8 @@ class MultitrackHmm(BaseHMM):
             finally:
                 self._algorithm = saved
             return [(a[0], a[1], b[0], b[1]) for a, b in zip(v, m)]
-        vlp, vst, msc, mst, flp = self._engine().decode_host_both(obs_list)
+        vlp, vst, msc, mst, flp = self._engine().decode_host_both(obs_list,
+                                                                  ratios=[self._seg_ratios(o) for o in obs_list])
         for lp in flp:
             self._note_forward_logprob(float(lp))
         return [(float(a), s, float(b), t) for a, s, b, t in zip(vlp, vst, msc, mst)]
