@@ -92,20 +92,14 @@ uint64_t tehmm_ctx_stream(tehmm_ctx *ctx);
 int64_t tehmm_ctx_launch_count(tehmm_ctx *ctx);
 /* options: "chunk_tiles" (tiles of 64 steps per chunk, 0 = auto),
  * "warmup" (speculative warm-up steps, 0 = auto), "max_repair" (passes),
- * "tile" (0 = never use the tensor-core tile kernels), "fine_len" (steps per
- * chunk of the fine partition, 0 = auto), "umma" (1 / 2 = forward pass of a
- * single-sequence batch of <= 32 states by the tcgen05 / tensor-memory kernel of
- * csrc/umma.cu with one / two threads per chunk; same results, 0.84 / 0.80 ms per
- * 10 M steps against 0.54 ms for the mma.sync kernel there),
- * "umma64" (default 1: the same kernel, 64 columns, and its backward twin ARE the
- * forward and the backward / posterior / MAP pass of single-sequence batches of
- * 33..64 states; 0 = one chunk per warp; stat "umma_passes" counts the launches
- * of any of them), "xi_tile" (0 = expected transition
- * counts by the one-chunk-per-warp backward kernel instead of the tensor-core
- * xi kernel), "timing" (1 = bracket the first
+ * "tile" (0 = CUDA-core kernels only: by default fp32 passes without segment ratios take
+ * the tensor-core kernels -- the mma.sync tile kernels and the xi kernel of the expected
+ * transition counts at <= 32 states, the tcgen05 / tensor-memory forward and backward /
+ * posterior / MAP kernels of csrc/umma.cu for the first pass over a single-sequence batch
+ * of 33..64 states; stats "tile_passes" and "umma_passes" count their launches),
+ * "fine_len" (steps per chunk of the fine partition, 0 = auto), "timing" (1 = bracket the first
  * launch of each main kernel with CUDA events on the context's stream), "defer" (see
- * tehmm_ctx_check), "bwd_tmap" (1 = the regular tiles of a single-sequence batch take the
- * tensor-map block kernel in the backward pass; experimental: bit-identical results, not faster),
+ * tehmm_ctx_check),
  * "fallback_after" (ordinary repair passes before the chunks still flagged are resolved exactly by
  * transfer operators and a float64 chain, csrc/fallback.cu; default 2, -1 = never: the plain loop, one
  * pass per link of a chain of failed boundaries; stats "fallbacks", "fallback_chunks", "mix_rho_ppm").

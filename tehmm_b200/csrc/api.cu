@@ -38,14 +38,14 @@ cudaError_t tehmm_launch_emission_stats(cudaStream_t, const TehmmModelDev &, con
 size_t tehmm_stats_smem_bytes(int tab_rows, int N, int K, int prec);
 cudaError_t tehmm_launch_widen(cudaStream_t, const uint8_t *, int64_t *, int64_t);
 cudaError_t tehmm_launch_forward_tile(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, const float *, const double *, float *, float *, float *, double *, const int *, int, int, int64_t);
-cudaError_t tehmm_launch_backward_tile(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const float *, const float *, float *, uint8_t *, double *, float *, float *, const int *, int, int, int64_t, int);
+cudaError_t tehmm_launch_backward_tile(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const float *, const float *, float *, uint8_t *, double *, float *, float *, const int *, int, int);
 int tehmm_tile_warps(void);
 bool tehmm_forward_umma_ok(const TehmmModelDev &, const TehmmBatchDev &, int, int64_t);
-cudaError_t tehmm_launch_forward_umma(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, const float *, const double *, float *, float *, float *, double *, int, int64_t, int *, int);
+cudaError_t tehmm_launch_forward_umma(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, const float *, const double *, float *, float *, float *, double *, int, int64_t, int *);
 bool tehmm_backward_umma_ok(const TehmmModelDev &, const TehmmBatchDev &, int, int, int64_t);
 cudaError_t tehmm_launch_backward_umma(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const float *, const float *, float *, uint8_t *, double *, float *, float *, int, int64_t, int *);
-cudaError_t tehmm_launch_xi_tile(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, const float *, const float *, double *, float *, double *, int);
-size_t tehmm_xi_tile_scratch_bytes(int sms);
+cudaError_t tehmm_launch_xi_mma(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, const float *, const float *, double *, float *, double *, int);
+size_t tehmm_xi_mma_scratch_bytes(int sms);
 cudaError_t tehmm_launch_convert(cudaStream_t, int, const void *, double *, int64_t);
 cudaError_t tehmm_launch_transfer_ops(cudaStream_t, const TehmmModelDev &, const TehmmChunk *, const int64_t *, int64_t, int, int, const void *, void *, double *, int);
 cudaError_t tehmm_launch_ratio_fold(cudaStream_t, const TehmmModelDev &, int64_t, int, const double *, void *, double *, int);
@@ -94,17 +94,13 @@ struct tehmm_ctx {
     cudaStream_t own_stream = nullptr;
     int64_t launches = 0;
     int64_t opt_chunk_tiles = 0, opt_warmup = 0, opt_max_repair = 0;
-    int64_t opt_tile = 1, opt_fine_len = 0;   // tensor-core tile kernels on / fine chunk length (0 = auto)
+    int64_t opt_tile = 1, opt_fine_len = 0;   // tensor-core kernels (tile.cu, umma.cu) on / fine chunk length (0 = auto)
     // option "timing": CUDA events around the first (speculative) launch of each main kernel, on the
     // launching stream; read back in microseconds with tehmm_ctx_get_stat("us_<kernel>")
     int64_t opt_timing = 0;
-    int64_t opt_umma = 0;             // 1: forward pass on tcgen05 / TMEM (umma.cu) for <= 32 states too -- correct, not faster there
-    int64_t opt_umma64 = 1;           // 33..64 states, one sequence: forward pass on tcgen05 / TMEM (default; 0 = one chunk per warp)
     int *d_fault = nullptr;           // raised by a kernel whose barrier protocol timed out
     int64_t stat_umma_passes = 0;
     int64_t opt_rescore = 0;          // 1: the Viterbi log-probability is always the float64 re-score of the returned path (default: the fp32 DP's own normaliser sum where the lean kernel runs)
-    int64_t opt_bwd_tmap = 0;         // 1: backward pass of the regular tiles by bwd_tile_tmap_kernel (tensor-map blocks) -- correct, not faster (profiles/r01_notes_v4.md)
-    int64_t opt_xi_tile = 1;          // expected transition counts by xi_tile_kernel (0: one-chunk-per-warp backward)
     // ordinary repair passes before the chunks still flagged are resolved exactly by transfer operators
     // (fallback.cu; -1 = never: the plain loop, one pass per link of a chain of bad chunks)
     int64_t opt_fallback_after = 2;
@@ -231,11 +227,7 @@ int tehmm_ctx_set_option(tehmm_ctx *c, const char *name, int64_t v)
     else if (!strcmp(name, "tile")) c->opt_tile = v;
     else if (!strcmp(name, "timing")) { c->opt_timing = v; for (int i = 0; i < TEHMM_NTIMED; ++i) c->ev_n[i] = 0; }
     else if (!strcmp(name, "fine_len")) c->opt_fine_len = v;
-    else if (!strcmp(name, "umma")) c->opt_umma = v;
-    else if (!strcmp(name, "umma64")) c->opt_umma64 = v;
-    else if (!strcmp(name, "xi_tile")) c->opt_xi_tile = v;
     else if (!strcmp(name, "defer")) c->opt_defer = v;
-    else if (!strcmp(name, "bwd_tmap")) c->opt_bwd_tmap = v;
     else if (!strcmp(name, "rescore")) c->opt_rescore = v;
     else if (!strcmp(name, "fallback_after")) c->opt_fallback_after = v;
     else return fail(TEHMM_EINVAL, "unknown option %s", name);
@@ -886,7 +878,7 @@ static Scratch carve(const tehmm_ctx *c, int prec)
     s.part_a = o; o = align_up(o + nb * 8);
     s.bad = o; o = align_up(o + nb * 4);
     s.nbad = o; o = align_up(o + 4);
-    s.xi = o; o = align_up(o + std::max(nc * NP * NP * ts, tehmm_xi_tile_scratch_bytes(c->sms)));
+    s.xi = o; o = align_up(o + std::max(nc * NP * NP * ts, tehmm_xi_mma_scratch_bytes(c->sms)));
     s.xdiag = o; o = align_up(o + nc * NP * ts);
     s.gamma0 = o; o = align_up(o + (size_t)c->b.nseq * NP * ts);
     s.tilemap = o; o = align_up(o + (size_t)c->b.ntiles * NP);
@@ -1211,11 +1203,69 @@ static double tolerance_after_fallback(const tehmm_ctx *c, int prec, bool log_sp
 }
 #define TEHMM_MAX_FALLBACK_ROUNDS 10    // reach 8 * 4^round chunks: far beyond any partition; then the plain loop
 
-// The tensor-core tile kernels (tile.cu) take the fp32, N <= 32, no
-// segment-ratio case; everything else runs one chunk per warp.
+// The speculate / verify / repair loop of the forward (kind 0), backward (1) and Viterbi DP (2) passes over the
+// chunks of partition PB: the first pass (timed), then verify -> repair until every chunk boundary stands.
+// launch(mode) runs the pass (mode 0: every chunk, speculated starts; mode 1: the flagged chunks from start_vec).
+// kind, lat and the exact fallback are resolve_flagged's (linear space for 0 / 1, log space for 2); lkap: the
+// forward pass's per-chunk log factors (verify_kernel).  The fallback needs a chain without segment ratios.
+// umma_used (forward / backward): raised by launch when the tcgen05 kernel took the first pass -- its fault flag
+// is checked after that pass and its verification count is never deferred.
+}   // extern "C" (a template below)
+template <typename Launch>
+static int repair_loop(tehmm_ctx *c, cudaStream_t st, const TehmmBatchDev &PB, int prec, int kind, const void *lat,
+                       void *sv, void *ev, int *bad, int *nbad, double *lkap, bool fallback_ok,
+                       const bool *umma_used, Launch launch)
+{
+    static const int timer[3] = {TK_FORWARD, TK_BACKWARD, TK_VITERBI_DP};
+    static const char *const what[3] = {"forward", "backward", "viterbi"};
+    static const char *const umma_kernel[3] = {"fwd_umma_kernel", "bwd_umma_kernel", ""};
+    int64_t *const stat_repair[3] = {&c->stat_repair_fwd, &c->stat_repair_bwd, &c->stat_repair_vit};
+    int64_t *const stat_bad[3] = {&c->stat_bad_fwd, &c->stat_bad_bwd, &c->stat_bad_vit};
+    const bool log_space = kind == 2;
+    tk_begin(c, timer[kind]);
+    CU(launch(0));
+    tk_end(c, timer[kind]);
+    c->launches += 1;
+    const bool umma = umma_used && *umma_used;
+    double tol = tolerance(prec, log_space);
+    const int64_t max_pass = c->opt_max_repair > 0 ? c->opt_max_repair : PB.nchunks + 1;
+    int fb_rounds = 0;
+    for (int64_t pass = 0;; ++pass) {
+        CU(tehmm_launch_verify(st, PB, prec, c->m.NP, sv, ev, tol, kind == 1 ? -1 : +1, log_space ? 0 : 1, bad, nbad, lkap));
+        c->launches += 1;
+        int nb = 0;
+        if (umma && pass == 0) CU(cudaMemcpyAsync(c->h_nbad + 1, c->d_fault, sizeof(int), cudaMemcpyDeviceToHost, st));
+        if (read_nbad(c, nbad, &nb, !umma)) return TEHMM_ECUDA;
+        if (umma && pass == 0 && c->h_nbad[1]) {
+            CU(cudaMemsetAsync(c->d_fault, 0, sizeof(int), st));
+            return fail(TEHMM_ECUDA, "%s: a barrier wait timed out (tensor-memory protocol fault)", umma_kernel[kind]);
+        }
+        if (pass == 0) adapt_warmup(c, nb, PB.nchunks);
+        if (nb == 0) break;
+        if (pass >= max_pass) return fail(TEHMM_ESTATE, "%s repair did not converge (%d chunks left)", what[kind], nb);
+        if (c->opt_fallback_after >= 0 && pass >= c->opt_fallback_after && fallback_ok && fb_rounds < TEHMM_MAX_FALLBACK_ROUNDS) {
+            // slow mixing: resolve the flagged chunks exactly (transfer operators + chain) instead of one link per pass
+            if (resolve_flagged(c, st, PB, prec, kind, lat, sv, ev, bad, (int64_t)8 << (2 * fb_rounds))) return TEHMM_ECUDA;
+            tol = tolerance_after_fallback(c, prec, log_space);
+            fb_rounds += 1;
+        }
+        *stat_repair[kind] += 1; *stat_bad[kind] += nb;
+        CU(launch(1));
+        c->launches += 1;
+    }
+    return TEHMM_OK;
+}
+extern "C" {
+
+// fp32 without segment ratios, unless option "tile" is 0: the mma.sync tile kernels (tile.cu) at <= 32 states,
+// the tcgen05 kernels (umma.cu) for the first pass over a single-sequence batch at 33..64 states
 static bool use_tile(const tehmm_ctx *c, int prec, const double *d_ratios)
 {
-    return c->opt_tile != 0 && prec == TEHMM_F32 && c->m.NS == 1 && c->m.LD == 32 && d_ratios == nullptr;
+    return c->opt_tile != 0 && prec == TEHMM_F32 && c->m.NS == 1 && d_ratios == nullptr;
+}
+static bool use_umma(const tehmm_ctx *c, int prec, const double *d_ratios)
+{
+    return c->opt_tile != 0 && prec == TEHMM_F32 && c->m.NS == 2 && d_ratios == nullptr && c->b.nseq == 1;
 }
 
 int tehmm_run_forward(tehmm_ctx *c, int prec, const void *d_blin, const double *d_rowmax,
@@ -1233,17 +1283,16 @@ int tehmm_run_forward(tehmm_ctx *c, int prec, const void *d_blin, const double *
     // 33..64 states: the tcgen05 kernel (csrc/umma.cu, M128 N64 K8 tf32, state and accumulator in tensor memory,
     // transition matrix in shared memory) takes the first pass over a single-sequence batch on the fine
     // partition; repairs and everything else stay with the one-chunk-per-warp kernel
-    const bool wide_umma = c->opt_umma64 != 0 && c->opt_tile != 0 && prec == TEHMM_F32 && c->m.NS == 2 && c->m.LD == 64 &&
-                           d_ratios == nullptr && c->b.nseq == 1;
+    const bool wide_umma = use_umma(c, prec, d_ratios);
     const TehmmBatchDev &PB = (tile || wide_umma) ? c->bf : c->b;       // the partition this pass runs on
     bool umma_used = false;
     auto launch = [&](int mode) -> cudaError_t {
-        if (((tile && c->opt_umma) || wide_umma) && tehmm_forward_umma_ok(c->m, PB, mode, c->fine_len)) {
+        if (wide_umma && tehmm_forward_umma_ok(c->m, PB, mode, c->fine_len)) {
             cudaError_t eu = tehmm_launch_forward_umma(st, c->m, PB, (const float *)d_blin, d_rowmax, (float *)d_alpha,
-                                                       (float *)sv, (float *)ev, cs, c->sms, c->fine_len, c->d_fault, c->opt_umma == 2 ? 2 : 1);
+                                                       (float *)sv, (float *)ev, cs, c->sms, c->fine_len, c->d_fault);
             if (eu == cudaSuccess) { c->stat_umma_passes += 1; umma_used = true; return eu; }
             if (eu != cudaErrorNotSupported) return eu;
-            cudaGetLastError();          // no tensor map: the mma.sync kernel below
+            cudaGetLastError();          // no tensor map: the one-chunk-per-warp kernel below
         }
         if (tile) {
             c->stat_tile_passes += 1;
@@ -1251,36 +1300,7 @@ int tehmm_run_forward(tehmm_ctx *c, int prec, const void *d_blin, const double *
         }
         return tehmm_launch_forward(st, c->m, PB, prec, d_blin, d_rowmax, d_ratios, d_alpha, sv, ev, cs, bad, mode, grid);
     };
-    tk_begin(c, TK_FORWARD);
-    CU(launch(0));
-    tk_end(c, TK_FORWARD);
-    c->launches += 1;
-    double tol = tolerance(prec, false);
-    const int64_t max_pass = c->opt_max_repair > 0 ? c->opt_max_repair : PB.nchunks + 1;
-    int fb_rounds = 0;
-    for (int64_t pass = 0;; ++pass) {
-        CU(tehmm_launch_verify(st, PB, prec, c->m.NP, sv, ev, tol, +1, 1, bad, nbad, lkap));
-        c->launches += 1;
-        int nb = 0;
-        if (umma_used && pass == 0) CU(cudaMemcpyAsync(c->h_nbad + 1, c->d_fault, sizeof(int), cudaMemcpyDeviceToHost, st));
-        if (read_nbad(c, nbad, &nb, !umma_used)) return TEHMM_ECUDA;
-        if (umma_used && pass == 0 && c->h_nbad[1]) {
-            CU(cudaMemsetAsync(c->d_fault, 0, sizeof(int), st));
-            return fail(TEHMM_ECUDA, "fwd_umma_kernel: a barrier wait timed out (tensor-memory protocol fault)");
-        }
-        if (pass == 0) adapt_warmup(c, nb, PB.nchunks);
-        if (nb == 0) break;
-        if (pass >= max_pass) return fail(TEHMM_ESTATE, "forward repair did not converge (%d chunks left)", nb);
-        if (c->opt_fallback_after >= 0 && pass >= c->opt_fallback_after && d_ratios == nullptr && fb_rounds < TEHMM_MAX_FALLBACK_ROUNDS) {
-            // slow mixing: resolve the flagged chunks exactly (transfer operators + chain) instead of one link per pass
-            if (resolve_flagged(c, st, PB, prec, 0, d_blin, sv, ev, bad, (int64_t)8 << (2 * fb_rounds))) return TEHMM_ECUDA;
-            tol = tolerance_after_fallback(c, prec, false);
-            fb_rounds += 1;
-        }
-        c->stat_repair_fwd += 1; c->stat_bad_fwd += nb;
-        CU(launch(1));
-        c->launches += 1;
-    }
+    if (int rc = repair_loop(c, st, PB, prec, 0, d_blin, sv, ev, bad, nbad, lkap, d_ratios == nullptr, &umma_used, launch)) return rc;
     CU(tehmm_launch_forward_logprob(st, PB, prec, c->m.NP, ev, cs, lkap, d_logprob));
     c->launches += 1;
     return TEHMM_OK;
@@ -1303,15 +1323,14 @@ int tehmm_run_backward(tehmm_ctx *c, int prec, int flags, const void *d_blin, co
     void *xi = w + s.xi, *xd = w + s.xdiag, *g0 = w + s.gamma0;
     const int grid = scan_grid(c);
     // Expected transition counts on the tensor-core path: posteriors from bwd_tile_kernel, then
-    // xi_tile_kernel (two dense products per 16 steps).  Needs the posterior lattice, un-renormalised.
-    const bool xi_tile = use_tile(c, prec, d_ratios) && (flags & TEHMM_BWD_TRANS) && (flags & TEHMM_BWD_POSTERIORS) &&
-                         !(flags & TEHMM_BWD_RENORM_EPS) && c->opt_xi_tile != 0;
-    if (xi_tile) flags &= ~TEHMM_BWD_TRANS;
+    // xi_mma_kernel (two dense products per 16 steps).  Needs the posterior lattice, un-renormalised.
+    const bool xi_mma = use_tile(c, prec, d_ratios) && (flags & TEHMM_BWD_TRANS) && (flags & TEHMM_BWD_POSTERIORS) &&
+                         !(flags & TEHMM_BWD_RENORM_EPS);
+    if (xi_mma) flags &= ~TEHMM_BWD_TRANS;
     const bool tile = use_tile(c, prec, d_ratios) && !(flags & TEHMM_BWD_TRANS);
     // 33..64 states, one sequence, no transition counts: the tcgen05 twin of the forward kernel (csrc/umma.cu) takes the
     // first pass on the fine partition; repairs stay with the one-chunk-per-warp kernel on the same partition
-    const bool wide_umma = c->opt_umma64 != 0 && c->opt_tile != 0 && prec == TEHMM_F32 && c->m.NS == 2 && c->m.LD == 64 &&
-                           d_ratios == nullptr && c->b.nseq == 1 && !(flags & TEHMM_BWD_TRANS);
+    const bool wide_umma = use_umma(c, prec, d_ratios) && !(flags & TEHMM_BWD_TRANS);
     const TehmmBatchDev &PB = (tile || wide_umma) ? c->bf : c->b;
     bool umma_used = false;
     auto launch = [&](int mode) -> cudaError_t {
@@ -1324,44 +1343,16 @@ int tehmm_run_backward(tehmm_ctx *c, int prec, int flags, const void *d_blin, co
         }
         if (tile) {
             c->stat_tile_passes += 1;
-            return tehmm_launch_backward_tile(st, c->m, PB, flags, (const float *)d_blin, (const float *)d_alpha, (float *)d_post, d_map_states, mp, (float *)sv, (float *)ev, bad, mode, c->sms, c->fine_len, (int)c->opt_bwd_tmap);
+            return tehmm_launch_backward_tile(st, c->m, PB, flags, (const float *)d_blin, (const float *)d_alpha, (float *)d_post, d_map_states, mp, (float *)sv, (float *)ev, bad, mode, c->sms);
         }
         return tehmm_launch_backward(st, c->m, PB, prec, flags, d_blin, d_alpha, d_ratios, d_post, d_map_states, mp, xi, xd, g0, sv, ev, bad, mode, grid);
     };
-    tk_begin(c, TK_BACKWARD);
-    CU(launch(0));
-    tk_end(c, TK_BACKWARD);
-    c->launches += 1;
-    double tol = tolerance(prec, false);
-    const int64_t max_pass = c->opt_max_repair > 0 ? c->opt_max_repair : PB.nchunks + 1;
-    int fb_rounds = 0;
-    for (int64_t pass = 0;; ++pass) {
-        CU(tehmm_launch_verify(st, PB, prec, c->m.NP, sv, ev, tol, -1, 1, bad, nbad, nullptr));
-        c->launches += 1;
-        int nb = 0;
-        if (umma_used && pass == 0) CU(cudaMemcpyAsync(c->h_nbad + 1, c->d_fault, sizeof(int), cudaMemcpyDeviceToHost, st));
-        if (read_nbad(c, nbad, &nb, !umma_used)) return TEHMM_ECUDA;
-        if (umma_used && pass == 0 && c->h_nbad[1]) {
-            CU(cudaMemsetAsync(c->d_fault, 0, sizeof(int), st));
-            return fail(TEHMM_ECUDA, "bwd_umma_kernel: a barrier wait timed out (tensor-memory protocol fault)");
-        }
-        if (pass == 0) adapt_warmup(c, nb, PB.nchunks);
-        if (nb == 0) break;
-        if (pass >= max_pass) return fail(TEHMM_ESTATE, "backward repair did not converge (%d chunks left)", nb);
-        if (c->opt_fallback_after >= 0 && pass >= c->opt_fallback_after && d_ratios == nullptr && fb_rounds < TEHMM_MAX_FALLBACK_ROUNDS) {
-            if (resolve_flagged(c, st, PB, prec, 1, d_blin, sv, ev, bad, (int64_t)8 << (2 * fb_rounds))) return TEHMM_ECUDA;
-            tol = tolerance_after_fallback(c, prec, false);
-            fb_rounds += 1;
-        }
-        c->stat_repair_bwd += 1; c->stat_bad_bwd += nb;
-        CU(launch(1));
-        c->launches += 1;
-    }
+    if (int rc = repair_loop(c, st, PB, prec, 1, d_blin, sv, ev, bad, nbad, nullptr, d_ratios == nullptr, &umma_used, launch)) return rc;
     if (flags & TEHMM_BWD_MAP) { CU(tehmm_launch_map_reduce(st, PB, mp, d_map_score)); c->launches += 1; }
     if (flags & TEHMM_BWD_TRANS) { CU(tehmm_launch_trans_reduce(st, c->m, c->b, prec, xi, xd, g0, d_start_trans)); c->launches += 1; }
-    if (xi_tile) {
+    if (xi_mma) {
         tk_begin(c, TK_XI);
-        CU(tehmm_launch_xi_tile(st, c->m, c->bf, (const float *)d_alpha, (const float *)d_post, (double *)xi, (float *)g0, d_start_trans, c->sms));
+        CU(tehmm_launch_xi_mma(st, c->m, c->bf, (const float *)d_alpha, (const float *)d_post, (double *)xi, (float *)g0, d_start_trans, c->sms));
         tk_end(c, TK_XI);
         c->launches += 2;
     }
@@ -1424,7 +1415,6 @@ int tehmm_run_viterbi(tehmm_ctx *c, int prec, const void *d_elog, const double *
     uint8_t *spec_end = (uint8_t *)(w + s.cmap), *pred = spec_end + TBP.nchunks, *forced = pred + TBP.nchunks;
     const int grid = scan_grid(c);
     const int tb_grid = (int)std::max<int64_t>(1, std::min<int64_t>((TBP.nchunks + TEHMM_WARPS_PER_CTA - 1) / TEHMM_WARPS_PER_CTA, (int64_t)c->sms * 5));
-    const TehmmBatchDev &PB = c->b;
     const int64_t max_pass = c->opt_max_repair > 0 ? c->opt_max_repair : c->b.nchunks + 1;
     // The log-probability: the DP's own value (sum of the row maxima it takes out, float64 across steps,
     // plus rowmax) where the lean fp32 kernel runs and the caller passed rowmax; otherwise -- float64
@@ -1432,29 +1422,10 @@ int tehmm_run_viterbi(tehmm_ctx *c, int prec, const void *d_elog, const double *
     const bool dp_score = d_rowmax != nullptr && c->opt_rescore == 0 && tehmm_viterbi_dp_scores(c->m, prec, d_ratios_dp);
     double *dsp = dp_score ? (double *)(w + s.cscale) : nullptr;
     // ---- DP: delta lattice, chunk starts speculated / verified / repaired
-    tk_begin(c, TK_VITERBI_DP);
-    CU(tehmm_launch_viterbi(st, c->m, c->b, prec, d_elog, d_ratios_dp, d_lattice, sv, ev, bad, 0, grid, d_rowmax, dsp));
-    tk_end(c, TK_VITERBI_DP);
-    c->launches += 1;
-    double tol = tolerance(prec, true);
-    int fb_rounds = 0;
-    for (int64_t pass = 0;; ++pass) {
-        CU(tehmm_launch_verify(st, c->b, prec, c->m.NP, sv, ev, tol, +1, 0, bad, nbad, nullptr));
-        c->launches += 1;
-        int nb = 0;
-        if (read_nbad(c, nbad, &nb)) return TEHMM_ECUDA;
-        if (pass == 0) adapt_warmup(c, nb, PB.nchunks);
-        if (nb == 0) break;
-        if (pass >= max_pass) return fail(TEHMM_ESTATE, "viterbi repair did not converge (%d chunks left)", nb);
-        if (c->opt_fallback_after >= 0 && pass >= c->opt_fallback_after && d_ratios_dp == nullptr && fb_rounds < TEHMM_MAX_FALLBACK_ROUNDS) {
-            if (resolve_flagged(c, st, PB, prec, 2, d_elog, sv, ev, bad, (int64_t)8 << (2 * fb_rounds))) return TEHMM_ECUDA;
-            tol = tolerance_after_fallback(c, prec, true);
-            fb_rounds += 1;
-        }
-        c->stat_repair_vit += 1; c->stat_bad_vit += nb;
-        CU(tehmm_launch_viterbi(st, c->m, c->b, prec, d_elog, d_ratios_dp, d_lattice, sv, ev, bad, 1, grid, d_rowmax, dsp));
-        c->launches += 1;
-    }
+    auto launch = [&](int mode) -> cudaError_t {
+        return tehmm_launch_viterbi(st, c->m, c->b, prec, d_elog, d_ratios_dp, d_lattice, sv, ev, bad, mode, grid, d_rowmax, dsp);
+    };
+    if (int rc = repair_loop(c, st, c->b, prec, 2, d_elog, sv, ev, bad, nbad, nullptr, d_ratios_dp == nullptr, nullptr, launch)) return rc;
     // ---- traceback: chunk end states speculated / verified / repaired
     CU(cudaMemsetAsync(bad, 0, sizeof(int) * (size_t)TBP.nchunks, st));
     tk_begin(c, TK_TRACEBACK);

@@ -58,18 +58,12 @@
 #include <cstring>
 
 #define TILE_WARPS 8
-#ifndef TEHMM_TILE_TENSOR
 #define TEHMM_TILE_TENSOR 1     // 3-D tensor-map block loads where the batch is one regularly chunked sequence
-#endif
 // Measured on B200 (10 M x 30, forward with / without the alpha store, ms):
 //   per-lane LDGSTS + STG.128 0.887 / 0.525;  TB=2,NBL=4,NBS=2 0.845 / 0.738;
 //   TB=4,NBL=2,NBS=1 0.668 / 0.542  -- small bulk copies are TMA issue bound.
-#ifndef FWD_NBL
 #define FWD_NBL 2       // forward: bulk-load block buffers (TB time steps each)
-#endif
-#ifndef FWD_NBS
 #define FWD_NBS 1       // forward: bulk-store block buffers
-#endif
 #define BWD_STAGES 5    // time steps of b and alpha staged ahead
 #define TILE_STAGE_BYTES 2048   // per warp per stage: 16 rows x 128 bytes
 #define TILE_NEVER 0x7fffffff
@@ -258,9 +252,7 @@ __device__ __forceinline__ void store_row8(float *p, bool on, const float (&v)[8
 // until the LSU has read them) this takes the global traffic off the LSU queue:
 // the per-lane path spent two thirds of its time in mio_throttle / scoreboard
 // stalls (profiles/).
-#ifndef TB
 #define TB 4                          // time steps per bulk block
-#endif
 #define TMA_RS (TB * 128 + 16)        // bytes between tile rows of a block (pad: conflict-free LDS.128)
 #define TMA_BUF (16 * TMA_RS)         // bytes of one block buffer
 #define FWD_WARP_BYTES ((((FWD_NBL + FWD_NBS) * TMA_BUF + 64) + 127) & ~127)   // per warp, 128-byte aligned (tensor copies)
@@ -614,9 +606,8 @@ bwd_tile_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
                 const float *__restrict__ alpha, float *__restrict__ post,
                 uint8_t *__restrict__ map_states, double *__restrict__ map_part,
                 float *__restrict__ start_vec, float *__restrict__ end_vec,
-                const int *__restrict__ bad, int mode, int64_t group0)
+                const int *__restrict__ bad, int mode)
 {
-    // group0: first tile this launch handles (the tiles before it went to bwd_tile_tmap_kernel)
     constexpr bool want_post = (OUT & TEHMM_BWD_POSTERIORS) != 0;
     constexpr bool want_map = (OUT & TEHMM_BWD_MAP) != 0;
     extern __shared__ __align__(128) unsigned char tile_smem[];
@@ -639,7 +630,7 @@ bwd_tile_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
     for (int i = 0; i < 8; ++i) ones[i] = 8 * q + i < N ? 1.f : 0.f;
 
     const int64_t ngroups = (b.nchunks + 15) / 16;
-    for (int64_t gi = group0 + (int64_t)blockIdx.x * TILE_WARPS + warp; gi < ngroups;
+    for (int64_t gi = (int64_t)blockIdx.x * TILE_WARPS + warp; gi < ngroups;
          gi += (int64_t)gridDim.x * TILE_WARPS) {
         // ---- schedule: at clock k the row is at time t1 - 1 + W - k
         int ks[2], ke[2], kbv[2];      // kbv: first clock whose b_{t+1} exists
@@ -877,221 +868,6 @@ bwd_tile_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
     }
 }
 
-// ------------------------------------------------------------------ backward, tensor-map blocks
-// The regular part of a single-sequence batch (tiles of sixteen full-length chunks that all have
-// more than `warmup` steps of the sequence to their right), first pass only: every row of such a
-// tile has the same schedule -- clock k is time t1 - 1 + W - k, start from a flat vector at k = 0,
-// outputs for W <= k < W + lf -- so there is no per-row bookkeeping, and the rows b_{t+1} / alpha_t
-// of BT_TB clocks x 16 chunks arrive as ONE tensor-map box each (cp.async.bulk.tensor.3d, one lane,
-// completion counted on a per-warp mbarrier) instead of 8 per-lane LDGSTS per clock through the LSU
-// queue, where bwd_tile_kernel spends its stalls (profiles/r01_notes_v3.md).  The b lattice is
-// described by a map whose base is ONE ROW further on, so that (chunk, step) addresses b_{t+1}
-// with the coordinates of alpha_t.  Clocks run right to left: a box holds the steps of a block in
-// ascending order and is consumed last row first.  Everything else -- arithmetic, scaling, the
-// posterior one clock late behind the MMAs, outputs -- is bwd_tile_kernel's, so results are
-// bit-identical.  Irregular tiles and repair passes stay with bwd_tile_kernel (group0 argument).
-#define BT_TB 2                                   // clocks per block
-#define BT_NB 3                                   // block buffers per warp
-#define BT_BOX (16 * BT_TB * 128)                 // bytes of one box (one lattice)
-#define BT_WARP_BYTES (BT_NB * 2 * BT_BOX + 128)  // per warp: buffers {b box, alpha box}, then the mbarriers
-
-template <int OUT>
-__global__ void __launch_bounds__(TILE_WARPS * 32, 1)
-bwd_tile_tmap_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, float *__restrict__ post,
-                     uint8_t *__restrict__ map_states, double *__restrict__ map_part,
-                     float *__restrict__ start_vec, float *__restrict__ end_vec,
-                     const __grid_constant__ CUtensorMap tmap_b1, const __grid_constant__ CUtensorMap tmap_a,
-                     int lf, int64_t ngroups)
-{
-    constexpr bool want_post = (OUT & TEHMM_BWD_POSTERIORS) != 0;
-    constexpr bool want_map = (OUT & TEHMM_BWD_MAP) != 0;
-    extern __shared__ __align__(128) unsigned char tile_smem[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int g = lane >> 2, q = lane & 3;
-    const int N = m.N, W = b.warmup;
-    constexpr int LD = 32;
-    const uint32_t wbase = (uint32_t)__cvta_generic_to_shared(tile_smem) + (uint32_t)(warp * BT_WARP_BYTES);
-    const uint32_t bars = wbase + BT_NB * 2 * BT_BOX;
-    // this lane's tile rows g and g+8 inside a box: [chunk][step][32 floats]
-    const uint32_t myoff = (uint32_t)(g * BT_TB * 128 + 32 * q);
-    if (lane == 0) {
-#pragma unroll
-        for (int i = 0; i < BT_NB; ++i) mbar_init(bars + 8 * i, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    fence_async_smem();
-    __syncwarp();
-    uint32_t nblk_done = 0;
-    const bool renorm = (flags & TEHMM_BWD_RENORM_EPS) != 0;
-    const float eps32 = 1.1920928955078125e-07f;
-    const double renorm_inv = 1.0 / (1.0 + (double)N * 1.1920928955078125e-07);
-    const float renorm_invf = (float)renorm_inv;
-
-    TransFrag A;
-    load_trans<true>(m, g, q, A);
-    float ones[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) ones[i] = 8 * q + i < N ? 1.f : 0.f;
-
-    const int kmax = W + lf, nblk = kmax / BT_TB;
-    for (int64_t gi = (int64_t)blockIdx.x * TILE_WARPS + warp; gi < ngroups;
-         gi += (int64_t)gridDim.x * TILE_WARPS) {
-        int64_t cid[2];
-        float *pp_[2];
-        uint8_t *mp_[2];
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-            cid[r] = gi * 16 + g + 8 * r;
-            const int64_t trow = (cid[r] + 1) * (int64_t)lf - 1 + W;     // time of clock 0
-            pp_[r] = want_post ? post + trow * LD + 8 * q : nullptr;
-            mp_[r] = want_map ? map_states + trow : nullptr;
-        }
-        u64 up[8];
-        float scp[2] = {1.f, 1.f};
-        double mapsum[2] = {0.0, 0.0};
-#pragma unroll
-        for (int c = 0; c < 8; ++c) up[c] = 0ull;
-
-        auto issue_load = [&](int j) {
-            const uint32_t slot = (nblk_done + (uint32_t)j) % BT_NB;
-            const int k0 = j * BT_TB;
-            fence_async_smem();                   // earlier reads of this buffer are done (WAR across proxies)
-            __syncwarp();
-            if (lane == 0) {
-                const bool warm = k0 < W;         // the warm-up walks the head of the chunk to the right
-                const int y = warm ? W - k0 - BT_TB : lf - (k0 - W) - BT_TB;
-                const int z = (int)(gi * 16) + (warm ? 1 : 0);
-                const uint32_t buf = wbase + slot * 2 * BT_BOX;
-                mbar_expect_tx(bars + 8 * slot, warm ? (uint32_t)BT_BOX : 2u * BT_BOX);
-                tensor_load3(buf, &tmap_b1, 0, y, z, bars + 8 * slot);
-                if (!warm) tensor_load3(buf + BT_BOX, &tmap_a, 0, y, z, bars + 8 * slot);
-            }
-        };
-
-        u64 prq[8];
-        bool pend = false;
-        auto post_out = [&](const u64 (&pr)[8], int back) {
-            u64 zs = 0ull;
-#pragma unroll
-            for (int c = 0; c < 8; ++c) zs = fadd2(zs, pr[c]);
-            const float Z0 = quad_sum(lo2(zs)), Z1 = quad_sum(hi2(zs));
-            const float invZ[2] = {__frcp_rn(Z0), __frcp_rn(Z1)};
-#pragma unroll
-            for (int r = 0; r < 2; ++r) {
-                float p[8];
-#pragma unroll
-                for (int c = 0; c < 8; ++c) p[c] = r ? hi2(pr[c]) : lo2(pr[c]);
-                if constexpr (want_map) {
-                    const float best = quad_max(fmaxf(fmax3(fmax3(p[0], p[1], p[2]), p[3], p[4]), fmax3(p[5], p[6], p[7])));
-                    int idx = 99;
-#pragma unroll
-                    for (int i = 7; i >= 0; --i)
-                        if (p[i] == best) idx = 8 * q + i;
-                    idx = min(idx, __shfl_xor_sync(TEHMM_FULL, idx, 1));
-                    idx = min(idx, __shfl_xor_sync(TEHMM_FULL, idx, 2));
-                    if (q == 0) {
-                        mp_[r][back] = (uint8_t)(idx < N ? idx : 0);
-                        const float bg = best * invZ[r];
-                        mapsum[r] += renorm ? ((double)bg + (double)eps32) * renorm_inv : (double)bg;
-                    }
-                }
-                if constexpr (want_post) {
-                    float gv[8];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        gv[i] = p[i] * invZ[r];
-                        if (renorm) gv[i] = (gv[i] + eps32) * renorm_invf * ones[i];
-                    }
-                    store_row8(pp_[r] + (int64_t)back * LD, true, gv);
-                }
-            }
-        };
-
-        for (int j = 0; j < BT_NB - 1 && j < nblk; ++j) issue_load(j);
-        for (int j = 0; j < nblk; ++j) {
-            if (j + BT_NB - 1 < nblk) issue_load(j + BT_NB - 1);
-            const uint32_t slot = (nblk_done + (uint32_t)j) % BT_NB;
-            mbar_wait(bars + 8 * slot, ((nblk_done + (uint32_t)j) / BT_NB) & 1u);
-            const uint32_t lbuf = wbase + slot * 2 * BT_BOX + myoff;
-#pragma unroll
-            for (int s = 0; s < BT_TB; ++s) {
-                const int k = j * BT_TB + s;
-                const uint32_t rowa = lbuf + (uint32_t)((BT_TB - 1 - s) * 128);      // last step of the box first
-                float at[2][8], bt[2][8];
-                lds128(rowa, bt[0], 0);
-                lds128(rowa + 16, bt[0], 4);
-                lds128(rowa + 8 * BT_TB * 128, bt[1], 0);
-                lds128(rowa + 8 * BT_TB * 128 + 16, bt[1], 4);
-                if (k >= W) {
-                    lds128(rowa + BT_BOX, at[0], 0);
-                    lds128(rowa + BT_BOX + 16, at[0], 4);
-                    lds128(rowa + BT_BOX + 8 * BT_TB * 128, at[1], 0);
-                    lds128(rowa + BT_BOX + 8 * BT_TB * 128 + 16, at[1], 4);
-                }
-                if (k == 0) {                     // speculate from a flat vector
-                    set_row(up, 0, ones);
-                    set_row(up, 1, ones);
-                    scp[0] = scp[1] = 1.f;
-                }
-                // ---- w = (b_{t+1} 2^-sh) .* beta'_{t+1};  beta'_t = w A^T
-                u64 wp[8];
-                {
-                    u64 bs[2][4];
-#pragma unroll
-                    for (int r = 0; r < 2; ++r) {
-                        const u64 s2 = pk2(scp[r], scp[r]);
-#pragma unroll
-                        for (int p = 0; p < 4; ++p) bs[r][p] = fmul2(pk2(bt[r][2 * p], bt[r][2 * p + 1]), s2);
-                    }
-#pragma unroll
-                    for (int p = 0; p < 4; ++p) {
-                        wp[2 * p] = fmul2(up[2 * p], pk2(lo2(bs[0][p]), lo2(bs[1][p])));
-                        wp[2 * p + 1] = fmul2(up[2 * p + 1], pk2(hi2(bs[0][p]), hi2(bs[1][p])));
-                    }
-                }
-                float acc[4][4];
-                tile_matmul(wp, A, acc);
-                if (pend) post_out(prq, 1);       // the previous clock's posterior, behind this clock's MMAs
-                float m0 = 0.f, m1 = 0.f;
-#pragma unroll
-                for (int nt = 0; nt < 4; ++nt) {
-                    up[2 * nt] = pk2(acc[nt][0], acc[nt][2]);
-                    up[2 * nt + 1] = pk2(acc[nt][1], acc[nt][3]);
-                    m0 = fmax3(m0, acc[nt][0], acc[nt][1]);
-                    m1 = fmax3(m1, acc[nt][2], acc[nt][3]);
-                }
-                {
-                    int dummy;
-                    scale_of(quad_max(m0), scp[0], dummy);
-                    scale_of(quad_max(m1), scp[1], dummy);
-                }
-                if (k >= W) {
-#pragma unroll
-                    for (int c = 0; c < 8; ++c) prq[c] = fmul2(up[c], pk2(at[0][c], at[1][c]));
-                    pend = true;
-                } else if (k == W - 1) {
-                    store_row_vec32(start_vec + cid[0] * 32 + 8 * q, up, 0);
-                    store_row_vec32(start_vec + cid[1] * 32 + 8 * q, up, 1);
-                }
-                if (k + 1 == kmax) {
-                    store_row_vec32(end_vec + cid[0] * 32 + 8 * q, up, 0);
-                    store_row_vec32(end_vec + cid[1] * 32 + 8 * q, up, 1);
-                }
-#pragma unroll
-                for (int r = 0; r < 2; ++r) {
-                    if constexpr (want_post) pp_[r] -= LD;
-                    if constexpr (want_map) mp_[r] -= 1;
-                }
-            }
-        }
-        nblk_done += (uint32_t)nblk;
-        if (pend) post_out(prq, 1);               // the last clock's posterior
-        if constexpr (want_map) {
-            if (q == 0) { map_part[cid[0]] = mapsum[0]; map_part[cid[1]] = mapsum[1]; }
-        }
-    }
-}
-
 // ------------------------------------------------------------------ transition counts (xi)
 // Expected transition counts of Baum-Welch (hmm.py:545-568 -> _hmm.pyx:62-117) as two
 // dense products per tile of 16 CONSECUTIVE time steps, from the lattices the E-step keeps
@@ -1117,7 +893,7 @@ __device__ __forceinline__ void tf32_split(float x, uint32_t &hi, uint32_t &lo)
 }
 
 __global__ void __launch_bounds__(TILE_WARPS * 32, 1)
-xi_tile_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ alpha,
+xi_mma_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ alpha,
                const float *__restrict__ post, double *__restrict__ xi_part, float *__restrict__ gamma0)
 {
     extern __shared__ __align__(128) unsigned char tile_smem[];
@@ -1265,13 +1041,9 @@ static int tile_grid(const TehmmBatchDev &b, int sms)
 }
 
 // [chunk][step][32 floats] view of a lattice holding ONE sequence cut into chunks of `lf` steps
-// (full-length chunks only).  false: no tensor map (driver entry point missing, odd shape).
-static bool make_lattice_tmap_tb(CUtensorMap *tm, const float *base, int64_t lf, int64_t nfull, int tb);
+// (full-length chunks only), boxes of TB steps x 16 chunks.  false: no tensor map (driver entry
+// point missing, odd shape).
 static bool make_lattice_tmap(CUtensorMap *tm, const float *base, int64_t lf, int64_t nfull)
-{
-    return make_lattice_tmap_tb(tm, base, lf, nfull, TB);
-}
-static bool make_lattice_tmap_tb(CUtensorMap *tm, const float *base, int64_t lf, int64_t nfull, int tb)
 {
     typedef CUresult (*encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
@@ -1288,10 +1060,10 @@ static bool make_lattice_tmap_tb(CUtensorMap *tm, const float *base, int64_t lf,
         else
             cudaGetLastError();
     }
-    if (!encode || nfull < 1 || lf < tb || lf > (1 << 30) || nfull > (1 << 30)) return false;
+    if (!encode || nfull < 1 || lf < TB || lf > (1 << 30) || nfull > (1 << 30)) return false;
     const cuuint64_t dims[3] = {32, (cuuint64_t)lf, (cuuint64_t)nfull};
     const cuuint64_t strides[2] = {128, (cuuint64_t)lf * 128};
-    const cuuint32_t box[3] = {32, (cuuint32_t)tb, 16}, estr[3] = {1, 1, 1};
+    const cuuint32_t box[3] = {32, (cuuint32_t)TB, 16}, estr[3] = {1, 1, 1};
     return encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void *)base, dims, strides, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
@@ -1320,57 +1092,18 @@ cudaError_t tehmm_launch_forward_tile(cudaStream_t st, const TehmmModelDev &m, c
     return cudaGetLastError();
 }
 
-// same view with one buffer's geometry for the backward blocks
-static bool make_lattice_tmap_tb(CUtensorMap *tm, const float *base, int64_t lf, int64_t nfull, int tb);
-
 cudaError_t tehmm_launch_backward_tile(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
                                        int flags, const float *blin, const float *alpha, float *post,
                                        uint8_t *map_states, double *map_part, float *start_vec,
-                                       float *end_vec, const int *bad, int mode, int sms, int64_t fine_len,
-                                       int use_tmap)
+                                       float *end_vec, const int *bad, int mode, int sms)
 {
     const int th = TILE_WARPS * 32;
     const int smem = TILE_WARPS * BWD_STAGES * 2 * TILE_STAGE_BYTES;
-    const int out = flags & (TEHMM_BWD_POSTERIORS | TEHMM_BWD_MAP);
     const int outr = flags & (TEHMM_BWD_POSTERIORS | TEHMM_BWD_MAP | TEHMM_BWD_RENORM_EPS);
-    // ---- the regular tiles of a single-sequence batch, first pass: tensor-map blocks
-    int64_t group0 = 0;
-    if (TEHMM_TILE_TENSOR && use_tmap && b.nseq == 1 && mode == 0 && fine_len > b.warmup && fine_len % BT_TB == 0 &&
-        b.warmup % BT_TB == 0 && b.warmup >= BT_TB) {
-        const int64_t lf = fine_len;
-        const int64_t nfull_b = std::min<int64_t>(b.total / lf, (b.total - 1) / lf);   // rows of b start one row in
-        const int64_t ngroups = nfull_b > 0 ? (nfull_b - 1) / 16 : 0;                 // tile + the chunk to its right inside the maps
-        CUtensorMap tmb, tma;
-        memset(&tmb, 0, sizeof tmb);
-        memset(&tma, 0, sizeof tma);
-        if (ngroups > 0 && make_lattice_tmap_tb(&tmb, blin + 32, lf, nfull_b, BT_TB) &&
-            make_lattice_tmap_tb(&tma, alpha, lf, nfull_b, BT_TB)) {
-            const int tsmem = TILE_WARPS * BT_WARP_BYTES;
-            const int64_t need = (ngroups + TILE_WARPS - 1) / TILE_WARPS;
-            const int tgrid = (int)(need < sms ? need : sms);
-#define BWD_TMAP(O) do { cudaError_t e = cudaFuncSetAttribute(bwd_tile_tmap_kernel<O>, cudaFuncAttributeMaxDynamicSharedMemorySize, tsmem); \
-                         if (e != cudaSuccess) return e; \
-                         bwd_tile_tmap_kernel<O><<<tgrid, th, tsmem, st>>>(m, b, flags, post, map_states, map_part, start_vec, end_vec, tmb, tma, (int)lf, ngroups); } while (0)
-            switch (out) {
-            case 0: BWD_TMAP(0); break;
-            case TEHMM_BWD_POSTERIORS: BWD_TMAP(TEHMM_BWD_POSTERIORS); break;
-            case TEHMM_BWD_MAP: BWD_TMAP(TEHMM_BWD_MAP); break;
-            default: BWD_TMAP(TEHMM_BWD_POSTERIORS | TEHMM_BWD_MAP); break;
-            }
-#undef BWD_TMAP
-            cudaError_t e = cudaGetLastError();
-            if (e != cudaSuccess) return e;
-            group0 = ngroups;
-        }
-    }
-    // ---- everything else (ragged tiles, sequence ends, several sequences, repair passes)
-    const int64_t left = (b.nchunks + 15) / 16 - group0;
-    if (left <= 0) return cudaSuccess;
-    const int64_t need = (left + TILE_WARPS - 1) / TILE_WARPS;
-    const int grid = (int)(need < 1 ? 1 : (need < sms ? need : sms));
+    const int grid = tile_grid(b, sms);
 #define BWD_TILE(O) do { cudaError_t e = cudaFuncSetAttribute(bwd_tile_kernel<O>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); \
                          if (e != cudaSuccess) return e; \
-                         bwd_tile_kernel<O><<<grid, th, smem, st>>>(m, b, flags, blin, alpha, post, map_states, map_part, start_vec, end_vec, bad, mode, group0); } while (0)
+                         bwd_tile_kernel<O><<<grid, th, smem, st>>>(m, b, flags, blin, alpha, post, map_states, map_part, start_vec, end_vec, bad, mode); } while (0)
     switch (outr) {
     case 0: BWD_TILE(0); break;
     case TEHMM_BWD_POSTERIORS: BWD_TILE(TEHMM_BWD_POSTERIORS); break;
@@ -1389,17 +1122,17 @@ int tehmm_tile_warps(void) { return TILE_WARPS; }
 
 // expected start / transition counts from the alpha and posterior lattices (fine partition b);
 // xi_part: sms * TILE_WARPS * 1024 doubles, gamma0: nseq * 32 floats.  2 launches.
-cudaError_t tehmm_launch_xi_tile(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
+cudaError_t tehmm_launch_xi_mma(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
                                  const float *alpha, const float *post, double *xi_part, float *gamma0,
                                  double *start_trans, int sms)
 {
     const int smem = TILE_WARPS * 2 * 16 * XI_LDS * 4;
     const int64_t need = (b.nchunks + TILE_WARPS - 1) / TILE_WARPS;       // a chunk at a time per warp
     const int grid = (int)(need < 1 ? 1 : (need < sms ? need : sms));
-    cudaError_t e = cudaFuncSetAttribute(xi_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    cudaError_t e = cudaFuncSetAttribute(xi_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return e;
-    xi_tile_kernel<<<grid, TILE_WARPS * 32, smem, st>>>(m, b, alpha, post, xi_part, gamma0);
+    xi_mma_kernel<<<grid, TILE_WARPS * 32, smem, st>>>(m, b, alpha, post, xi_part, gamma0);
     xi_reduce_kernel<<<(m.N * m.N + 127) / 128, 128, 0, st>>>(m, b, xi_part, grid * TILE_WARPS, gamma0, start_trans);
     return cudaGetLastError();
 }
-size_t tehmm_xi_tile_scratch_bytes(int sms) { return (size_t)sms * TILE_WARPS * 1024 * sizeof(double); }
+size_t tehmm_xi_mma_scratch_bytes(int sms) { return (size_t)sms * TILE_WARPS * 1024 * sizeof(double); }

@@ -1,67 +1,45 @@
-// Forward pass on the 5th-generation tensor cores: tcgen05.mma with the accumulator AND the
-// state operand in tensor memory (hmm.py:678-713 -> _hmm.pyx:120-158).
+// Forward and backward passes at 33..64 states on the 5th-generation tensor cores: tcgen05.mma
+// with the accumulator AND the state operand in tensor memory (hmm.py:678-729 -> _hmm.pyx:120-198).
 //
-// fwd_tile_kernel (tile.cu) advances 16 chunks per warp with mma.sync and keeps the recursion
-// in registers; it runs at ~40 % of the (legacy) tensor pipe and 36 % issue utilisation, and
-// neither more warps nor fewer registers move it.  Here a CTA of four warps advances ONE TILE
-// OF 128 CHUNKS (thread = chunk = TMEM lane) per step:
+// At 33..64 states the one-chunk-per-warp kernels (forward.cu, backward.cu) hold 128 registers of
+// transition matrix per lane and are issue bound on the mat-vec.  Here a CTA of eight warps advances
+// ONE TILE OF 128 CHUNKS (chunk = TMEM lane) per step, TWO threads per chunk:
 //
-//     D[128 x 32] = X_lo A_hi + X_hi A_lo + X_hi A_hi        12 tcgen05.mma (M128 N32 K8, kind::tf32),
+//     D[128 x 64] = X_lo A_hi + X_hi A_lo + X_hi A_hi        24 tcgen05.mma (M128 N64 K8, kind::tf32),
 //                                                             issued by one thread, D and X in TMEM,
 //                                                             A (hi / lo parts) in shared memory
-//     x' = D .* b_t * 2^-shift                                epilogue: tcgen05.ld of the thread's row,
-//                                                             its own maximum (no shuffles), power-of-two
-//                                                             scale with a one-step lag, mask split into
-//                                                             hi / lo, tcgen05.st back as the next X
+//     x' = D .* b_t * 2^-shift                                epilogue: tcgen05.ld of the thread's 32 columns,
+//                                                             the row maximum from both halves, power-of-two
+//                                                             scale with a one-step lag, split into hi / lo,
+//                                                             tcgen05.st back as the next X
 //
-// b rows arrive and alpha rows leave as 3-D tensor-map boxes {32 floats, TB steps, 128 chunks}
-// (SWIZZLE_128B, so that a thread reading "its" 128-byte row does not collide with its
-// neighbours), double buffered, one elected thread issuing.  Same chunk partition, same
-// speculate / verify / repair protocol, same start_vec / end_vec / cscale conventions as
-// fwd_tile_kernel, whose alpha lattice this one's is interchangeable with (everything downstream
-// is scale free).  Used for a batch that is ONE sequence (first pass); everything else takes
-// fwd_tile_kernel.
+// Warps 0-3 take columns 0-31 of the rows, warps 4-7 columns 32-63 (a warp reaches the 32 tensor-memory
+// lanes of its index modulo 4), which halves the serial epilogue between two tensor-core steps; the halves
+// of a row exchange their maxima through shared memory behind the step's one CTA barrier.  b rows arrive and
+// alpha rows leave as pairs of 3-D tensor-map boxes {32 floats, 1 step, 128 chunks} side by side (SWIZZLE_128B,
+// so that a thread reading "its" 128-byte row does not collide with its neighbours), double buffered, one
+// elected thread issuing.  Same chunk partition, same speculate / verify / repair protocol, same start_vec /
+// end_vec / cscale conventions as forward_kernel, whose alpha lattice this one's is interchangeable with
+// (everything downstream is scale free).  Used for the first pass over a batch that is ONE sequence; repairs
+// and everything else take the one-chunk-per-warp kernels.
 //
-// STATUS (measured on B200, 10 M x 30): results agree with fwd_tile_kernel (log-likelihood to
-// 5e-9 relative, identical MAP paths, no repairs) but a step of one 128-row tile takes ~2 450
-// cycles, 0.77 ms in all against 0.55 ms: the twelve MMAs cost ~190 cycles of it (dropping eight
-// of them saves 35 us); the rest is the serial round trip issue -> commit -> mbarrier ->
-// tcgen05.ld (16 KB at 64 B/cycle) -> ~310 instructions per thread with one warp per sub-partition
-// -> tcgen05.st -> CTA barrier.  Two or three CTAs per SM (TB = 1, own chunk partition) reach
-// 0.68 ms, no further: an SM-wide resource saturates near 2 000 cycles per tile step.  It is
-// therefore opt-in (context option "umma"); the next steps are packed fp32 in the epilogue, two
-// threads per row, and a second tile in flight per CTA so that the tensor core never waits.
+// Measured on B200, 10 M steps of one sequence: 1.26 ms against 2.30 ms for forward_kernel at 33, 50 and
+// 64 states (DESIGN.md §5, where the measured reason is also given why <= 32 states stay on fwd_tile_kernel).
 #include "scan.cuh"
 #include <cuda.h>
 #include <cstring>
 #include <cstdio>
 
-#ifndef UM_TB
-#define UM_TB 2                       // time steps per box
-#endif
-#ifndef UM_CTAS
-#define UM_CTAS 1                     // resident CTAs per SM
-#endif
 #define UM_ROWS 128
 #define UM_NLD 2                      // load buffers
 #define UM_NST 2                      // store buffers
-// NH = number of 32-column halves of a lattice row: 1 for <= 32 states (row stride 32), 2 for 33..64 states
-// (row stride 64; round 2).  A box is always {32 floats, TB steps, 128 chunks} with the 128-byte swizzle, so a
-// block of a 64-state lattice is two boxes side by side; TB = 1 there (shared memory).
-template <int NH> struct UmCfg {
-    static constexpr int TB = NH == 1 ? UM_TB : 1;
-    static constexpr int BOX = UM_ROWS * TB * 128;           // bytes of one box
-    static constexpr int BLK = NH * BOX;                     // bytes of one block buffer
-    static constexpr int NP = 32 * NH;
-    static constexpr int BMAT = NP * NP * 4;                 // one part (hi or lo) of the transition matrix
-    static constexpr int SMEM = 1024 + (UM_NLD + UM_NST) * BLK + 2 * BMAT + 256 + 2048;
-    static constexpr unsigned TMEM_COLS = NH == 1 ? 128u : 256u;
-};
-#ifdef UM_PROFILE
-#define UM_T(i) do { const long long now_ = clock64(); tacc[i] += now_ - tlast; tlast = now_; } while (0)
-#else
-#define UM_T(i) do { } while (0)
-#endif
+// A lattice row is 64 floats: two boxes {32 floats, 1 step, 128 chunks} with the 128-byte swizzle side by side.
+constexpr int UM_NP = 64;                                    // lattice row stride, columns of D / X
+constexpr int UM_BOX = UM_ROWS * 128;                        // bytes of one box
+constexpr int UM_BLK = 2 * UM_BOX;                           // bytes of one block buffer (one step of the tile)
+constexpr int UM_BMAT = UM_NP * UM_NP * 4;                   // one part (hi or lo) of the transition matrix
+constexpr unsigned UM_TMEM_COLS = 256u;                      // D, X hi, X lo
+constexpr int UM_FWD_SMEM = 1024 + (UM_NLD + UM_NST) * UM_BLK + 2 * UM_BMAT + 256 + 2048;
 
 __device__ __forceinline__ void um_mbar_init(uint32_t bar, int count)
 {
@@ -120,28 +98,6 @@ __device__ __forceinline__ void um_tmem_st32(uint32_t taddr, const uint32_t (&v)
                     "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
                  : "memory");
 }
-__device__ __forceinline__ void um_tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
-{
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32"
-                 "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                 : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void um_tmem_st16(uint32_t taddr, const uint32_t (&v)[16])
-{
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0],"
-                 "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};\n"
-                 :: "r"(taddr),
-                    "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]),
-                    "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-                 : "memory");
-}
-__device__ __forceinline__ void um_tmem_ld(uint32_t taddr, uint32_t (&v)[32]) { um_tmem_ld32(taddr, v); }
-__device__ __forceinline__ void um_tmem_ld(uint32_t taddr, uint32_t (&v)[16]) { um_tmem_ld16(taddr, v); }
-__device__ __forceinline__ void um_tmem_st(uint32_t taddr, const uint32_t (&v)[32]) { um_tmem_st32(taddr, v); }
-__device__ __forceinline__ void um_tmem_st(uint32_t taddr, const uint32_t (&v)[16]) { um_tmem_st16(taddr, v); }
 // D[tmem] (+)= A[tmem] * B[smem descriptor]; one thread issues on behalf of the CTA
 __device__ __forceinline__ void um_mma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate)
 {
@@ -163,22 +119,15 @@ __device__ __forceinline__ uint64_t um_smem_desc(uint32_t addr, uint32_t lbo, ui
            ((uint64_t)((sbo >> 4) & 0x3fff) << 32) | (1ull << 46);
 }
 
-// NH == 2 runs TWO threads per chunk (256 per CTA): warps 0-3 take columns 0-31 of the rows, warps 4-7 columns
-// 32-63 (a warp reaches the 32 tensor-memory lanes of its index modulo 4), which halves the serial epilogue
-// between two tensor-core steps; the halves of a row exchange their maxima through shared memory.
-// TPR = threads per chunk: 2 for NH == 2; 1 or 2 for NH == 1 (two threads of 16 columns each: round 2, option "umma" = 2).
-template <int NH, int TPR>
-__global__ void __launch_bounds__(UM_ROWS * TPR, UM_CTAS)
+__global__ void __launch_bounds__(UM_ROWS * 2, 1)
 fwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ blin,
                 const double *__restrict__ rowmax, float *__restrict__ alpha,
                 float *__restrict__ start_vec, float *__restrict__ end_vec, double *__restrict__ cscale,
                 const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_a,
                 int lf, int nfull, int *__restrict__ fault)
 {
-    typedef UmCfg<NH> C;
-    constexpr int UMTB = C::TB, NP = C::NP, LDS_ = 32 * NH;       // LDS_: lattice row stride in floats
-    constexpr int CPT = 32 * NH / TPR, CQ = CPT / 4, C2 = CPT / 2; // columns per thread, in 16-byte chunks, in pairs
-    constexpr uint32_t UMBOX = C::BOX, UMBLK = C::BLK, BMAT = C::BMAT;
+    constexpr int NP = UM_NP;
+    constexpr uint32_t UMBOX = UM_BOX, UMBLK = UM_BLK, BMAT = UM_BMAT;
     extern __shared__ unsigned char um_raw[];
     const uint32_t raw = (uint32_t)__cvta_generic_to_shared(um_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;                 // SWIZZLE_128B boxes: 1024-byte aligned
@@ -189,11 +138,10 @@ fwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ blin
     int *esum_s = reinterpret_cast<int *>(gbase);                 // reused after the main loop (load buffer 0)
     float *mxs = reinterpret_cast<float *>(gbase + (UM_NLD + UM_NST) * UMBLK + 2 * BMAT + 256);   // [parity][half][row]
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int row = tid % UM_ROWS, hh = tid / UM_ROWS;           // this thread's chunk of the tile and its column part
-    constexpr int NTHR = UM_ROWS * TPR;
-    const int col0 = CPT * hh;                                    // its first column
-    const uint32_t boxoff = (uint32_t)(col0 / 32) * UMBOX;        // the box its columns are in, the 16-byte chunk they start at
-    const uint32_t cq0 = (uint32_t)(col0 % 32) / 4u;
+    const int row = tid % UM_ROWS, hh = tid / UM_ROWS;           // this thread's chunk of the tile and its column half
+    constexpr int NTHR = UM_ROWS * 2;
+    const int col0 = 32 * hh;                                     // its first column
+    const uint32_t boxoff = (uint32_t)hh * UMBOX;                 // the box its columns are in
     const int N = m.N, W = b.warmup;
 
     // ---- transition matrix, hi / lo TF32 parts, canonical K-major layout: B[n = j][k = i] = A[i][j]
@@ -216,7 +164,7 @@ fwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ blin
     }
     if (warp == 0) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"((uint32_t)__cvta_generic_to_shared(tmem_slot)), "r"(C::TMEM_COLS) : "memory");
+                     :: "r"((uint32_t)__cvta_generic_to_shared(tmem_slot)), "r"(UM_TMEM_COLS) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // B parts (generic writes) -> tensor core (async proxy)
@@ -243,33 +191,32 @@ fwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ blin
         const int ks = first ? W : 0, ke = W + len;
         const bool boxed = valid && len == lf && c < nfull;      // its rows travel in the boxes
         const int kmax = W + lf;
-        const int nblk = (kmax + UMTB - 1) / UMTB;
         const int c0 = (int)(tile * UM_ROWS);
-        const float *brow0 = blin + (ch.t0 - W) * LDS_;          // row of clock 0 (direct path only)
-        float *arow0 = alpha ? alpha + (ch.t0 - W) * LDS_ : nullptr;
+        const float *brow0 = blin + (ch.t0 - W) * NP;            // row of clock 0 (direct path only)
+        float *arow0 = alpha ? alpha + (ch.t0 - W) * NP : nullptr;
+        const uint32_t line = (uint32_t)row;                      // 128-byte line of this thread's row in a box
 
-        auto issue_load = [&](int j) {                           // thread 0
-            const int k0 = j * UMTB;
-            const bool warm = k0 < W;
-            const uint32_t bar = bars + 8 * (j % UM_NLD);
+        auto issue_load = [&](int k) {                           // thread 0: the b rows of clock k
+            const bool warm = k < W;
+            const uint32_t bar = bars + 8 * (k % UM_NLD);
             um_mbar_expect_tx(bar, UMBLK);
 #pragma unroll
-            for (int hh = 0; hh < NH; ++hh)
-                um_tensor_load3(ldbuf + (j % UM_NLD) * UMBLK + hh * UMBOX, &tmap_b, 32 * hh, warm ? lf - W + k0 : k0 - W, c0 - (warm ? 1 : 0), bar);
+            for (int h2 = 0; h2 < 2; ++h2)
+                um_tensor_load3(ldbuf + (k % UM_NLD) * UMBLK + h2 * UMBOX, &tmap_b, 32 * h2, warm ? lf - W + k : k - W, c0 - (warm ? 1 : 0), bar);
         };
         if (tid == 0)
-            for (int j = 0; j < UM_NLD && j < nblk; ++j) issue_load(j);
+            for (int k = 0; k < UM_NLD && k < kmax; ++k) issue_load(k);
 
         // ---- initial operand: a flat vector (a row that starts its sequence stays empty until clock W)
-        uint32_t xh[CPT], xl[CPT];
+        uint32_t xh[32], xl[32];
         {
 #pragma unroll
-            for (int i = 0; i < CPT; ++i) {
+            for (int i = 0; i < 32; ++i) {
                 xh[i] = (valid && !first && col0 + i < N) ? __float_as_uint(1.f) : 0u;
                 xl[i] = 0u;
             }
-            um_tmem_st(t_hi + col0 + my_lane, xh);
-            um_tmem_st(t_lo + col0 + my_lane, xl);
+            um_tmem_st32(t_hi + col0 + my_lane, xh);
+            um_tmem_st32(t_lo + col0 + my_lane, xl);
         }
         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
         float scp = 1.f;
@@ -281,162 +228,137 @@ fwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ blin
 #pragma unroll
             for (int kk = 0; kk < NP / 8; ++kk)
                 um_mma_tf32_ts(t_d, t_lo + kk * 8, um_smem_desc(bhi + kk * KSTEP, LBO, 128), idesc, kk > 0);
-#ifndef UM_EXP_ONE_PRODUCT
 #pragma unroll
             for (int kk = 0; kk < NP / 8; ++kk)
                 um_mma_tf32_ts(t_d, t_hi + kk * 8, um_smem_desc(blo + kk * KSTEP, LBO, 128), idesc, 1);
 #pragma unroll
             for (int kk = 0; kk < NP / 8; ++kk)
                 um_mma_tf32_ts(t_d, t_hi + kk * 8, um_smem_desc(bhi + kk * KSTEP, LBO, 128), idesc, 1);
-#endif
             asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar_mma) : "memory");
         };
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         __syncthreads();
         if (tid == 0) issue_mma();
 
-#ifdef UM_PROFILE
-        long long tacc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tlast = clock64();
-#endif
-        for (int j = 0; j < nblk; ++j) {
-            const uint32_t lb = ldbuf + (j % UM_NLD) * UMBLK, sb = stbuf + (j % UM_NST) * UMBLK;
-            um_mbar_wait(bars + 8 * (j % UM_NLD), (ld_phase >> (j % UM_NLD)) & 1u, vfault);
-            ld_phase ^= 1u << (j % UM_NLD);
-            UM_T(0);
-            const bool storing = alpha != nullptr && j * UMTB + UMTB > W;
-            if (storing && j >= UM_NST) {                        // the store that last used this buffer has read it
+        for (int k = 0; k < kmax; ++k) {
+            const uint32_t lb = ldbuf + (k % UM_NLD) * UMBLK, sb = stbuf + (k % UM_NST) * UMBLK;
+            um_mbar_wait(bars + 8 * (k % UM_NLD), (ld_phase >> (k % UM_NLD)) & 1u, vfault);
+            ld_phase ^= 1u << (k % UM_NLD);
+            const bool storing = alpha != nullptr && k >= W;
+            if (storing && k >= UM_NST) {                        // the store that last used this buffer has read it
                 if (tid == 0) asm volatile("cp.async.bulk.wait_group.read %0;" :: "n"(UM_NST - 1) : "memory");
                 __syncthreads();
             }
+            const bool on = valid && k >= ks && k < ke;
+            const bool start_here = first && k == ks;
+            // D of this clock
+            um_mbar_wait(bar_mma, mma_phase, vfault);
+            mma_phase ^= 1u;
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const u64 sc2 = pk2(scp, scp);
+            const int sh_now = start_here ? 0 : shp;
+            float mx = 0.f;
+            {
+                // b row half of this clock: from the box (16-byte chunks XOR-swizzled) or direct
+                float bt[32];
+                if (boxed) {
 #pragma unroll
-            for (int s = 0; s < UMTB; ++s) {
-                const int k = j * UMTB + s;
-                if (k >= kmax) break;
-                const uint32_t line = (uint32_t)(row * UMTB + s);      // 128-byte line of this thread's row in a box
-                const bool on = valid && k >= ks && k < ke;
-                const bool start_here = first && k == ks;
-                // D of this clock
-                UM_T(1);
-                um_mbar_wait(bar_mma, mma_phase, vfault);
-                mma_phase ^= 1u;
-                UM_T(2);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const u64 sc2 = pk2(scp, scp);
-                const int sh_now = start_here ? 0 : shp;
-                float mx = 0.f;
-                {
-                    // b row half of this clock: from the box (16-byte chunks XOR-swizzled) or direct
-                    float bt[CPT];
-                    if (boxed) {
+                    for (int q = 0; q < 8; ++q)
+                        asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];"
+                                     : "=f"(bt[4 * q]), "=f"(bt[4 * q + 1]), "=f"(bt[4 * q + 2]), "=f"(bt[4 * q + 3])
+                                     : "r"(lb + boxoff + line * 128u + (((uint32_t)q ^ (line & 7u)) << 4)) : "memory");
+                } else {
 #pragma unroll
-                        for (int q = 0; q < CQ; ++q)
-                            asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];"
-                                         : "=f"(bt[4 * q]), "=f"(bt[4 * q + 1]), "=f"(bt[4 * q + 2]), "=f"(bt[4 * q + 3])
-                                         : "r"(lb + boxoff + line * 128u + (((cq0 + (uint32_t)q) ^ (line & 7u)) << 4)) : "memory");
-                    } else {
-#pragma unroll
-                        for (int q = 0; q < CQ; ++q) {
-                            const float4 v = on ? *reinterpret_cast<const float4 *>(brow0 + (int64_t)k * LDS_ + col0 + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
-                            bt[4 * q] = v.x; bt[4 * q + 1] = v.y; bt[4 * q + 2] = v.z; bt[4 * q + 3] = v.w;
-                        }
+                    for (int q = 0; q < 8; ++q) {
+                        const float4 v = on ? *reinterpret_cast<const float4 *>(brow0 + (int64_t)k * NP + col0 + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
+                        bt[4 * q] = v.x; bt[4 * q + 1] = v.y; bt[4 * q + 2] = v.z; bt[4 * q + 3] = v.w;
                     }
-                    uint32_t dv[CPT];
-                    um_tmem_ld(t_d + col0 + my_lane, dv);
-                    UM_T(3);
-                    // x' = D .* b * scale in packed fp32 (FMUL2), maximum as a 3-input tree
-                    u64 a2[C2];
-                    float m0 = 0.f, m1 = 0.f;
-#pragma unroll
-                    for (int i = 0; i < C2; ++i) {
-                        const u64 d2 = ((u64)dv[2 * i + 1] << 32) | (u64)dv[2 * i];
-                        a2[i] = um_fmul2(d2, um_fmul2(pk2(bt[2 * i], bt[2 * i + 1]), sc2));
-                        if (i & 1) m1 = fmax3(m1, lo2(a2[i]), hi2(a2[i])); else m0 = fmax3(m0, lo2(a2[i]), hi2(a2[i]));
-                    }
-                    float mh = fmaxf(m0, m1);
-                    if (start_here) {                            // alpha_0 = pi .* b_0
-                        mh = 0.f;
-#pragma unroll
-                        for (int i = 0; i < C2; ++i) {
-                            const float p0 = (float)m.lin_start[col0 + 2 * i] * bt[2 * i], p1 = (float)m.lin_start[col0 + 2 * i + 1] * bt[2 * i + 1];
-                            a2[i] = pk2(p0, p1);
-                            mh = fmax3(mh, p0, p1);
-                        }
-                    }
-                    if (!valid || k < ks) {
-#pragma unroll
-                        for (int i = 0; i < C2; ++i) a2[i] = 0ull;
-                        mh = 0.f;
-                    }
-                    mx = fmaxf(mx, mh);
-                    if (k >= W) {
-                        if (alpha) {
-                            if (boxed) {
-#pragma unroll
-                                for (int q = 0; q < CQ; ++q)
-                                    asm volatile("st.shared.v2.u64 [%0], {%1,%2};"
-                                                 :: "r"(sb + boxoff + line * 128u + (((cq0 + (uint32_t)q) ^ (line & 7u)) << 4)), "l"(a2[2 * q]), "l"(a2[2 * q + 1]) : "memory");
-                            } else if (valid && k < ke) {
-#pragma unroll
-                                for (int q = 0; q < CQ; ++q)
-                                    *reinterpret_cast<ulonglong2 *>(arow0 + (int64_t)k * LDS_ + col0 + 4 * q) = make_ulonglong2(a2[2 * q], a2[2 * q + 1]);
-                            }
-                        }
-                    } else if (k == W - 1 && pred) {
-#pragma unroll
-                        for (int q = 0; q < CQ; ++q)
-                            *reinterpret_cast<ulonglong2 *>(start_vec + c * NP + col0 + 4 * q) = make_ulonglong2(a2[2 * q], a2[2 * q + 1]);
-                    }
-                    if (valid && k + 1 == ke) {
-#pragma unroll
-                        for (int q = 0; q < CQ; ++q)
-                            *reinterpret_cast<ulonglong2 *>(end_vec + c * NP + col0 + 4 * q) = make_ulonglong2(a2[2 * q], a2[2 * q + 1]);
-                    }
-                    // next operand: hi = the 11 leading bits (a TF32 number), lo = the rest, exactly (FFMA2: a - hi)
-                    const u64 neg1 = pk2(-1.f, -1.f);
-#pragma unroll
-                    for (int i = 0; i < C2; ++i) {
-                        const u64 h2 = a2[i] & 0xffffe000ffffe000ull;
-                        const u64 l2 = ffma2(h2, neg1, a2[i]);
-                        xh[2 * i] = (uint32_t)h2; xh[2 * i + 1] = (uint32_t)(h2 >> 32);
-                        xl[2 * i] = (uint32_t)l2; xl[2 * i + 1] = (uint32_t)(l2 >> 32);
-                    }
-                    UM_T(4);
-                    um_tmem_st(t_hi + col0 + my_lane, xh);
-                    um_tmem_st(t_lo + col0 + my_lane, xl);
                 }
-                if (TPR == 2) mxs[((k & 1) * 2 + hh) * UM_ROWS + row] = mx;       // the other half of the row reads it behind the barrier
-                if (k >= W) esum += k < ke ? sh_now : 0;
-                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                UM_T(5);
-                if (s == UMTB - 1 || k + 1 >= kmax) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // alpha rows -> TMA store
-                __syncthreads();
-                if (TPR == 2) mx = fmaxf(mx, mxs[((k & 1) * 2 + (hh ^ 1)) * UM_ROWS + row]);
-                {   // exact power-of-two scale for the NEXT step (scale_of in tile.cu)
-                    const unsigned mb = __float_as_uint(mx);
-                    scp = __uint_as_float(0x7f000000u - (mb & 0x7f800000u));
-                    shp = (int)(mb >> 23) - 127;
+                uint32_t dv[32];
+                um_tmem_ld32(t_d + col0 + my_lane, dv);
+                // x' = D .* b * scale in packed fp32 (FMUL2), maximum as a 3-input tree
+                u64 a2[16];
+                float m0 = 0.f, m1 = 0.f;
+#pragma unroll
+                for (int i = 0; i < 16; ++i) {
+                    const u64 d2 = ((u64)dv[2 * i + 1] << 32) | (u64)dv[2 * i];
+                    a2[i] = um_fmul2(d2, um_fmul2(pk2(bt[2 * i], bt[2 * i + 1]), sc2));
+                    if (i & 1) m1 = fmax3(m1, lo2(a2[i]), hi2(a2[i])); else m0 = fmax3(m0, lo2(a2[i]), hi2(a2[i]));
                 }
-                UM_T(6);
-                if (tid == 0 && k + 1 < kmax) issue_mma();
-                UM_T(7);
+                float mh = fmaxf(m0, m1);
+                if (start_here) {                            // alpha_0 = pi .* b_0
+                    mh = 0.f;
+#pragma unroll
+                    for (int i = 0; i < 16; ++i) {
+                        const float p0 = (float)m.lin_start[col0 + 2 * i] * bt[2 * i], p1 = (float)m.lin_start[col0 + 2 * i + 1] * bt[2 * i + 1];
+                        a2[i] = pk2(p0, p1);
+                        mh = fmax3(mh, p0, p1);
+                    }
+                }
+                if (!valid || k < ks) {
+#pragma unroll
+                    for (int i = 0; i < 16; ++i) a2[i] = 0ull;
+                    mh = 0.f;
+                }
+                mx = fmaxf(mx, mh);
+                if (k >= W) {
+                    if (alpha) {
+                        if (boxed) {
+#pragma unroll
+                            for (int q = 0; q < 8; ++q)
+                                asm volatile("st.shared.v2.u64 [%0], {%1,%2};"
+                                             :: "r"(sb + boxoff + line * 128u + (((uint32_t)q ^ (line & 7u)) << 4)), "l"(a2[2 * q]), "l"(a2[2 * q + 1]) : "memory");
+                        } else if (valid && k < ke) {
+#pragma unroll
+                            for (int q = 0; q < 8; ++q)
+                                *reinterpret_cast<ulonglong2 *>(arow0 + (int64_t)k * NP + col0 + 4 * q) = make_ulonglong2(a2[2 * q], a2[2 * q + 1]);
+                        }
+                    }
+                } else if (k == W - 1 && pred) {
+#pragma unroll
+                    for (int q = 0; q < 8; ++q)
+                        *reinterpret_cast<ulonglong2 *>(start_vec + c * NP + col0 + 4 * q) = make_ulonglong2(a2[2 * q], a2[2 * q + 1]);
+                }
+                if (valid && k + 1 == ke) {
+#pragma unroll
+                    for (int q = 0; q < 8; ++q)
+                        *reinterpret_cast<ulonglong2 *>(end_vec + c * NP + col0 + 4 * q) = make_ulonglong2(a2[2 * q], a2[2 * q + 1]);
+                }
+                // next operand: hi = the 11 leading bits (a TF32 number), lo = the rest, exactly (FFMA2: a - hi)
+                const u64 neg1 = pk2(-1.f, -1.f);
+#pragma unroll
+                for (int i = 0; i < 16; ++i) {
+                    const u64 h2 = a2[i] & 0xffffe000ffffe000ull;
+                    const u64 l2 = ffma2(h2, neg1, a2[i]);
+                    xh[2 * i] = (uint32_t)h2; xh[2 * i + 1] = (uint32_t)(h2 >> 32);
+                    xl[2 * i] = (uint32_t)l2; xl[2 * i + 1] = (uint32_t)(l2 >> 32);
+                }
+                um_tmem_st32(t_hi + col0 + my_lane, xh);
+                um_tmem_st32(t_lo + col0 + my_lane, xl);
             }
+            mxs[((k & 1) * 2 + hh) * UM_ROWS + row] = mx;       // the other half of the row reads it behind the barrier
+            if (k >= W) esum += k < ke ? sh_now : 0;
+            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // alpha rows -> TMA store
+            __syncthreads();
+            mx = fmaxf(mx, mxs[((k & 1) * 2 + (hh ^ 1)) * UM_ROWS + row]);
+            {   // exact power-of-two scale for the NEXT step (scale_of in tile.cu)
+                const unsigned mb = __float_as_uint(mx);
+                scp = __uint_as_float(0x7f000000u - (mb & 0x7f800000u));
+                shp = (int)(mb >> 23) - 127;
+            }
+            if (tid == 0 && k + 1 < kmax) issue_mma();
             if (tid == 0) {
                 if (storing) {
-                    const int k0 = j * UMTB;
 #pragma unroll
-                    for (int hh = 0; hh < NH; ++hh)
-                        um_tensor_store3(&tmap_a, 32 * hh, k0 - W, c0, sb + hh * UMBOX);       // clocks before W are never in a storing block: W % TB == 0
+                    for (int h2 = 0; h2 < 2; ++h2)
+                        um_tensor_store3(&tmap_a, 32 * h2, k - W, c0, sb + h2 * UMBOX);
                     asm volatile("cp.async.bulk.commit_group;" ::: "memory");
                 }
-                if (j + UM_NLD < nblk) issue_load(j + UM_NLD);           // every thread has passed the barrier after reading lb
+                if (k + UM_NLD < kmax) issue_load(k + UM_NLD);           // every thread has passed the barrier after reading lb
             }
         }
-#ifdef UM_PROFILE
-        if (blockIdx.x == 3 && (tid == 0 || tid == 64))
-            printf("umma tid %d cycles/step: ldwait %lld  b-load %lld  mmawait %lld  ldtm %lld  math %lld  sttm %lld  barrier %lld  issue %lld\n", tid,
-                   tacc[0] / kmax, tacc[1] / kmax, tacc[2] / kmax, tacc[3] / kmax, tacc[4] / kmax, tacc[5] / kmax, tacc[6] / kmax, tacc[7] / kmax);
-#endif
         if (tid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
         __syncthreads();
 
@@ -457,11 +379,11 @@ fwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ blin
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(C::TMEM_COLS) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(UM_TMEM_COLS) : "memory");
 }
 
-// [chunk][step][32 * NH floats] view, boxes {32, TB, 128}, 128-byte swizzle
-static bool um_make_tmap(CUtensorMap *tm, const float *base, int64_t lf, int64_t nfull, int nh, int tb)
+// [chunk][step][64 floats] view, boxes {32, 1, 128}, 128-byte swizzle
+static bool um_make_tmap(CUtensorMap *tm, const float *base, int64_t lf, int64_t nfull)
 {
     typedef CUresult (*encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
@@ -478,44 +400,19 @@ static bool um_make_tmap(CUtensorMap *tm, const float *base, int64_t lf, int64_t
         else
             cudaGetLastError();
     }
-    if (!encode || nfull < 1 || lf < tb) return false;
-    const cuuint64_t dims[3] = {(cuuint64_t)(32 * nh), (cuuint64_t)lf, (cuuint64_t)nfull};
-    const cuuint64_t strides[2] = {(cuuint64_t)(128 * nh), (cuuint64_t)lf * 128 * nh};
-    const cuuint32_t box[3] = {32, (cuuint32_t)tb, UM_ROWS}, estr[3] = {1, 1, 1};
+    if (!encode || nfull < 1 || lf < 1) return false;
+    const cuuint64_t dims[3] = {(cuuint64_t)UM_NP, (cuuint64_t)lf, (cuuint64_t)nfull};
+    const cuuint64_t strides[2] = {(cuuint64_t)(4 * UM_NP), (cuuint64_t)lf * 4 * UM_NP};
+    const cuuint32_t box[3] = {32, 1, UM_ROWS}, estr[3] = {1, 1, 1};
     return encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void *)base, dims, strides, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// whether this batch / pass can take the tcgen05 kernel: one sequence, first pass, lattice rows of 32 or 64 floats
+// whether this batch / pass can take the tcgen05 forward kernel: 33..64 states, one sequence, first pass
 bool tehmm_forward_umma_ok(const TehmmModelDev &m, const TehmmBatchDev &b, int mode, int64_t fine_len)
 {
-    const int nh = m.NS;
-    const int tb = nh == 1 ? UM_TB : 1;
-    return m.LD == 32 * nh && b.nseq == 1 && mode == 0 && fine_len >= b.warmup && (b.warmup % tb) == 0 &&
-           b.total / fine_len >= 1;
-}
-
-template <int NH, int TPR>
-static cudaError_t launch_umma(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
-                               const float *blin, const double *rowmax, float *alpha,
-                               float *start_vec, float *end_vec, double *cscale, int sms,
-                               int64_t fine_len, int *fault)
-{
-    typedef UmCfg<NH> C;
-    CUtensorMap tb, ta;
-    memset(&tb, 0, sizeof tb);
-    memset(&ta, 0, sizeof ta);
-    const int64_t nfull = b.total / fine_len;
-    if (!um_make_tmap(&tb, blin, fine_len, nfull, NH, C::TB) || (alpha && !um_make_tmap(&ta, alpha, fine_len, nfull, NH, C::TB)))
-        return cudaErrorNotSupported;
-    cudaError_t e = cudaFuncSetAttribute(fwd_umma_kernel<NH, TPR>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM);
-    if (e != cudaSuccess) return e;
-    const int64_t tiles = (b.nchunks + UM_ROWS - 1) / UM_ROWS;
-    const int grid = (int)(tiles < (int64_t)sms * UM_CTAS ? tiles : (int64_t)sms * UM_CTAS);
-    fwd_umma_kernel<NH, TPR><<<grid, UM_ROWS * TPR, C::SMEM, st>>>(m, b, blin, rowmax, alpha, start_vec, end_vec, cscale, tb, ta,
-                                                        (int)fine_len, (int)nfull, fault);
-    return cudaGetLastError();
+    return m.NS == 2 && b.nseq == 1 && mode == 0 && fine_len >= b.warmup && b.total / fine_len >= 1;
 }
 
 // ------------------------------------------------------------------ backward twin (33..64 states)
@@ -533,28 +430,19 @@ static cudaError_t launch_umma(cudaStream_t st, const TehmmModelDev &m, const Te
 // single-sequence batch only; repairs and transition counts stay with backward_kernel (backward.cu), whose
 // start_vec / end_vec / map_part conventions these are.
 #define UM_NA 3
-template <int NH> struct UmBwdCfg {
-    static constexpr int BOX = UM_ROWS * 128;
-    static constexpr int BLK = NH * BOX;
-    static constexpr int NP = 32 * NH;
-    static constexpr int BMAT = NP * NP * 4;
-    static constexpr int XCH = 4 * 2 * NH * UM_ROWS * 4;       // row maximum, Z, best, arg-max: [parity][half][row]
-    static constexpr int SMEM = 1024 + (UM_NLD + UM_NA) * BLK + 2 * BMAT + 256 + XCH;
-    static constexpr unsigned TMEM_COLS = NH == 1 ? 128u : 256u;
-};
+constexpr int UM_XCH = 4 * 2 * 2 * UM_ROWS * 4;          // row maximum, Z, best, arg-max: [parity][half][row]
+constexpr int UM_BWD_SMEM = 1024 + (UM_NLD + UM_NA) * UM_BLK + 2 * UM_BMAT + 256 + UM_XCH;
 
-template <int NH>
-__global__ void __launch_bounds__(UM_ROWS * NH, 1)
+__global__ void __launch_bounds__(UM_ROWS * 2, 1)
 bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__restrict__ blin,
                 const float *__restrict__ alpha, float *__restrict__ post, uint8_t *__restrict__ map_states,
                 double *__restrict__ map_part, float *__restrict__ start_vec, float *__restrict__ end_vec,
                 const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_a,
                 const __grid_constant__ CUtensorMap tmap_p, int lf, int nfull, int *fault)
 {
-    typedef UmBwdCfg<NH> C;
-    constexpr int NP = C::NP, LDS_ = 32 * NH;
-    constexpr uint32_t UMBOX = C::BOX, UMBLK = C::BLK, BMAT = C::BMAT;
-    constexpr int OFF_MAT = (UM_NLD + UM_NA) * C::BLK, OFF_BAR = OFF_MAT + 2 * C::BMAT;
+    constexpr int NP = UM_NP, NH = 2;                             // NH: column halves of a row, one thread each
+    constexpr uint32_t UMBOX = UM_BOX, UMBLK = UM_BLK, BMAT = UM_BMAT;
+    constexpr int OFF_MAT = (UM_NLD + UM_NA) * UM_BLK, OFF_BAR = OFF_MAT + 2 * UM_BMAT;
     extern __shared__ unsigned char um_raw[];
     const uint32_t raw = (uint32_t)__cvta_generic_to_shared(um_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;
@@ -594,7 +482,7 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
     }
     if (warp == 0) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"((uint32_t)__cvta_generic_to_shared(tmem_slot)), "r"(C::TMEM_COLS) : "memory");
+                     :: "r"((uint32_t)__cvta_generic_to_shared(tmem_slot)), "r"(UM_TMEM_COLS) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -623,9 +511,9 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
         const int kmax = W + lf;
         const int c0 = (int)(tile * UM_ROWS);
         const int64_t trow = ch.t1 - 1 + W;                       // time of clock 0
-        const float *bclk0 = blin + trow * LDS_ + 32 * hh;
-        const float *aclk0 = alpha + trow * LDS_ + 32 * hh;
-        float *pclk0 = want_post ? post + trow * LDS_ + 32 * hh : nullptr;
+        const float *bclk0 = blin + trow * NP + 32 * hh;
+        const float *aclk0 = alpha + trow * NP + 32 * hh;
+        float *pclk0 = want_post ? post + trow * NP + 32 * hh : nullptr;
         uint8_t *mclk0 = want_map ? map_states + trow : nullptr;
         double mapsum = 0.0;
 
@@ -706,7 +594,7 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
             } else {
 #pragma unroll
                 for (int q = 0; q < 8; ++q) {
-                    const float4 v = on ? *reinterpret_cast<const float4 *>(bclk0 - (int64_t)k * LDS_ + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
+                    const float4 v = on ? *reinterpret_cast<const float4 *>(bclk0 - (int64_t)k * NP + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
                     bt[4 * q] = v.x; bt[4 * q + 1] = v.y; bt[4 * q + 2] = v.z; bt[4 * q + 3] = v.w;
                 }
             }
@@ -747,7 +635,7 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
                 um_tmem_st32(t_hi + 32 * hh + my_lane, xh);
                 um_tmem_st32(t_lo + 32 * hh + my_lane, xl);
             }
-            if (NH == 2) mxs[(par * NH + hh) * UM_ROWS + row] = mx;
+            mxs[(par * NH + hh) * UM_ROWS + row] = mx;
             // chunk boundary vectors (beta' itself, any scale: the verification is ratio based)
             if (k == W - 1 && succ && k >= ks) {
 #pragma unroll
@@ -775,7 +663,7 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
                 } else {
 #pragma unroll
                     for (int q = 0; q < 8; ++q) {
-                        const float4 v = outp ? *reinterpret_cast<const float4 *>(aclk0 - (int64_t)k * LDS_ + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
+                        const float4 v = outp ? *reinterpret_cast<const float4 *>(aclk0 - (int64_t)k * NP + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
                         at[4 * q] = v.x; at[4 * q + 1] = v.y; at[4 * q + 2] = v.z; at[4 * q + 3] = v.w;
                     }
                 }
@@ -794,17 +682,15 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
                     for (int i = 31; i >= 0; --i)
                         if (p[i] == best) idx = 32 * hh + i;       // lowest state among the maxima (np.argmax, basehmm.py:357)
                 }
-                if (NH == 2) {
-                    zs[(par * NH + hh) * UM_ROWS + row] = z0 + z1;
-                    bests[(par * NH + hh) * UM_ROWS + row] = best;
-                    idxs[(par * NH + hh) * UM_ROWS + row] = idx;
-                }
+                zs[(par * NH + hh) * UM_ROWS + row] = z0 + z1;
+                bests[(par * NH + hh) * UM_ROWS + row] = best;
+                idxs[(par * NH + hh) * UM_ROWS + row] = idx;
                 zown = z0 + z1; bown = best; iown = idx;
             }
             asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncthreads();
-            if (NH == 2) mx = fmaxf(mx, mxs[(par * NH + (hh ^ 1)) * UM_ROWS + row]);
+            mx = fmaxf(mx, mxs[(par * NH + (hh ^ 1)) * UM_ROWS + row]);
             {
                 const unsigned mb = __float_as_uint(mx);
                 scp = __uint_as_float(0x7f000000u - (mb & 0x7f800000u));
@@ -813,13 +699,11 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
             if (!warm) {
                 int idx = iown;
                 float Z = zown, best = bown;
-                if (NH == 2) {
-                    const float zo = zs[(par * NH + (hh ^ 1)) * UM_ROWS + row];
-                    const float bo = bests[(par * NH + (hh ^ 1)) * UM_ROWS + row];
-                    const int io = idxs[(par * NH + (hh ^ 1)) * UM_ROWS + row];
-                    Z = hh == 0 ? Z + zo : zo + Z;                // the same sum in both halves
-                    if (bo > best || (bo == best && io < idx)) { best = bo; idx = io; }
-                }
+                const float zo = zs[(par * NH + (hh ^ 1)) * UM_ROWS + row];
+                const float bo = bests[(par * NH + (hh ^ 1)) * UM_ROWS + row];
+                const int io = idxs[(par * NH + (hh ^ 1)) * UM_ROWS + row];
+                Z = hh == 0 ? Z + zo : zo + Z;                // the same sum in both halves
+                if (bo > best || (bo == best && io < idx)) { best = bo; idx = io; }
                 const float invZ = __frcp_rn(Z);
                 if (want_map && hh == 0 && outp) {
                     mclk0[-(int64_t)k] = (uint8_t)(idx < N ? idx : 0);
@@ -841,7 +725,7 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
                     } else if (outp) {
 #pragma unroll
                         for (int q = 0; q < 8; ++q)
-                            *reinterpret_cast<float4 *>(pclk0 - (int64_t)k * LDS_ + 4 * q) = make_float4(p[4 * q], p[4 * q + 1], p[4 * q + 2], p[4 * q + 3]);
+                            *reinterpret_cast<float4 *>(pclk0 - (int64_t)k * NP + 4 * q) = make_float4(p[4 * q], p[4 * q + 1], p[4 * q + 2], p[4 * q + 3]);
                     }
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // posterior rows -> TMA store (behind the next barrier)
                 }
@@ -883,12 +767,12 @@ bwd_umma_kernel(TehmmModelDev m, TehmmBatchDev b, int flags, const float *__rest
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(C::TMEM_COLS) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(UM_TMEM_COLS) : "memory");
 }
 
 bool tehmm_backward_umma_ok(const TehmmModelDev &m, const TehmmBatchDev &b, int flags, int mode, int64_t fine_len)
 {
-    return m.NS == 2 && m.LD == 64 && b.nseq == 1 && mode == 0 && !(flags & TEHMM_BWD_TRANS) && fine_len >= b.warmup &&
+    return m.NS == 2 && b.nseq == 1 && mode == 0 && !(flags & TEHMM_BWD_TRANS) && fine_len >= b.warmup &&
            b.total / fine_len >= 1;
 }
 
@@ -897,21 +781,20 @@ cudaError_t tehmm_launch_backward_umma(cudaStream_t st, const TehmmModelDev &m, 
                                        double *map_part, float *start_vec, float *end_vec, int sms,
                                        int64_t fine_len, int *fault)
 {
-    typedef UmBwdCfg<2> C;
     CUtensorMap tb, ta, tp;
     memset(&tb, 0, sizeof tb);
     memset(&ta, 0, sizeof ta);
     memset(&tp, 0, sizeof tp);
     const int64_t nfull = b.total / fine_len;
     const bool want_post = (flags & TEHMM_BWD_POSTERIORS) != 0 && post != nullptr;
-    if (!um_make_tmap(&tb, blin, fine_len, nfull, 2, 1) || !um_make_tmap(&ta, alpha, fine_len, nfull, 2, 1) ||
-        (want_post && !um_make_tmap(&tp, post, fine_len, nfull, 2, 1)))
+    if (!um_make_tmap(&tb, blin, fine_len, nfull) || !um_make_tmap(&ta, alpha, fine_len, nfull) ||
+        (want_post && !um_make_tmap(&tp, post, fine_len, nfull)))
         return cudaErrorNotSupported;
-    cudaError_t e = cudaFuncSetAttribute(bwd_umma_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM);
+    cudaError_t e = cudaFuncSetAttribute(bwd_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, UM_BWD_SMEM);
     if (e != cudaSuccess) return e;
     const int64_t tiles = (b.nchunks + UM_ROWS - 1) / UM_ROWS;
     const int grid = (int)(tiles < (int64_t)sms ? tiles : (int64_t)sms);
-    bwd_umma_kernel<2><<<grid, UM_ROWS * 2, C::SMEM, st>>>(m, b, flags, blin, alpha, post, map_states, map_part, start_vec, end_vec,
+    bwd_umma_kernel<<<grid, UM_ROWS * 2, UM_BWD_SMEM, st>>>(m, b, flags, blin, alpha, post, map_states, map_part, start_vec, end_vec,
                                                         tb, ta, tp, (int)fine_len, (int)nfull, fault);
     return cudaGetLastError();
 }
@@ -919,9 +802,19 @@ cudaError_t tehmm_launch_backward_umma(cudaStream_t st, const TehmmModelDev &m, 
 cudaError_t tehmm_launch_forward_umma(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
                                       const float *blin, const double *rowmax, float *alpha,
                                       float *start_vec, float *end_vec, double *cscale, int sms,
-                                      int64_t fine_len, int *fault, int threads_per_chunk)
+                                      int64_t fine_len, int *fault)
 {
-    if (m.NS == 1 && threads_per_chunk == 2) return launch_umma<1, 2>(st, m, b, blin, rowmax, alpha, start_vec, end_vec, cscale, sms, fine_len, fault);
-    if (m.NS == 1) return launch_umma<1, 1>(st, m, b, blin, rowmax, alpha, start_vec, end_vec, cscale, sms, fine_len, fault);
-    return launch_umma<2, 2>(st, m, b, blin, rowmax, alpha, start_vec, end_vec, cscale, sms, fine_len, fault);
+    CUtensorMap tb, ta;
+    memset(&tb, 0, sizeof tb);
+    memset(&ta, 0, sizeof ta);
+    const int64_t nfull = b.total / fine_len;
+    if (!um_make_tmap(&tb, blin, fine_len, nfull) || (alpha && !um_make_tmap(&ta, alpha, fine_len, nfull)))
+        return cudaErrorNotSupported;
+    cudaError_t e = cudaFuncSetAttribute(fwd_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, UM_FWD_SMEM);
+    if (e != cudaSuccess) return e;
+    const int64_t tiles = (b.nchunks + UM_ROWS - 1) / UM_ROWS;
+    const int grid = (int)(tiles < (int64_t)sms ? tiles : (int64_t)sms);
+    fwd_umma_kernel<<<grid, UM_ROWS * 2, UM_FWD_SMEM, st>>>(m, b, blin, rowmax, alpha, start_vec, end_vec, cscale, tb, ta,
+                                                            (int)fine_len, (int)nfull, fault);
+    return cudaGetLastError();
 }

@@ -1,18 +1,18 @@
 // Chunked parallel-in-time Viterbi with on-device parallel traceback
 // (hmm.py:668-676 -> _hmm.pyx:201-259).
 //
-// DP (viterbi_kernel; viterbi_lean_kernel for the fp32 production case, see there):
+// DP (viterbi_kernel, float64; the fp32 kernels are viterbi_lean_kernel at <= 32
+// states and viterbi_wide_kernel at 33..64, see there):
 // one warp per chunk, lane j owns column j of log A in
 // registers, delta is kept max-normalised (max = 0) and broadcast through
 // shared memory.  The kernel is issue-bound, so it computes VALUES only:
 //     delta_t[j] = max_i(delta_{t-1}[i] + logA[i][j]) + e_t[j]
-// with packed FADD2 + 3-input FMNMX3 (one instruction per candidate instead of
-// four with an explicit arg-max) and writes the normalised delta lattice.
+// and writes the normalised delta lattice.
 // Chunks that do not begin a sequence speculate their start vector with
 // `warmup` steps from a flat vector and are verified / repaired like forward.cu.
 //
-// Traceback (vit_traceback_kernel): back-pointers are needed only ALONG the
-// best path, so they are recomputed there: with state s at time t,
+// Traceback (vit_traceback_kernel, float64; vit_traceback4_kernel in fp32): back-pointers
+// are needed only ALONG the best path, so they are recomputed there: with state s at time t,
 //     s_{t-1} = lowest i maximising delta_{t-1}[i] + logA[i][s]
 // from the stored lattice, lane i evaluating candidate i with exactly the
 // operands the DP used (so ties fall as in the reference: strict '>' scanning
@@ -22,8 +22,11 @@
 // beyond the chunk end, best paths coalesce), then verified against the state
 // the right neighbour really reaches, and repaired where different.
 //
-// The returned log-probability is a float64 re-score of the returned path
-// against the float64 tables, so it does not carry fp32 DP rounding.
+// The returned log-probability: where viterbi_lean_kernel runs without segment
+// ratios and the caller passes the emission row maxima, it is the DP's own value
+// (the row maxima it takes out, summed in float64, plus those); otherwise (float64, segment ratios, more than 32
+// states, option "rescore") it is a float64 re-score of the returned path against
+// the float64 tables.
 //
 // Segment ratios (RATIO kernels): a NEGATIVE ratio marks a step of a sequence
 // that has no ratios (segRatios=None).  Such a step gets the plain recursion:
@@ -38,45 +41,42 @@
 #define VIT_U 4
 #define TB_PF 6    // delta rows in flight ahead of the traceback walk
 
-#ifndef VIT_WIDE_WARPS
-#define VIT_WIDE_WARPS 12     // fp32, 33..64 states: warps per CTA (one CTA per SM; <= 168 registers)
-#endif
-template <typename T, int NS, bool RATIO, int WARPS = TEHMM_WARPS_PER_CTA>
-__global__ void __launch_bounds__(WARPS * 32, (sizeof(T) == 4 && NS == 1) ? 3 : 1)
-viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
-               const double *__restrict__ ratios, T *__restrict__ lattice,
-               T *__restrict__ start_vec, T *__restrict__ end_vec,
+template <int NS, bool RATIO>
+__global__ void __launch_bounds__(TEHMM_WARPS_PER_CTA * 32, 1)
+viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const double *__restrict__ elog,
+               const double *__restrict__ ratios, double *__restrict__ lattice,
+               double *__restrict__ start_vec, double *__restrict__ end_vec,
                const int *__restrict__ bad, int mode)
 {
     constexpr int NP = 32 * NS;
-    __shared__ __align__(16) T ds_all[WARPS][2][NP];
+    __shared__ __align__(16) double ds_all[TEHMM_WARPS_PER_CTA][2][NP];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    T(*ds)[NP] = ds_all[warp];
+    double(*ds)[NP] = ds_all[warp];
     const int N = m.N;
     const unsigned Nu = (unsigned)m.LD;      // lattice row stride
-    const T NEG = (T)-INFINITY;
+    const double NEG = -INFINITY;
 
-    MatSlice<T, NS> A;       // column j of log A (-inf beyond N and for zero transitions)
-    T ls[NS], dg[NS];
+    MatSlice<double, NS> A;       // column j of log A (-inf beyond N and for zero transitions)
+    double ls[NS], dg[NS];
     unsigned jc[NS];
     bool own[NS];
 #pragma unroll
     for (int s = 0; s < NS; ++s) {
         const int j = lane + 32 * s;
 #pragma unroll
-        for (int i = 0; i < NP; ++i) A.set(s, i, (T)m.cut_trans[(int64_t)i * NP + j]);
-        ls[s] = (T)m.cut_start[j];
-        dg[s] = (T)m.cut_trans[(int64_t)j * NP + j];
+        for (int i = 0; i < NP; ++i) A.set(s, i, m.cut_trans[(int64_t)i * NP + j]);
+        ls[s] = m.cut_start[j];
+        dg[s] = m.cut_trans[(int64_t)j * NP + j];
         own[s] = j < N;
         jc[s] = (unsigned)min(j, N - 1);
     }
-    const T a00 = (T)m.cut_trans[0];
+    const double a00 = m.cut_trans[0];
 
-    for (int64_t ci = (int64_t)blockIdx.x * WARPS + warp; ci < b.nchunks;
-         ci += (int64_t)gridDim.x * WARPS) {
+    for (int64_t ci = (int64_t)blockIdx.x * TEHMM_WARPS_PER_CTA + warp; ci < b.nchunks;
+         ci += (int64_t)gridDim.x * TEHMM_WARPS_PER_CTA) {
         if (mode == 1 && !bad[ci]) continue;
         const TehmmChunk ch = b.chunks[ci];
-        T d[NS];
+        double d[NS];
         int buf = 0;
 
         int64_t tw = ch.t0;
@@ -85,14 +85,14 @@ viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
             tw = ch.t0 - b.warmup;
             if (tw <= ch.s0) { tw = ch.s0; from_start = true; }
         }
-        const T *__restrict__ ee = elog + tw * m.LD;
-        T *__restrict__ ll = lattice + tw * m.LD;
+        const double *__restrict__ ee = elog + tw * m.LD;
+        double *__restrict__ ll = lattice + tw * m.LD;
         const double *__restrict__ rr = RATIO ? ratios + tw : nullptr;
 
-        auto load_e = [&](unsigned row, T (&et)[NS]) {
+        auto load_e = [&](unsigned row, double (&et)[NS]) {
 #pragma unroll
             for (int s = 0; s < NS; ++s) {
-                const T v = ee[row * Nu + jc[s]];
+                const double v = ee[row * Nu + jc[s]];
                 et[s] = own[s] ? v : NEG;
             }
         };
@@ -101,44 +101,42 @@ viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
             for (int s = 0; s < NS; ++s)     // padding columns (N..LD-1) carry -inf
                 if (lane + 32 * s < m.LD) ll[row * Nu + (unsigned)(lane + 32 * s)] = own[s] ? d[s] : NEG;
         };
-        auto init = [&](unsigned row, const T (&et)[NS]) {
+        auto init = [&](unsigned row, const double (&et)[NS]) {
 #pragma unroll
             for (int s = 0; s < NS; ++s) {
                 d[s] = ls[s] + et[s];
                 if (RATIO) {
                     const double r = rr[row];
-                    if (r > 1.0) d[s] += dg[s] * (T)(r - 1.0);
+                    if (r > 1.0) d[s] += dg[s] * (r - 1.0);
                 }
             }
-            log_normalise<T, NS>(d);
+            log_normalise<double, NS>(d);
         };
-        auto step = [&](unsigned row, const T (&et)[NS]) {
+        auto step = [&](unsigned row, const double (&et)[NS]) {
 #pragma unroll
             for (int s = 0; s < NS; ++s) ds[buf][lane + 32 * s] = d[s];
             __syncwarp();
-            T y[NS];
+            double y[NS];
             if (!RATIO) {
                 matvec_maxval<NS>(ds[buf], A, y);
             } else {
                 // _hmm.pyx:234-237 vs 243-244: from-state 0 always gets A_jj*r (minus A_00
                 // when j==0); the other from-states get A_jj*(r-1), and only if r>1.
-                const T r = (T)rr[row];
-                const bool seg = r >= (T)0;        // negative: a sequence without ratios
-                const T x0 = ds[buf][0];
+                const double r = rr[row];
+                const bool seg = r >= 0.0;        // negative: a sequence without ratios
+                const double x0 = ds[buf][0];
 #pragma unroll
                 for (int s = 0; s < NS; ++s) {
-                    const T common = r > (T)1 ? dg[s] * (r - (T)1) : (T)0;
+                    const double common = r > 1.0 ? dg[s] * (r - 1.0) : 0.0;
                     // (a zero-probability self transition would give inf-inf here; the
                     //  reference's finite -1e100 sentinel has no fp32 twin, see DESIGN.md)
-                    T extra0 = seg && dg[s] > NEG ? dg[s] * r - common : (T)0;
+                    double extra0 = seg && dg[s] > NEG ? dg[s] * r - common : 0.0;
                     if (seg && lane + 32 * s == 0 && a00 > NEG) extra0 -= a00;
-                    T rest = NEG;      // max over from-states >= 1
-                    T c0 = NEG;
+                    double rest = NEG;      // max over from-states >= 1
+                    double c0 = NEG;
 #pragma unroll
                     for (int i = 0; i < NP; ++i) {
-                        T c;
-                        if constexpr (sizeof(T) == 4) c = (i & 1) ? hi2(A.c[s][i >> 1]) : lo2(A.c[s][i >> 1]);
-                        else c = A.c[s][i];
+                        const double c = A.c[s][i];
                         if (i == 0) c0 = c;
                         else rest = fmax(rest, ds[buf][i] + c);
                     }
@@ -148,7 +146,7 @@ viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
             buf ^= 1;
 #pragma unroll
             for (int s = 0; s < NS; ++s) d[s] = y[s] + et[s];
-            log_normalise<T, NS>(d);
+            log_normalise<double, NS>(d);
         };
 
         unsigned row = 0;
@@ -157,18 +155,18 @@ viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
 #pragma unroll
             for (int s = 0; s < NS; ++s) d[s] = start_vec[ci * NP + lane + 32 * s];
         } else if (from_start) {
-            T et[NS];
+            double et[NS];
             load_e(0, et);
             init(0, et);
             if (row0 == 0) store_d(0);
             row = 1;
         } else {
 #pragma unroll
-            for (int s = 0; s < NS; ++s) d[s] = own[s] ? (T)0 : NEG;
+            for (int s = 0; s < NS; ++s) d[s] = own[s] ? 0.0 : NEG;
         }
         if (mode == 0 && row0 > 0) {
             for (; row < row0; ++row) {
-                T et[NS];
+                double et[NS];
                 load_e(row, et);
                 step(row, et);
             }
@@ -176,13 +174,13 @@ viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
             for (int s = 0; s < NS; ++s) start_vec[ci * NP + lane + 32 * s] = d[s];
         }
 
-        T en[VIT_U][NS];
+        double en[VIT_U][NS];
         if (row + VIT_U <= row1) {
 #pragma unroll
             for (int u = 0; u < VIT_U; ++u) load_e(row + u, en[u]);
         }
         while (row + 2 * VIT_U <= row1) {
-            T ec[VIT_U][NS];
+            double ec[VIT_U][NS];
 #pragma unroll
             for (int u = 0; u < VIT_U; ++u) {
 #pragma unroll
@@ -206,7 +204,7 @@ viterbi_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ elog,
             row += VIT_U;
         }
         for (; row < row1; ++row) {
-            T et[NS];
+            double et[NS];
             load_e(row, et);
             step(row, et);
             store_d(row);
@@ -426,9 +424,6 @@ viterbi_lean_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
 // lane's e; the from-state-0 correction goes to the first candidate of the lanes of group h = 0, which hold
 // from-state 0 for their four to-states.
 #define VW_PAIRS 8
-#ifndef VW_ENABLED
-#define VW_ENABLED 1
-#endif
 template <bool RATIO>
 __global__ void __launch_bounds__(VW_PAIRS * 64, 1)
 viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ elog,
@@ -604,43 +599,30 @@ viterbi_wide_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ 
     }
 }
 
-// order-preserving key of a float for REDUX (larger value -> larger key)
-__device__ __forceinline__ unsigned order_key(float v)
-{
-    const unsigned bts = __float_as_uint(v);
-    return bts ^ ((unsigned)((int)bts >> 31) | 0x80000000u);
-}
-
 // lowest state index among the maxima of a warp-distributed vector
-template <typename T, int NS>
-__device__ __forceinline__ int warp_argmax_first(const T (&v)[NS], int lane)
+template <int NS>
+__device__ __forceinline__ int warp_argmax_first(const double (&v)[NS], int lane)
 {
-    if constexpr (sizeof(T) == 4 && NS == 1) {
-        const unsigned key = order_key((float)v[0]);
-        const unsigned mx = __reduce_max_sync(TEHMM_FULL, key);
-        return __ffs(__ballot_sync(TEHMM_FULL, key == mx)) - 1;
-    } else {
-        T best = v[0];
-        int arg = lane;
+    double best = v[0];
+    int arg = lane;
 #pragma unroll
-        for (int s = 1; s < NS; ++s)
-            if (v[s] > best) { best = v[s]; arg = lane + 32 * s; }
+    for (int s = 1; s < NS; ++s)
+        if (v[s] > best) { best = v[s]; arg = lane + 32 * s; }
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const T ob = __shfl_xor_sync(TEHMM_FULL, best, o);
-            const int oa = __shfl_xor_sync(TEHMM_FULL, arg, o);
-            if (ob > best || (ob == best && oa < arg)) { best = ob; arg = oa; }
-        }
-        return arg;
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ob = __shfl_xor_sync(TEHMM_FULL, best, o);
+        const int oa = __shfl_xor_sync(TEHMM_FULL, arg, o);
+        if (ob > best || (ob == best && oa < arg)) { best = ob; arg = oa; }
     }
+    return arg;
 }
 
 // One warp per chunk.  mode 0: speculate the chunk's end state, walk the chunk,
 // record the state it implies for the left neighbour (pred).  mode 1: redo the
 // chunks whose end state was wrong, from the forced end state.
-template <typename T, int NS, bool RATIO>
-__global__ void __launch_bounds__(TEHMM_WARPS_PER_CTA * 32, (sizeof(T) == 4 && NS == 1) ? 5 : 1)
-vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lattice,
+template <int NS, bool RATIO>
+__global__ void __launch_bounds__(TEHMM_WARPS_PER_CTA * 32, 1)
+vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const double *__restrict__ lattice,
                      const double *__restrict__ ratios, uint8_t *__restrict__ states,
                      int64_t *__restrict__ states64, uint8_t *__restrict__ spec_end,
                      uint8_t *__restrict__ pred, const uint8_t *__restrict__ forced_end,
@@ -648,17 +630,17 @@ vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lat
 {
     constexpr int NP = 32 * NS;
     extern __shared__ __align__(16) unsigned char tb_smem[];
-    T *AT = reinterpret_cast<T *>(tb_smem);               // AT[s*NP + i] = logA[i][s]
+    double *AT = reinterpret_cast<double *>(tb_smem);               // AT[s*NP + i] = logA[i][s]
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int N = m.N;
     const unsigned Nu = (unsigned)m.LD;      // lattice row stride
-    const T NEG = (T)-INFINITY;
+    const double NEG = -INFINITY;
     for (int e = threadIdx.x; e < NP * NP; e += blockDim.x) {
         const int s = e / NP, i = e - s * NP;
-        AT[e] = (T)m.cut_trans[(int64_t)i * NP + s];
+        AT[e] = m.cut_trans[(int64_t)i * NP + s];
     }
     __syncthreads();
-    const T a00 = (T)m.cut_trans[0];
+    const double a00 = m.cut_trans[0];
     unsigned jc[NS];
     bool own[NS];
 #pragma unroll
@@ -673,35 +655,35 @@ vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lat
         const TehmmChunk ch = b.chunks[ci];
         // rows relative to t0 - 1 (row 0 = the left neighbour's last step, if any)
         const int64_t tbase = ch.t0 > ch.s0 ? ch.t0 - 1 : ch.t0;
-        const T *__restrict__ ll = lattice + tbase * m.LD;
+        const double *__restrict__ ll = lattice + tbase * m.LD;
         const double *__restrict__ rr = RATIO ? ratios + tbase : nullptr;
         const unsigned rfirst = (unsigned)(ch.t0 - tbase);            // row of t0 (0 or 1)
         const unsigned rlast = (unsigned)(ch.t1 - 1 - tbase);         // row of t1-1
 
-        auto load_d = [&](unsigned row, T (&dv)[NS]) {
+        auto load_d = [&](unsigned row, double (&dv)[NS]) {
 #pragma unroll
             for (int s = 0; s < NS; ++s) {
-                const T v = ll[row * Nu + jc[s]];
+                const double v = ll[row * Nu + jc[s]];
                 dv[s] = own[s] ? v : NEG;
             }
         };
         // state at row-1 given state st at `row`, from delta[row-1] (already loaded)
-        auto back = [&](unsigned row, int st, const T (&dprev)[NS]) -> int {
-            T cand[NS];
+        auto back = [&](unsigned row, int st, const double (&dprev)[NS]) -> int {
+            double cand[NS];
 #pragma unroll
             for (int s = 0; s < NS; ++s) cand[s] = dprev[s] + AT[st * NP + lane + 32 * s];
             if (RATIO) {
                 // only the from-state-0 candidate differs between from-states (see viterbi_kernel)
-                const T r = (T)rr[row];
-                if (lane == 0 && r >= (T)0) {           // negative: a sequence without ratios
-                    const T dgs = AT[st * NP + st];
-                    const T common = r > (T)1 ? dgs * (r - (T)1) : (T)0;
-                    T extra0 = dgs > NEG ? dgs * r - common : (T)0;
+                const double r = rr[row];
+                if (lane == 0 && r >= 0.0) {           // negative: a sequence without ratios
+                    const double dgs = AT[st * NP + st];
+                    const double common = r > 1.0 ? dgs * (r - 1.0) : 0.0;
+                    double extra0 = dgs > NEG ? dgs * r - common : 0.0;
                     if (st == 0 && a00 > NEG) extra0 -= a00;
                     cand[0] += extra0;
                 }
             }
-            return warp_argmax_first<T, NS>(cand, lane);
+            return warp_argmax_first<NS>(cand, lane);
         };
 
         // Walk rows hi, hi-1, ..., lo+1 (state at `hi` known), calling emit(row, st)
@@ -718,11 +700,11 @@ vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lat
             // full groups of TB_PF rows, unconditional so the ring stays in registers:
             // cur[q] = delta[row-1-q]; the next group's rows are in flight meanwhile
             if (row >= lo + 2 * TB_PF) {
-                T nxt[TB_PF][NS];
+                double nxt[TB_PF][NS];
 #pragma unroll
                 for (int q = 0; q < TB_PF; ++q) load_d(row - 1 - (unsigned)q, nxt[q]);
                 while (row >= lo + 2 * TB_PF) {
-                    T cur[TB_PF][NS];
+                    double cur[TB_PF][NS];
 #pragma unroll
                     for (int q = 0; q < TB_PF; ++q) {
 #pragma unroll
@@ -746,7 +728,7 @@ vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lat
                 row -= TB_PF;
             }
             for (; row > lo; --row) {
-                T dc[NS];
+                double dc[NS];
                 load_d(row - 1, dc);
                 emit(row, st);
                 st = back(row, st, dc);
@@ -758,17 +740,17 @@ vit_traceback_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lat
         if (mode == 1) {
             st = forced_end[ci];
         } else if (ch.t1 == ch.s1) {
-            T dv[NS];
+            double dv[NS];
             load_d(rlast, dv);
-            st = warp_argmax_first<T, NS>(dv, lane);        // np.argmax of the last row
+            st = warp_argmax_first<NS>(dv, lane);        // np.argmax of the last row
         } else {
             // speculate: enter from `warmup` steps to the right (or the sequence end)
             unsigned rq = rlast + (unsigned)b.warmup;
             const unsigned rseq = (unsigned)(ch.s1 - 1 - tbase);
             if (rq > rseq) rq = rseq;
-            T dv[NS];
+            double dv[NS];
             load_d(rq, dv);
-            st = warp_argmax_first<T, NS>(dv, lane);
+            st = warp_argmax_first<NS>(dv, lane);
             st = walk(rq, rlast, st, false);
         }
         if (lane == 0) spec_end[ci] = (uint8_t)st;
@@ -990,27 +972,22 @@ __global__ void vit_score_reduce_kernel(TehmmBatchDev b, const double *__restric
     if (threadIdx.x == 0) logprob[s] = acc;
 }
 
-template <typename T, int NS>
+template <int NS>
 static cudaError_t launch_vit(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
-                              const T *elog, const double *ratios, T *lattice, T *start_vec,
-                              T *end_vec, const int *bad, int mode, int grid)
+                              const double *elog, const double *ratios, double *lattice, double *start_vec,
+                              double *end_vec, const int *bad, int mode, int grid)
 {
     if (ratios)
-        viterbi_kernel<T, NS, true><<<grid, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, elog, ratios, lattice, start_vec, end_vec, bad, mode);
-    else if (sizeof(T) == 4 && NS == 2) {
-        // one CTA per SM either way (the transition matrix alone is 128 registers per lane): twelve warps at <= 168 registers
-        const int64_t need = (b.nchunks + VIT_WIDE_WARPS - 1) / VIT_WIDE_WARPS;
-        const int g = (int)(need < grid ? need : grid);
-        viterbi_kernel<T, NS, false, VIT_WIDE_WARPS><<<g, VIT_WIDE_WARPS * 32, 0, st>>>(m, b, elog, ratios, lattice, start_vec, end_vec, bad, mode);
-    } else
-        viterbi_kernel<T, NS, false><<<grid, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, elog, ratios, lattice, start_vec, end_vec, bad, mode);
+        viterbi_kernel<NS, true><<<grid, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, elog, ratios, lattice, start_vec, end_vec, bad, mode);
+    else
+        viterbi_kernel<NS, false><<<grid, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, elog, ratios, lattice, start_vec, end_vec, bad, mode);
     return cudaGetLastError();
 }
 
 // the DP that can return the log-probability itself (viterbi_lean_kernel's score_part)
 bool tehmm_viterbi_dp_scores(const TehmmModelDev &m, int prec, const double *ratios)
 {
-    return prec == TEHMM_F32 && m.NS == 1 && m.LD == 32 && !ratios;
+    return prec == TEHMM_F32 && m.NS == 1 && !ratios;
 }
 
 cudaError_t tehmm_launch_viterbi(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
@@ -1019,42 +996,38 @@ cudaError_t tehmm_launch_viterbi(cudaStream_t st, const TehmmModelDev &m, const 
                                  const double *rowmax, double *score_part)
 {
     if (prec == TEHMM_F32) {
-        if (m.NS == 1 && m.LD == 32) {
+        if (m.NS == 1) {
             if (ratios)
                 viterbi_lean_kernel<true><<<grid, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, nullptr, nullptr, ratios);
             else
                 viterbi_lean_kernel<false><<<grid, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, rowmax, rowmax ? score_part : nullptr, nullptr);
             return cudaGetLastError();
         }
-        if (m.NS == 1) return launch_vit<float, 1>(st, m, b, (const float *)elog, ratios, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, grid);
-        if (m.LD == 64 && VW_ENABLED) {
-            const int64_t need = (b.nchunks + VW_PAIRS - 1) / VW_PAIRS;
-            const int g = (int)(need < grid ? need : grid);
-            if (ratios)
-                viterbi_wide_kernel<true><<<g, VW_PAIRS * 64, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, ratios);
-            else
-                viterbi_wide_kernel<false><<<g, VW_PAIRS * 64, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, nullptr);
-            return cudaGetLastError();
-        }
-        return launch_vit<float, 2>(st, m, b, (const float *)elog, ratios, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, grid);
+        const int64_t need = (b.nchunks + VW_PAIRS - 1) / VW_PAIRS;
+        const int g = (int)(need < grid ? need : grid);
+        if (ratios)
+            viterbi_wide_kernel<true><<<g, VW_PAIRS * 64, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, ratios);
+        else
+            viterbi_wide_kernel<false><<<g, VW_PAIRS * 64, 0, st>>>(m, b, (const float *)elog, (float *)lattice, (float *)start_vec, (float *)end_vec, bad, mode, nullptr);
+        return cudaGetLastError();
     }
-    if (m.NS == 1) return launch_vit<double, 1>(st, m, b, (const double *)elog, ratios, (double *)lattice, (double *)start_vec, (double *)end_vec, bad, mode, grid);
-    return launch_vit<double, 2>(st, m, b, (const double *)elog, ratios, (double *)lattice, (double *)start_vec, (double *)end_vec, bad, mode, grid);
+    if (m.NS == 1) return launch_vit<1>(st, m, b, (const double *)elog, ratios, (double *)lattice, (double *)start_vec, (double *)end_vec, bad, mode, grid);
+    return launch_vit<2>(st, m, b, (const double *)elog, ratios, (double *)lattice, (double *)start_vec, (double *)end_vec, bad, mode, grid);
 }
 
-template <typename T, int NS>
+template <int NS>
 static cudaError_t launch_tb(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b,
-                             const T *lattice, const double *ratios, uint8_t *states,
+                             const double *lattice, const double *ratios, uint8_t *states,
                              int64_t *states64, uint8_t *spec_end, uint8_t *pred,
                              const uint8_t *forced_end, const int *bad, int mode, int grid)
 {
-    const size_t smem = (size_t)m.NP * m.NP * sizeof(T);
+    const size_t smem = (size_t)m.NP * m.NP * sizeof(double);
     if (ratios) {
-        auto k = vit_traceback_kernel<T, NS, true>;
+        auto k = vit_traceback_kernel<NS, true>;
         cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         k<<<grid, TEHMM_WARPS_PER_CTA * 32, smem, st>>>(m, b, lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode);
     } else {
-        auto k = vit_traceback_kernel<T, NS, false>;
+        auto k = vit_traceback_kernel<NS, false>;
         cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         k<<<grid, TEHMM_WARPS_PER_CTA * 32, smem, st>>>(m, b, lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode);
     }
@@ -1068,28 +1041,24 @@ cudaError_t tehmm_launch_traceback(cudaStream_t st, const TehmmModelDev &m, cons
                                    int mode, int grid)
 {
     if (prec == TEHMM_F32) {
-        if (m.LD == 32 * m.NS) {
-            const int cpw = m.NS == 1 ? 4 : 2;
-            const int64_t need = ((b.nchunks + cpw - 1) / cpw + TEHMM_WARPS_PER_CTA - 1) / TEHMM_WARPS_PER_CTA;
-            const int g4 = (int)(need < grid ? (need < 1 ? 1 : need) : grid);
-            if (m.NS == 1) {
-                if (ratios)
-                    vit_traceback4_kernel<true, 1><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, ratios);
-                else
-                    vit_traceback4_kernel<false, 1><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, nullptr);
-            } else {
-                if (ratios)
-                    vit_traceback4_kernel<true, 2><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, ratios);
-                else
-                    vit_traceback4_kernel<false, 2><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, nullptr);
-            }
-            return cudaGetLastError();
+        const int cpw = m.NS == 1 ? 4 : 2;
+        const int64_t need = ((b.nchunks + cpw - 1) / cpw + TEHMM_WARPS_PER_CTA - 1) / TEHMM_WARPS_PER_CTA;
+        const int g4 = (int)(need < grid ? (need < 1 ? 1 : need) : grid);
+        if (m.NS == 1) {
+            if (ratios)
+                vit_traceback4_kernel<true, 1><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, ratios);
+            else
+                vit_traceback4_kernel<false, 1><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, nullptr);
+        } else {
+            if (ratios)
+                vit_traceback4_kernel<true, 2><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, ratios);
+            else
+                vit_traceback4_kernel<false, 2><<<g4, TEHMM_WARPS_PER_CTA * 32, 0, st>>>(m, b, (const float *)lattice, states, states64, spec_end, pred, forced_end, bad, mode, nullptr);
         }
-        if (m.NS == 1) return launch_tb<float, 1>(st, m, b, (const float *)lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode, grid);
-        return launch_tb<float, 2>(st, m, b, (const float *)lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode, grid);
+        return cudaGetLastError();
     }
-    if (m.NS == 1) return launch_tb<double, 1>(st, m, b, (const double *)lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode, grid);
-    return launch_tb<double, 2>(st, m, b, (const double *)lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode, grid);
+    if (m.NS == 1) return launch_tb<1>(st, m, b, (const double *)lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode, grid);
+    return launch_tb<2>(st, m, b, (const double *)lattice, ratios, states, states64, spec_end, pred, forced_end, bad, mode, grid);
 }
 
 cudaError_t tehmm_launch_tb_verify(cudaStream_t st, const TehmmBatchDev &b, uint8_t *spec_end,

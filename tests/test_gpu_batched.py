@@ -349,7 +349,7 @@ def test_tile_and_warp_kernels_interoperate(oracle):
         assert_allclose(post, base[1], rtol=TOL["f32"], atol=ATOL["f32"])
 
 
-def test_xi_tensor_core_kernel_vs_scan_and_f64():
+def test_xi_tensor_core_kernel_vs_cuda_core_and_f64():
     """Expected transition counts: the tensor-core xi kernel (two dense products per 16 steps,
     csrc/tile.cu) against the one-chunk-per-warp accumulation it replaces and against the
     float64 verification mode, at a size where per-entry counts span six decades; and the
@@ -362,9 +362,9 @@ def test_xi_tensor_core_kernel_vs_scan_and_f64():
     eng.upload_model(m["log_start"], m["log_trans"], m["table"], 1.0, m["widths"])
     eng.upload_batch(obs)
     ref = eng.estep(precision="f64")
-    eng.ctx.set_option("xi_tile", 0)
+    eng.ctx.set_option("tile", 0)
     scan = eng.estep(precision="f32")
-    eng.ctx.set_option("xi_tile", 1)
+    eng.ctx.set_option("tile", 1)
     before = eng.ctx.stat("launches")
     tile = eng.estep(precision="f32")
     assert eng.ctx.stat("launches") > before
@@ -392,8 +392,9 @@ def test_forward_tensor_map_blocks_single_sequence(oracle, fine_len, warmup):
     eng = engine(fine_len=fine_len, warmup=warmup, tile=1)
     eng.upload_model(m["log_start"], m["log_trans"], m["table"], 1.0, m["widths"])
     eng.upload_batch([obs])
+    before = eng.ctx.stat("tile_passes")
     out = eng.posteriors(renorm_eps=False, want_map=True, precision="f32")
-    assert eng.ctx.stat("tile_passes") > 0
+    assert eng.ctx.stat("tile_passes") > before
     assert out["logprob"][0] == pytest.approx(ref["logprob"], rel=TOL["f32"])
     assert_allclose(out["post"][0], ref["post"], rtol=TOL["f32"], atol=ATOL["f32"])
     eng2 = engine(fine_len=fine_len, warmup=warmup, tile=0)
@@ -404,32 +405,22 @@ def test_forward_tensor_map_blocks_single_sequence(oracle, fine_len, warmup):
 
 
 @pytest.mark.parametrize("fine_len,warmup", [(0, 0), (96, 64), (200, 32), (64, 64), (66, 2), (128, 126)])
-def test_backward_tensor_map_blocks_single_sequence(oracle, fine_len, warmup):
-    """bwd_tile_tmap_kernel (context option "bwd_tmap", off by default): the regular tiles of ONE regularly chunked sequence get their
-    b_{t+1} / alpha_t rows as tensor-map boxes (the b map starts one row in); ragged tiles, the
-    sequence end and warm-ups that do not fit a chunk stay with bwd_tile_kernel.  Same arithmetic:
-    posteriors, MAP path and score must be BIT-identical to the per-lane-copy kernel, and agree
-    with the oracle (basehmm.py:265-272,332-359)."""
+def test_backward_tile_kernel_single_sequence(oracle, fine_len, warmup):
+    """bwd_tile_kernel on ONE regularly chunked sequence whose forward pass took the tensor-map
+    blocks: regular and ragged tiles, the sequence end and warm-ups that do not fit a chunk.
+    Posteriors against the oracle (basehmm.py:265-272,332-359)."""
     from tehmm_b200 import synth
     m = synth.make_model(N=30, seed=23)
     T = 70_011
     obs, _ = synth.sample_obs(m, T, seed=24)
     ref = oracle_all(oracle, obs, m["table"], 1.0, m["log_start"], m["log_trans"])
-    res = {}
-    for tm in (1, 0):
-        eng = engine(fine_len=fine_len, warmup=warmup, tile=1)
-        eng.ctx.set_option("bwd_tmap", tm)
-        eng.upload_model(m["log_start"], m["log_trans"], m["table"], 1.0, m["widths"])
-        eng.upload_batch([obs])
-        res[tm] = (eng.posteriors(renorm_eps=False, want_map=True, precision="f32"),
-                   eng.posteriors(renorm_eps=True, want_map=True, want_post=False, precision="f32"))
-    engine().ctx.set_option("bwd_tmap", 0)
-    for a, b in zip(res[1], res[0]):
-        assert_array_equal(a["map_states"][0], b["map_states"][0])
-        assert a["map_score"][0] == b["map_score"][0]
-        assert a["logprob"][0] == b["logprob"][0]
-    assert_array_equal(res[1][0]["post"][0], res[0][0]["post"][0])
-    assert_allclose(res[1][0]["post"][0], ref["post"], rtol=TOL["f32"], atol=ATOL["f32"])
+    eng = engine(fine_len=fine_len, warmup=warmup, tile=1)
+    eng.upload_model(m["log_start"], m["log_trans"], m["table"], 1.0, m["widths"])
+    eng.upload_batch([obs])
+    before = eng.ctx.stat("tile_passes")
+    out = eng.posteriors(renorm_eps=False, want_map=True, precision="f32")
+    assert eng.ctx.stat("tile_passes") > before
+    assert_allclose(out["post"][0], ref["post"], rtol=TOL["f32"], atol=ATOL["f32"])
 
 
 def test_full_size_c2_properties(oracle):
@@ -488,37 +479,9 @@ def test_full_size_c2_properties(oracle):
     assert np.mean(out["map_states"][0][:150_000] == ref["map_states"][:150_000]) > 0.9999
 
 
-@pytest.mark.parametrize("threads_per_chunk", [1, 2])
-def test_forward_tcgen05_kernel_matches(oracle, threads_per_chunk):
-    """csrc/umma.cu (context option "umma" = threads per chunk): the forward pass of a single-sequence batch on
-    tcgen05.mma with accumulator and state in tensor memory, b / alpha rows as swizzled 3-D
-    tensor-map boxes.  Same log-likelihood, posteriors and MAP path as the oracle and as the
-    mma.sync kernel, including a ragged last chunk handled outside the boxes."""
-    from tehmm_b200 import synth
-    m = synth.make_model(N=30, seed=31)
-    T = 150_007
-    obs, _ = synth.sample_obs(m, T, seed=32)
-    ref = oracle_all(oracle, obs, m["table"], 1.0, m["log_start"], m["log_trans"])
-    eng = engine(fine_len=200)
-    eng.upload_model(m["log_start"], m["log_trans"], m["table"], 1.0, m["widths"])
-    eng.upload_batch([obs])
-    base = eng.posteriors(renorm_eps=False, want_map=True, precision="f32")
-    before = eng.ctx.stat("umma_passes")
-    eng.ctx.set_option("umma", threads_per_chunk)
-    try:
-        out = eng.posteriors(renorm_eps=False, want_map=True, precision="f32")
-    finally:
-        eng.ctx.set_option("umma", 0)
-    assert eng.ctx.stat("umma_passes") >= before + 1
-    assert out["logprob"][0] == pytest.approx(ref["logprob"], rel=TOL["f32"])
-    assert_allclose(out["post"][0], ref["post"], rtol=TOL["f32"], atol=ATOL["f32"])
-    assert out["logprob"][0] == pytest.approx(base["logprob"][0], rel=1e-7)
-    assert np.mean(out["map_states"][0] == base["map_states"][0]) > 0.9999
-
-
 @pytest.mark.parametrize("N,T", [(33, 60_011), (50, 60_000), (50, 60_100), (64, 45_020)])
-def test_tcgen05_kernels_are_the_default_for_33_to_64_states(oracle, N, T):
-    """fwd_umma_kernel<2> and its backward twin bwd_umma_kernel<2> (csrc/umma.cu; option "umma64", default on):
+def test_tcgen05_kernels_vs_cuda_core_for_33_to_64_states(oracle, N, T):
+    """fwd_umma_kernel and its backward twin bwd_umma_kernel (csrc/umma.cu; default unless option "tile" is 0):
     the forward pass and the backward / posterior / MAP pass of a single-sequence batch of 33..64 states on
     tcgen05.mma M128 N64 K8 with two threads per chunk.  Same log-likelihood, posteriors and MAP path as the
     oracle and as the one-chunk-per-warp kernels -- with no ragged last chunk (60 000 = 400 x 150), one shorter
@@ -536,12 +499,12 @@ def test_tcgen05_kernels_are_the_default_for_33_to_64_states(oracle, N, T):
     only_map = eng.posteriors(renorm_eps=False, want_post=False, want_map=True, precision="f32")
     assert eng.ctx.stat("umma_passes") == before + 4
     eps = eng.posteriors(renorm_eps=True, want_map=True, precision="f32")
-    eng.ctx.set_option("umma64", 0)
+    eng.ctx.set_option("tile", 0)
     try:
         base = eng.posteriors(renorm_eps=False, want_map=True, precision="f32")
         base_eps = eng.posteriors(renorm_eps=True, want_map=True, precision="f32")
     finally:
-        eng.ctx.set_option("umma64", 1)
+        eng.ctx.set_option("tile", 1)
     assert eng.ctx.stat("umma_passes") == before + 6
     assert eng.ctx.stat("repair_passes_backward") == repairs
     assert out["logprob"][0] == pytest.approx(ref["logprob"], rel=TOL["f32"])
@@ -560,9 +523,9 @@ def test_tcgen05_kernels_are_the_default_for_33_to_64_states(oracle, N, T):
     assert eng.ctx.stat("umma_passes") == before + 6
 
 
-def test_tcgen05_kernels_several_tiles_per_cta():
-    """More tiles of 128 chunks than SMs (1.3 M steps in chunks of 64: 159 tiles): a CTA of fwd_umma_kernel<2> /
-    bwd_umma_kernel<2> walks a second tile with the same barriers, tensor-memory columns and shared-memory rings.
+def test_tcgen05_kernels_several_tiles_per_cta_vs_cuda_core():
+    """More tiles of 128 chunks than SMs (1.3 M steps in chunks of 64: 159 tiles): a CTA of fwd_umma_kernel /
+    bwd_umma_kernel walks a second tile with the same barriers, tensor-memory columns and shared-memory rings.
     Against the one-chunk-per-warp kernels on the same partition."""
     from tehmm_b200 import synth
     m = synth.make_model(N=50, seed=43)
@@ -574,11 +537,11 @@ def test_tcgen05_kernels_several_tiles_per_cta():
     before = eng.ctx.stat("umma_passes")
     out = eng.posteriors(renorm_eps=False, want_post=True, want_map=True, precision="f32")
     assert eng.ctx.stat("umma_passes") == before + 2
-    eng.ctx.set_option("umma64", 0)
+    eng.ctx.set_option("tile", 0)
     try:
         base = eng.posteriors(renorm_eps=False, want_post=True, want_map=True, precision="f32")
     finally:
-        eng.ctx.set_option("umma64", 1)
+        eng.ctx.set_option("tile", 1)
     assert out["logprob"][0] == pytest.approx(base["logprob"][0], rel=1e-7)
     assert np.mean(out["map_states"][0] == base["map_states"][0]) > 0.99999
     assert_allclose(out["map_score"], base["map_score"], rtol=1e-6)

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""33..64 states, one sequence: forward pass by the tcgen05 kernel (option umma64, default) against the
-one-chunk-per-warp kernel; log-likelihoods must agree."""
+"""33..64 states, one sequence: forward pass by the tcgen05 kernel (default) against the one-chunk-per-warp
+kernel (option "tile" = 0); log-likelihoods must agree."""
 import json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -26,7 +26,7 @@ for N in (50, 64, 33):
     res = {}
     bres = {}
     for opt in (1, 0):
-        ctx.set_option("umma64", opt)
+        ctx.set_option("tile", opt)
         for _ in range(2):
             alpha, lp = ctx.optimistic(lambda: eng.run_forward(prec, tdt, blin, rowmax, None))
         torch.cuda.synchronize()
@@ -43,7 +43,7 @@ for N in (50, 64, 33):
             bres.setdefault(opt, {})[fl] = (ctx.stat("us_backward"), outs[1].cpu().numpy() if outs[1] is not None else None)
             del outs
         ctx.set_option("timing", 0)
-    ctx.set_option("umma64", 1)
+    ctx.set_option("tile", 1)
     elog, _, rm = eng.run_emission(prec, tdt, None, True, False)
     for _ in range(2):
         vs = ctx.optimistic(lambda: eng.run_viterbi(prec, elog, None, None, want64=False, rowmax=rm))
