@@ -98,13 +98,13 @@ int64_t tehmm_ctx_launch_count(tehmm_ctx *ctx);
  * posterior / MAP kernels of csrc/umma.cu for the first pass over a single-sequence batch
  * of 33..64 states; stats "tile_passes" and "umma_passes" count their launches),
  * "fine_len" (steps per chunk of the fine partition, 0 = auto), "timing" (1 = bracket the first
- * launch of each main kernel with CUDA events on the context's stream), "defer" (see
- * tehmm_ctx_check),
+ * launch of each main kernel with CUDA events on the context's stream), "defer" and
+ * "defer_skip" (see tehmm_ctx_check),
  * "fallback_after" (ordinary repair passes before the chunks still flagged are resolved exactly by
  * transfer operators and a float64 chain, csrc/fallback.cu; default 2, -1 = never: the plain loop, one
  * pass per link of a chain of failed boundaries; stats "fallbacks", "fallback_chunks", "mix_rho_ppm").
  * stats: "launches", "chunks", "fine_chunks", "repaired_chunks_<pass>",
- * "repair_passes_<pass>", "tile_passes", and with "timing" the mean duration in
+ * "repair_passes_<pass>", "tile_passes", "defer_skip", and with "timing" the mean duration in
  * microseconds (over the launches since "timing" was set, at most 32) of "us_emission", "us_forward", "us_backward",
  * "us_viterbi_dp", "us_traceback", "us_rescore", "us_emission_stats", "us_xi" launch
  * (blocks until that launch has finished; -1 if it never ran). */
@@ -117,7 +117,13 @@ int64_t tehmm_ctx_get_stat(tehmm_ctx *ctx, const char *name);
  * call carries on as if nothing had to be repaired.  tehmm_ctx_check waits for the stream
  * and returns in *unverified the number of failed boundaries since the last check: 0 =
  * every result stands (the common case); > 0 = recompute those results with "defer" = 0
- * (tehmm_decode_host does both steps itself).  Stats: "deferred_checks", "deferred_bad". */
+ * (tehmm_decode_host does both steps itself).  Stats: "deferred_checks", "deferred_bad".
+ * Back-off: a refused check (something was deferred and a boundary failed) sets the
+ * context's penalty to min(256, max(4, 2 x penalty)) and its countdown "defer_skip" to the
+ * penalty; a check that stands halves the penalty.  While "defer_skip" > 0, setting "defer"
+ * to 1 leaves it off and counts one call down: a refused attempt costs its stages twice,
+ * and a model / batch that needed repairs tends to need them again.  "defer_skip" is also
+ * an option, to reset the countdown. */
 int tehmm_ctx_check(tehmm_ctx *ctx, int64_t *unverified);
 
 /* ------------------------------------------------------------------ L0 strict
@@ -414,8 +420,7 @@ int tehmm_states_to_bed(int fd, const char *chrom, int64_t start, const int64_t 
 int tehmm_scores_to_bed(int fd, const char *chrom, int64_t start, const double *scores,
                         int64_t n, const int64_t *seg_len, const int32_t *mask_off, int64_t mask_n);
 
-/* widen / convert on the device before a D2H copy */
-int tehmm_widen_states(tehmm_ctx *ctx, const uint8_t *d_in, int64_t *d_out, int64_t n);
+/* convert on the device before a D2H copy */
 int tehmm_convert_lattice(tehmm_ctx *ctx, int prec, const void *d_in, double *d_out, int64_t n);
 
 #ifdef __cplusplus

@@ -87,7 +87,6 @@ SIGNATURES = {
     "tehmm_path_score": (_c_int, [_c_void, _c_void, _c_void, _c_void, _c_i64, _c_i64, _c_void, _c_void]),
     "tehmm_states_to_bed": (_c_int, [_c_int, ctypes.c_char_p, _c_i64, _c_void, _c_i64, _c_void, _c_void, _c_i64, _c_void, _c_int]),
     "tehmm_scores_to_bed": (_c_int, [_c_int, ctypes.c_char_p, _c_i64, _c_void, _c_i64, _c_void, _c_void, _c_i64]),
-    "tehmm_widen_states": (_c_int, [_c_void, _c_void, _c_void, _c_i64]),
     "tehmm_convert_lattice": (_c_int, [_c_void, _c_int, _c_void, _c_void, _c_i64]),
 }
 
@@ -181,28 +180,17 @@ class Context(object):
     def optimistic(self, fn):
         """run fn() with deferred verification; if any boundary failed, run it again with the
         synchronous verify / repair loop.  fn must be a pure function of device state it does
-        not overwrite (every engine pass is)."""
-        # a refused attempt costs the stages twice, and batches that need repairs tend to need them
-        # again (same model, same chunk boundaries): back off to the synchronous loop for a growing
-        # number of calls after a refusal, come back when attempts stand again
-        skip = getattr(self, "_defer_skip", 0)
+        not overwrite (every engine pass is).  After a refusal the library leaves "defer" off for
+        a growing number of calls (stat "defer_skip"; tehmm_ctx_check)."""
         if os.environ.get("TEHMM_NO_DEFER"):      # measurement switch: always the synchronous loop
-            return fn()
-        if skip > 0:
-            self._defer_skip = skip - 1
             return fn()
         self.set_option("defer", 1)
         try:
             out = fn()
         finally:
             self.set_option("defer", 0)
-        penalty = getattr(self, "_defer_penalty", 0)
         if self.check() != 0:
-            self._defer_penalty = min(256, max(4, 2 * penalty))
-            self._defer_skip = self._defer_penalty
             out = fn()
-        else:
-            self._defer_penalty = penalty // 2
         return out
 
     @property

@@ -36,7 +36,6 @@ cudaError_t tehmm_launch_tb_verify(cudaStream_t, const TehmmBatchDev &, uint8_t 
 cudaError_t tehmm_launch_rescore(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, const uint8_t *, const double *, const double *, double *, double *, int64_t, int64_t);
 cudaError_t tehmm_launch_emission_stats(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const void *, const double *, double *, double *, int, int);
 size_t tehmm_stats_smem_bytes(int tab_rows, int N, int K, int prec);
-cudaError_t tehmm_launch_widen(cudaStream_t, const uint8_t *, int64_t *, int64_t);
 cudaError_t tehmm_launch_forward_tile(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, const float *, const double *, float *, float *, float *, double *, const int *, int, int, int64_t);
 cudaError_t tehmm_launch_backward_tile(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const float *, const float *, float *, uint8_t *, double *, float *, float *, const int *, int, int);
 int tehmm_tile_warps(void);
@@ -122,6 +121,7 @@ struct tehmm_ctx {
     int64_t opt_defer = 0;
     int *h_pending = nullptr;         // pinned, TEHMM_NPENDING slots
     int npending = 0;
+    int64_t defer_skip = 0, defer_penalty = 0;   // back-off after a refused check (tehmm_ctx_check)
     int64_t stat_deferred_checks = 0, stat_deferred_bad = 0;
     // model
     bool has_model = false;
@@ -227,7 +227,11 @@ int tehmm_ctx_set_option(tehmm_ctx *c, const char *name, int64_t v)
     else if (!strcmp(name, "tile")) c->opt_tile = v;
     else if (!strcmp(name, "timing")) { c->opt_timing = v; for (int i = 0; i < TEHMM_NTIMED; ++i) c->ev_n[i] = 0; }
     else if (!strcmp(name, "fine_len")) c->opt_fine_len = v;
-    else if (!strcmp(name, "defer")) c->opt_defer = v;
+    else if (!strcmp(name, "defer")) {
+        if (v && c->defer_skip > 0) { c->defer_skip -= 1; v = 0; }
+        c->opt_defer = v;
+    }
+    else if (!strcmp(name, "defer_skip")) c->defer_skip = v;
     else if (!strcmp(name, "rescore")) c->opt_rescore = v;
     else if (!strcmp(name, "fallback_after")) c->opt_fallback_after = v;
     else return fail(TEHMM_EINVAL, "unknown option %s", name);
@@ -288,6 +292,7 @@ int64_t tehmm_ctx_get_stat(tehmm_ctx *c, const char *name)
     if (!strcmp(name, "sms")) return c->sms;
     if (!strcmp(name, "deferred_checks")) return c->stat_deferred_checks;
     if (!strcmp(name, "deferred_bad")) return c->stat_deferred_bad;
+    if (!strcmp(name, "defer_skip")) return c->defer_skip;
     if (!strcmp(name, "chunks")) return c->has_batch ? c->b.nchunks : 0;
     if (!strcmp(name, "fine_chunks")) return c->has_batch ? c->bf.nchunks : 0;
     if (!strcmp(name, "tile_passes")) return c->stat_tile_passes;
@@ -953,6 +958,10 @@ static int read_nbad(tehmm_ctx *c, const int *d_nbad, int *out, bool may_defer =
 // number of chunks whose speculated boundary failed verification in any pass run since the last
 // check.  0: every result produced since then stands.  > 0: those results must be recomputed
 // with the option off (the synchronous verify / repair loop); nothing else is invalidated.
+// When something was deferred, the check also moves the context's back-off: a refusal doubles the
+// penalty (4 .. 256) and leaves "defer" off for that many requests (set_option counts "defer_skip"
+// down), a check that stands halves it -- a refused attempt costs its stages twice, and a model /
+// batch that needed repairs tends to need them again.
 int tehmm_ctx_check(tehmm_ctx *c, int64_t *unverified)
 {
     if (!c || !unverified) return fail(TEHMM_EINVAL, "NULL argument");
@@ -960,6 +969,12 @@ int tehmm_ctx_check(tehmm_ctx *c, int64_t *unverified)
     CU(cudaStreamSynchronize(c->stream));
     int64_t n = 0;
     for (int i = 0; i < c->npending; ++i) n += c->h_pending[i];
+    if (n > 0) {
+        c->defer_penalty = std::min<int64_t>(256, std::max<int64_t>(4, 2 * c->defer_penalty));
+        c->defer_skip = c->defer_penalty;
+    } else if (c->npending > 0) {
+        c->defer_penalty /= 2;
+    }
     c->stat_deferred_checks += c->npending;
     c->stat_deferred_bad += n;
     c->npending = 0;
@@ -1475,16 +1490,6 @@ int tehmm_path_score(tehmm_ctx *c, const uint8_t *d_states, const double *d_rati
     return TEHMM_OK;
 }
 
-int tehmm_widen_states(tehmm_ctx *c, const uint8_t *d_in, int64_t *d_out, int64_t n)
-{
-    if (!c || !d_in || !d_out || n < 0) return fail(TEHMM_EINVAL, "bad argument");
-    CU(cudaSetDevice(c->device));
-    if (n == 0) return TEHMM_OK;
-    CU(tehmm_launch_widen(c->stream, d_in, d_out, n));
-    c->launches += 1;
-    return TEHMM_OK;
-}
-
 int tehmm_convert_lattice(tehmm_ctx *c, int prec, const void *d_in, double *d_out, int64_t n)
 {
     if (!c || !d_in || !d_out || n < 0) return fail(TEHMM_EINVAL, "bad argument");
@@ -1498,22 +1503,11 @@ int tehmm_convert_lattice(tehmm_ctx *c, int prec, const void *d_in, double *d_ou
 }   // extern "C"
 
 // ---------------------------------------------------------------- tiny utility kernels
-__global__ void widen_kernel(const uint8_t *__restrict__ in, int64_t *__restrict__ out, int64_t n)
-{
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        out[i] = in[i];
-}
 template <typename T>
 __global__ void convert_kernel(const T *__restrict__ in, double *__restrict__ out, int64_t n)
 {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         out[i] = (double)in[i];
-}
-cudaError_t tehmm_launch_widen(cudaStream_t st, const uint8_t *in, int64_t *out, int64_t n)
-{
-    int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 16);
-    widen_kernel<<<grid, 256, 0, st>>>(in, out, n);
-    return cudaGetLastError();
 }
 cudaError_t tehmm_launch_convert(cudaStream_t st, int prec, const void *in, double *out, int64_t n)
 {

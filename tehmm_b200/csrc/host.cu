@@ -159,8 +159,6 @@ struct HostPipe {
     size_t pin_out_bytes = 0;
     Pool *pool = nullptr;
     int64_t h2d_bytes = 0, d2h_bytes = 0;
-    int64_t redone = 0;                     // calls whose deferred verification failed and ran twice
-    int defer_skip = 0, defer_penalty = 0;  // back-off after a refusal
     double phase_ms[4] = {-1, -1, -1, -1};  // last traced call: set_batch, h2d+emission, trellis, d2h+widen (TEHMM_HOST_TRACE)
 
     ~HostPipe()
@@ -257,6 +255,297 @@ struct Trace {
     ~Trace() { if (print) fprintf(stderr, "[tehmm_decode_host ms]%s\n", line.c_str()); }
 };
 
+// The pinned staging slice of upload slot `slot` (ring entry r): allocated on first use, and free once the copy
+// out of it is done.  The caller records ring_ev[r] behind its next copy out of the slice and sets ring_used[r].
+int ring_slot(HostPipe *p, int64_t slot, unsigned char **slice)
+{
+    const int r = (int)(slot % NRING);
+    if (!p->ring[r]) {
+        HCU(cudaMallocHost((void **)&p->ring[r], SLICE));
+        HCU(cudaEventCreateWithFlags(&p->ring_ev[r], cudaEventDisableTiming));
+    }
+    if (p->ring_used[r]) HCU(cudaEventSynchronize(p->ring_ev[r]));
+    *slice = p->ring[r];
+    return TEHMM_OK;
+}
+
+// Event i of the per-slice events, created on first use and kept for later calls.
+int slice_event(HostPipe *p, size_t i, cudaEvent_t *ev)
+{
+    while (p->slice_ev.size() <= i) {
+        cudaEvent_t e;
+        HCU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        p->slice_ev.push_back(e);
+    }
+    *ev = p->slice_ev[i];
+    return TEHMM_OK;
+}
+
+// One tehmm_decode_host* call, stage by stage.
+struct Decode {
+    tehmm_ctx *c;
+    HostPipe *p;
+    cudaStream_t st;                // the context's (compute) stream
+    int prec;
+    bool viterbi, both;             // algorithm TEHMM_DECODE_VITERBI / TEHMM_DECODE_BOTH (neither: MAP)
+    int64_t nseq, total;
+    const int64_t *h_offsets;
+    // arena layout: obs | states | [states 2] | logprob, score | rowmax | lattice A | lattice B | [lattice C] | [ratios] | scratch
+    size_t o_obs = 0, o_states = 0, o_states2 = 0, o_lp = 0, o_rowmax = 0, o_la = 0, o_lb = 0, o_lc = 0, o_rat = 0, o_scratch = 0;
+    char *A = nullptr;              // the arena
+    void *em_log = nullptr, *em_lin = nullptr;   // emission lattices: log for the Viterbi DP, linear for forward / backward
+    const double *d_rat = nullptr;  // segment ratios on the device, or NULL
+    bool piecewise = false;         // the emission runs slice by slice behind the upload
+    int64_t slot = 0;               // upload slots used so far
+
+    // ---- set-up: the arena layout, grown if needed, and the batch described to the library
+    int setup_arena(int K, int obs_bytes, bool use_ratios)
+    {
+        const size_t lat = (size_t)total * tehmm_lattice_stride(c) * (prec == TEHMM_F32 ? 4 : 8);
+        size_t o = 0;
+        o_obs = o; o = up256(o + (size_t)total * K * obs_bytes);
+        o_states = o; o = up256(o + (size_t)total);
+        o_states2 = o; if (both) o = up256(o + (size_t)total);
+        o_lp = o; o = up256(o + (size_t)nseq * 32);        // [first logprob | score | second logprob] x nseq
+        o_rowmax = o; o = up256(o + (size_t)total * 8);
+        o_la = o; o = up256(o + lat);
+        o_lb = o; o = up256(o + lat);
+        o_lc = o; if (both) o = up256(o + lat);          // BOTH: A = log emission, C = linear emission, B = alpha, then delta
+        o_rat = o; if (use_ratios) o = up256(o + (size_t)total * 8);
+        o_scratch = o;
+        // the scratch size depends on the partition: describe the batch first, with the obs pointer
+        // the arena will have (the arena may have to grow before anything is enqueued)
+        auto ensure = [&](size_t need) -> int {
+            if (need <= p->arena_bytes) return TEHMM_OK;
+            HCU(cudaStreamSynchronize(st));
+            if (p->arena) { cudaFree(p->arena); p->arena = nullptr; p->arena_bytes = 0; }
+            const size_t want = need + need / 8;
+            HCU(cudaMalloc(&p->arena, want));
+            p->arena_bytes = want;
+            return TEHMM_OK;
+        };
+        HOK(ensure(o_scratch + ((size_t)96 << 20) + (size_t)total * 8));
+        HOK(tehmm_set_batch(c, (char *)p->arena + o_obs, obs_bytes, nseq, h_offsets));
+        const size_t scratch = (size_t)tehmm_scratch_bytes(c, prec);
+        if (o_scratch + scratch > p->arena_bytes) {
+            HOK(ensure(o_scratch + scratch));
+            HOK(tehmm_set_batch(c, (char *)p->arena + o_obs, obs_bytes, nseq, h_offsets));
+        }
+        A = (char *)p->arena;
+        em_log = (viterbi || both) ? (void *)(A + o_la) : nullptr;
+        em_lin = both ? (void *)(A + o_lc) : (viterbi ? nullptr : (void *)(A + o_la));
+        d_rat = use_ratios ? (const double *)(A + o_rat) : nullptr;
+        piecewise = tehmm_emission_rows_supported(c, prec) == 1;
+        return TEHMM_OK;
+    }
+
+    // ---- host -> device: the observations.  The copy runs on its own stream in slices of whole rows; the emission
+    // kernel of a slice is enqueued on the compute stream behind that slice's event, so it overlaps the transfer of
+    // the next one (the emission is the only stage that can start before the whole batch has arrived).
+    int upload_obs(const void *const *h_obs_ptrs, int64_t nptr, int obs_bytes, int K)
+    {
+        const size_t row_bytes = (size_t)K * obs_bytes;
+        // the batch as a list of host segments (one, or one per sequence -- no host-side concatenation)
+        struct Seg { const unsigned char *src; size_t off, n; };
+        std::vector<Seg> segs;
+        if (nptr == 1) segs.push_back(Seg{(const unsigned char *)h_obs_ptrs[0], 0, (size_t)total * row_bytes});
+        else
+            for (int64_t i = 0; i < nseq; ++i) {
+                const size_t off = (size_t)h_offsets[i] * row_bytes, n = (size_t)(h_offsets[i + 1] - h_offsets[i]) * row_bytes;
+                if (n) segs.push_back(Seg{(const unsigned char *)h_obs_ptrs[i], off, n});
+            }
+        bool pinned = nptr == 1;
+        if (pinned) {
+            cudaPointerAttributes attr;
+            if (cudaPointerGetAttributes(&attr, h_obs_ptrs[0]) == cudaSuccess) pinned = attr.type == cudaMemoryTypeHost;
+            else { cudaGetLastError(); pinned = false; }
+        }
+        if (!p->copy_stream) HCU(cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking));
+        const int64_t slice_rows = (int64_t)(SLICE / row_bytes) & ~(int64_t)31;
+        if (slice_rows < 32) return herr(TEHMM_ELIMIT, "a row of %zu bytes does not fit the staging slices", row_bytes);
+        const int nth = p->pool->size();
+        size_t si = 0;                                       // first segment that reaches into the slice
+        for (int64_t r0 = 0; r0 < total; r0 += slice_rows, ++slot) {
+            const int64_t r1 = std::min(total, r0 + slice_rows);
+            const size_t off = (size_t)r0 * row_bytes, n = (size_t)(r1 - r0) * row_bytes;
+            if (pinned) {
+                HCU(cudaMemcpyAsync(A + o_obs + off, (const unsigned char *)h_obs_ptrs[0] + off, n, cudaMemcpyHostToDevice, p->copy_stream));
+            } else {
+                // pageable: worker threads fill a pinned slice while the previous one is on the wire
+                unsigned char *dst;
+                HOK(ring_slot(p, slot, &dst));
+                while (si + 1 < segs.size() && segs[si].off + segs[si].n <= off) ++si;
+                const size_t per = ((n + nth - 1) / nth + 63) & ~(size_t)63;
+                const Seg *sg = segs.data();
+                const size_t nsg = segs.size(), si0 = si;
+                p->pool->parallel_for(nth, [&](int i) {
+                    size_t a = off + (size_t)i * per;                       // byte range [a, e) of the batch
+                    const size_t e = std::min(off + n, a + per);
+                    size_t k = si0;
+                    while (a < e) {
+                        while (k + 1 < nsg && sg[k].off + sg[k].n <= a) ++k;
+                        const size_t m = std::min(e, sg[k].off + sg[k].n) - a;
+                        memcpy(dst + (a - off), sg[k].src + (a - sg[k].off), m);
+                        a += m;
+                    }
+                });
+                HCU(cudaMemcpyAsync(A + o_obs + off, dst, n, cudaMemcpyHostToDevice, p->copy_stream));
+                HCU(cudaEventRecord(p->ring_ev[slot % NRING], p->copy_stream));
+                p->ring_used[slot % NRING] = true;
+            }
+            cudaEvent_t ev;
+            HOK(slice_event(p, (size_t)slot, &ev));
+            HCU(cudaEventRecord(ev, p->copy_stream));
+            HCU(cudaStreamWaitEvent(st, ev, 0));
+            if (piecewise) HOK(tehmm_run_emission_rows(c, prec, nullptr, em_log, em_lin, (double *)(A + o_rowmax), r0, r1, UINT64_MAX));
+        }
+        return TEHMM_OK;
+    }
+
+    // ---- host -> device: the segment ratios.  They follow the observations through the same ring and copy stream
+    // (the Viterbi DP is the first stage that needs them): the worker threads gather each slice from the per-sequence
+    // arrays, fill -1.0 for a sequence without ratios, and check every value on the way.
+    int upload_ratios(const double *const *h_ratio_ptrs)
+    {
+        const int nth = p->pool->size();
+        const int64_t rat_rows = (int64_t)(SLICE / sizeof(double));
+        for (int64_t r0 = 0; r0 < total; r0 += rat_rows, ++slot) {
+            const int64_t r1 = std::min(total, r0 + rat_rows);
+            unsigned char *slice;
+            HOK(ring_slot(p, slot, &slice));
+            double *dst = (double *)slice;
+            const int64_t per = ((r1 - r0 + nth - 1) / nth + 7) & ~(int64_t)7;
+            std::atomic<int64_t> bad_row(INT64_MAX);
+            p->pool->parallel_for(nth, [&](int t) {
+                int64_t a = r0 + (int64_t)t * per;
+                const int64_t e = std::min(r1, a + per);
+                if (a >= e) return;
+                int64_t i = std::upper_bound(h_offsets, h_offsets + nseq + 1, a) - h_offsets - 1;
+                while (a < e) {
+                    while (h_offsets[i + 1] <= a) ++i;                 // (empty sequences)
+                    const int64_t n = std::min(e, h_offsets[i + 1]) - a;
+                    double *d = dst + (a - r0);
+                    const double *src = h_ratio_ptrs[i];
+                    if (!src) {
+                        std::fill(d, d + n, -1.0);
+                    } else {
+                        src += a - h_offsets[i];
+                        bool ok = true;
+                        for (int64_t k = 0; k < n; ++k) {
+                            const double v = src[k];
+                            ok &= v > 0.0 && v != INFINITY;            // NaN fails the first test
+                            d[k] = v;
+                        }
+                        if (!ok) {
+                            int64_t k = 0;
+                            while (src[k] > 0.0 && src[k] != INFINITY) ++k;
+                            int64_t cur = bad_row.load();
+                            while (a + k < cur && !bad_row.compare_exchange_weak(cur, a + k)) {}
+                        }
+                    }
+                    a += n;
+                }
+            });
+            if (bad_row.load() != INT64_MAX) {
+                const int64_t row = bad_row.load();
+                const int64_t i = std::upper_bound(h_offsets, h_offsets + nseq + 1, row) - h_offsets - 1;
+                return herr(TEHMM_EINVAL, "segment ratio %g of sequence %lld, step %lld: ratios must be finite and > 0",
+                            h_ratio_ptrs[i][row - h_offsets[i]], (long long)i, (long long)(row - h_offsets[i]));
+            }
+            HCU(cudaMemcpyAsync(A + o_rat + (size_t)r0 * 8, dst, (size_t)(r1 - r0) * 8, cudaMemcpyHostToDevice, p->copy_stream));
+            HCU(cudaEventRecord(p->ring_ev[slot % NRING], p->copy_stream));
+            p->ring_used[slot % NRING] = true;
+        }
+        // one event behind the last ratio slice (the ratio slices themselves record only their ring events)
+        cudaEvent_t ev;
+        HOK(slice_event(p, (size_t)slot, &ev));
+        HCU(cudaEventRecord(ev, p->copy_stream));
+        HCU(cudaStreamWaitEvent(st, ev, 0));
+        return TEHMM_OK;
+    }
+
+    int run_viterbi()
+    {
+        return tehmm_run_viterbi(c, prec, A + o_la, (const double *)(A + o_rowmax), nullptr, d_rat, A + o_lb,
+                                 (uint8_t *)(A + o_states), nullptr, (double *)(A + o_lp), A + o_scratch);
+    }
+
+    // ---- the trellis: the emission (unless the upload ran it slice by slice), then the Viterbi DP and traceback,
+    // or forward + backward(MAP).  BOTH runs forward + backward(MAP) here; download queues its Viterbi stage.
+    int run_trellis()
+    {
+        double *rowmax = (double *)(A + o_rowmax), *d_lp = (double *)(A + o_lp);
+        if (!piecewise) HOK(tehmm_run_emission(c, prec, nullptr, em_log, em_lin, rowmax));
+        if (viterbi) return run_viterbi();
+        HOK(tehmm_run_forward(c, prec, em_lin, rowmax, nullptr, A + o_lb, both ? d_lp + 2 * nseq : d_lp, A + o_scratch));
+        return tehmm_run_backward(c, prec, TEHMM_BWD_MAP | TEHMM_BWD_RENORM_EPS, em_lin, A + o_lb, nullptr, nullptr,
+                                  (uint8_t *)(A + (both ? o_states2 : o_states)), d_lp + nseq, nullptr, A + o_scratch);
+    }
+
+    // ---- device -> host: one byte per step over PCIe, widened by the host's cores, in slices, so that the widening
+    // of slice i overlaps the transfer of slice i+1.  *pin_lp: the per-sequence scalars, in the pinned buffer.
+    int download(int64_t *h_states, int64_t *h_states_map, const double **pin_lp)
+    {
+        const size_t out_bytes = (both ? 2 : 1) * up256((size_t)total) + (size_t)nseq * 32;
+        if (p->pin_out_bytes < out_bytes) {
+            HCU(cudaStreamSynchronize(st));
+            if (p->pin_out) cudaFreeHost(p->pin_out);
+            p->pin_out = nullptr; p->pin_out_bytes = 0;
+            HCU(cudaMallocHost((void **)&p->pin_out, out_bytes + out_bytes / 8));
+            p->pin_out_bytes = out_bytes + out_bytes / 8;
+        }
+        double *lp = (double *)(p->pin_out + (both ? 2 : 1) * up256((size_t)total));
+        const int nsl = (int)std::min<int64_t>(8, (total + (1 << 20) - 1) >> 20);
+        const int64_t per_sl = ((total + nsl - 1) / nsl + 63) & ~(int64_t)63;
+        const int nth = p->pool->size();
+        // queue the copies of one path (`which` picks the half of the pinned buffer and of the events; the upload's
+        // events are long complete: they are reused)
+        auto queue_copies = [&](size_t o_src, int which, cudaStream_t cs) -> int {
+            for (int i = 0; i < nsl; ++i) {
+                const int64_t a = (int64_t)i * per_sl, n = std::min(per_sl, total - a);
+                cudaEvent_t ev;
+                HOK(slice_event(p, (size_t)(which * nsl + i), &ev));
+                if (n > 0) HCU(cudaMemcpyAsync(p->pin_out + which * up256((size_t)total) + a, A + o_src + a, (size_t)n, cudaMemcpyDeviceToHost, cs));
+                HCU(cudaEventRecord(ev, cs));
+            }
+            return TEHMM_OK;
+        };
+        int rc = TEHMM_OK;
+        auto widen_slices = [&](int64_t *h_dst, int which) {
+            for (int i = 0; i < nsl; ++i) {
+                const int64_t a = (int64_t)i * per_sl, n = std::min(per_sl, total - a);
+                cudaError_t e = cudaEventSynchronize(p->slice_ev[which * nsl + i]);
+                if (e != cudaSuccess) { rc = herr(TEHMM_ECUDA, "decode failed: %s", cudaGetErrorString(e)); continue; }
+                if (n <= 0 || rc != TEHMM_OK) continue;
+                const int64_t per = ((n + nth - 1) / nth + 63) & ~(int64_t)63;
+                const uint8_t *src = p->pin_out + which * up256((size_t)total) + a;
+                int64_t *dst = h_dst + a;
+                p->pool->parallel_for(nth, [&](int t) {
+                    const int64_t b0 = (int64_t)t * per;
+                    if (b0 < n) widen_u8_i64(src + b0, dst + b0, std::min(per, n - b0));
+                });
+            }
+        };
+        if (both) {
+            // the MAP path leaves on the copy stream behind the backward pass; the Viterbi stage is queued on
+            // the compute stream meanwhile, and the host widens the MAP path while those kernels run
+            if (!p->both_ev) HCU(cudaEventCreateWithFlags(&p->both_ev, cudaEventDisableTiming));
+            HCU(cudaEventRecord(p->both_ev, st));
+            HCU(cudaStreamWaitEvent(p->copy_stream, p->both_ev, 0));
+            HOK(queue_copies(o_states2, 1, p->copy_stream));
+            HOK(run_viterbi());
+        }
+        HCU(cudaMemcpyAsync(lp, A + o_lp, (size_t)nseq * 32, cudaMemcpyDeviceToHost, st));
+        HOK(queue_copies(o_states, 0, st));
+        if (both) widen_slices(h_states_map, 1);
+        widen_slices(h_states, 0);
+        if (rc != TEHMM_OK) return rc;
+        HCU(cudaStreamSynchronize(st));
+        *pin_lp = lp;
+        return TEHMM_OK;
+    }
+};
+
 }   // namespace
 
 // called by tehmm_ctx_destroy
@@ -309,329 +598,39 @@ static int decode_host_impl(tehmm_ctx *c, const void *const *h_obs_ptrs, int64_t
     bool use_ratios = false;
     if (h_ratio_ptrs && algorithm != TEHMM_DECODE_MAP)
         for (int64_t i = 0; i < nseq && !use_ratios; ++i) use_ratios = h_ratio_ptrs[i] && h_offsets[i + 1] > h_offsets[i];
-    const int LD = tehmm_lattice_stride(c);
-    const size_t ts = prec == TEHMM_F32 ? 4 : 8;
-    const size_t obs_bytes_total = (size_t)total * K * obs_bytes;
-    const size_t lat = (size_t)total * LD * ts;
-
-    // ---- arena layout: obs | states | logprob, score | rowmax | lattice A | lattice B | [int64 states] | [ratios] | scratch
-    size_t o = 0;
-    const size_t o_obs = o; o = up256(o + obs_bytes_total);
-    const size_t o_states = o; o = up256(o + (size_t)total);
-    const size_t o_states2 = o; if (both) o = up256(o + (size_t)total);
-    const size_t o_lp = o; o = up256(o + (size_t)nseq * 32);        // [first logprob | score | second logprob] x nseq
-    const size_t o_rowmax = o; o = up256(o + (size_t)total * 8);
-    const size_t o_la = o; o = up256(o + lat);
-    const size_t o_lb = o; o = up256(o + lat);
-    const size_t o_lc = o; if (both) o = up256(o + lat);          // BOTH: A = log emission, C = linear emission, B = alpha, then delta
-    // Where the widening to int64 happens.  Host (default): one byte per step over PCIe, the pool's threads
-    // widen behind the copy.  Device (TEHMM_WIDEN=gpu, and only when the caller's result array is page-locked:
-    // the Python layer registers its result pool under TEHMM_PIN_RESULTS=1): a kernel widens and the DMA engine
-    // writes the int64 path straight into the result.  Measured, not the default: 9.6 vs 8.7 ms per
-    // Viterbi + MAP pair on one GPU and 22.4 vs 18.2 ms with eight ranks on one host
-    // (profiles/r02_notes_e2e.md) -- eight times the bytes over PCIe and into host memory cost more than the
-    // host threads they save; the 1 -> 8 GPU end-to-end curve is bound by the host's memory system either way.
-    bool gpu_widen = false;
-    {
-        cudaPointerAttributes attr;
-        const bool pinned_out = cudaPointerGetAttributes(&attr, h_states) == cudaSuccess && attr.type == cudaMemoryTypeHost;
-        cudaGetLastError();
-        const char *w = getenv("TEHMM_WIDEN");
-        if (pinned_out) gpu_widen = w != nullptr && !strcmp(w, "gpu");
-    }
-    const size_t o_s64 = o; if (gpu_widen) o = up256(o + (size_t)total * 8);
-    const size_t o_rat = o; if (use_ratios) o = up256(o + (size_t)total * 8);
-    const size_t o_scratch = o;
-    // the scratch size depends on the partition: describe the batch first, with the obs pointer
-    // the arena will have (the arena may have to grow before anything is enqueued)
-    auto ensure = [&](size_t need) -> int {
-        if (need <= p->arena_bytes) return TEHMM_OK;
-        HCU(cudaStreamSynchronize(st));
-        if (p->arena) { cudaFree(p->arena); p->arena = nullptr; p->arena_bytes = 0; }
-        const size_t want = need + need / 8;
-        HCU(cudaMalloc(&p->arena, want));
-        p->arena_bytes = want;
-        return TEHMM_OK;
-    };
-    HOK(ensure(o_scratch + ((size_t)96 << 20) + (size_t)total * 8));
-    HOK(tehmm_set_batch(c, (char *)p->arena + o_obs, obs_bytes, nseq, h_offsets));
-    size_t scratch = (size_t)tehmm_scratch_bytes(c, prec);
-    if (o_scratch + scratch > p->arena_bytes) {
-        HOK(ensure(o_scratch + scratch));
-        HOK(tehmm_set_batch(c, (char *)p->arena + o_obs, obs_bytes, nseq, h_offsets));
-        scratch = (size_t)tehmm_scratch_bytes(c, prec);
-    }
-    char *A = (char *)p->arena;
+    Decode d{c, p, st, prec, algorithm == TEHMM_DECODE_VITERBI, both, nseq, total, h_offsets};
+    HOK(d.setup_arena(K, obs_bytes, use_ratios));
     tr.mark("set_batch", false);
 
-    // ---- host -> device
-    // the batch as a list of host segments (one, or one per sequence -- no host-side concatenation)
-    struct Seg { const unsigned char *src; size_t off, n; };
-    std::vector<Seg> segs;
-    if (nptr == 1) segs.push_back(Seg{(const unsigned char *)h_obs_ptrs[0], 0, obs_bytes_total});
-    else
-        for (int64_t i = 0; i < nseq; ++i) {
-            const size_t off = (size_t)h_offsets[i] * K * obs_bytes, n = (size_t)(h_offsets[i + 1] - h_offsets[i]) * K * obs_bytes;
-            if (n) segs.push_back(Seg{(const unsigned char *)h_obs_ptrs[i], off, n});
-        }
-    bool pinned = nptr == 1;
-    if (pinned) {
-        cudaPointerAttributes attr;
-        if (cudaPointerGetAttributes(&attr, h_obs_ptrs[0]) == cudaSuccess) pinned = attr.type == cudaMemoryTypeHost;
-        else { cudaGetLastError(); pinned = false; }
-    }
-    // The copy runs on its own stream in slices of whole rows; the emission kernel of a slice is
-    // enqueued on the compute stream behind that slice's event, so it overlaps the transfer of the
-    // next one (the emission is the only stage that can start before the whole batch has arrived).
-    if (!p->copy_stream) HCU(cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking));
-    if (!p->both_ev) HCU(cudaEventCreateWithFlags(&p->both_ev, cudaEventDisableTiming));
-    double *d_lp = (double *)(A + o_lp), *d_sc = d_lp + nseq, *d_lp2 = d_lp + 2 * nseq;
-    uint8_t *d_states = (uint8_t *)(A + o_states), *d_states2 = (uint8_t *)(A + o_states2);
-    const bool viterbi = algorithm == TEHMM_DECODE_VITERBI;
-    void *em_log = (viterbi || both) ? (void *)(A + o_la) : nullptr;
-    void *em_lin = both ? (void *)(A + o_lc) : (viterbi ? nullptr : (void *)(A + o_la));
-    const bool piecewise = tehmm_emission_rows_supported(c, prec) == 1;
-    const size_t row_bytes = (size_t)K * obs_bytes;
-    int64_t slice_rows = (int64_t)(SLICE / row_bytes) & ~(int64_t)31;
-    if (slice_rows < 32) return herr(TEHMM_ELIMIT, "a row of %zu bytes does not fit the staging slices", row_bytes);
-    const int nth = p->pool->size();
-    size_t si = 0;                                       // first segment that reaches into the slice
-    int64_t slot = 0;
-    for (int64_t r0 = 0; r0 < total; r0 += slice_rows, ++slot) {
-        const int64_t r1 = std::min(total, r0 + slice_rows);
-        const size_t off = (size_t)r0 * row_bytes, n = (size_t)(r1 - r0) * row_bytes;
-        if (pinned) {
-            HCU(cudaMemcpyAsync(A + o_obs + off, (const unsigned char *)h_obs_ptrs[0] + off, n, cudaMemcpyHostToDevice, p->copy_stream));
-        } else {
-            // pageable: worker threads fill a pinned slice while the previous one is on the wire
-            const int r = (int)(slot % NRING);
-            if (!p->ring[r]) {
-                HCU(cudaMallocHost((void **)&p->ring[r], SLICE));
-                HCU(cudaEventCreateWithFlags(&p->ring_ev[r], cudaEventDisableTiming));
-            }
-            if (p->ring_used[r]) HCU(cudaEventSynchronize(p->ring_ev[r]));
-            while (si + 1 < segs.size() && segs[si].off + segs[si].n <= off) ++si;
-            unsigned char *dst = p->ring[r];
-            const size_t per = ((n + nth - 1) / nth + 63) & ~(size_t)63;
-            const Seg *sg = segs.data();
-            const size_t nsg = segs.size(), si0 = si;
-            p->pool->parallel_for(nth, [&](int i) {
-                size_t a = off + (size_t)i * per;                       // byte range [a, e) of the batch
-                const size_t e = std::min(off + n, a + per);
-                size_t k = si0;
-                while (a < e) {
-                    while (k + 1 < nsg && sg[k].off + sg[k].n <= a) ++k;
-                    const size_t m = std::min(e, sg[k].off + sg[k].n) - a;
-                    memcpy(dst + (a - off), sg[k].src + (a - sg[k].off), m);
-                    a += m;
-                }
-            });
-            HCU(cudaMemcpyAsync(A + o_obs + off, dst, n, cudaMemcpyHostToDevice, p->copy_stream));
-            HCU(cudaEventRecord(p->ring_ev[r], p->copy_stream));
-            p->ring_used[r] = true;
-        }
-        if ((size_t)slot >= p->slice_ev.size()) {
-            cudaEvent_t ev;
-            HCU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            p->slice_ev.push_back(ev);
-        }
-        HCU(cudaEventRecord(p->slice_ev[slot], p->copy_stream));
-        HCU(cudaStreamWaitEvent(st, p->slice_ev[slot], 0));
-        if (piecewise) HOK(tehmm_run_emission_rows(c, prec, nullptr, em_log, em_lin, (double *)(A + o_rowmax), r0, r1, UINT64_MAX));
-    }
-    // The segment ratios follow the observations through the same ring and copy stream (the Viterbi DP is the
-    // first stage that needs them): the worker threads gather each slice from the per-sequence arrays, fill -1.0
-    // for a sequence without ratios, and check every value on the way.
-    const double *d_rat = use_ratios ? (const double *)(A + o_rat) : nullptr;
-    if (use_ratios) {
-        const int64_t rat_rows = (int64_t)(SLICE / sizeof(double));
-        for (int64_t r0 = 0; r0 < total; r0 += rat_rows, ++slot) {
-            const int64_t r1 = std::min(total, r0 + rat_rows);
-            const int r = (int)(slot % NRING);
-            if (!p->ring[r]) {
-                HCU(cudaMallocHost((void **)&p->ring[r], SLICE));
-                HCU(cudaEventCreateWithFlags(&p->ring_ev[r], cudaEventDisableTiming));
-            }
-            if (p->ring_used[r]) HCU(cudaEventSynchronize(p->ring_ev[r]));
-            double *dst = (double *)p->ring[r];
-            const int64_t per = ((r1 - r0 + nth - 1) / nth + 7) & ~(int64_t)7;
-            std::atomic<int64_t> bad_row(INT64_MAX);
-            p->pool->parallel_for(nth, [&](int t) {
-                int64_t a = r0 + (int64_t)t * per;
-                const int64_t e = std::min(r1, a + per);
-                if (a >= e) return;
-                int64_t i = std::upper_bound(h_offsets, h_offsets + nseq + 1, a) - h_offsets - 1;
-                while (a < e) {
-                    while (h_offsets[i + 1] <= a) ++i;                 // (empty sequences)
-                    const int64_t n = std::min(e, h_offsets[i + 1]) - a;
-                    double *d = dst + (a - r0);
-                    const double *src = h_ratio_ptrs[i];
-                    if (!src) {
-                        std::fill(d, d + n, -1.0);
-                    } else {
-                        src += a - h_offsets[i];
-                        bool ok = true;
-                        for (int64_t k = 0; k < n; ++k) {
-                            const double v = src[k];
-                            ok &= v > 0.0 && v != INFINITY;            // NaN fails the first test
-                            d[k] = v;
-                        }
-                        if (!ok) {
-                            int64_t k = 0;
-                            while (src[k] > 0.0 && src[k] != INFINITY) ++k;
-                            int64_t cur = bad_row.load();
-                            while (a + k < cur && !bad_row.compare_exchange_weak(cur, a + k)) {}
-                        }
-                    }
-                    a += n;
-                }
-            });
-            if (bad_row.load() != INT64_MAX) {
-                const int64_t row = bad_row.load();
-                const int64_t i = std::upper_bound(h_offsets, h_offsets + nseq + 1, row) - h_offsets - 1;
-                return herr(TEHMM_EINVAL, "segment ratio %g of sequence %lld, step %lld: ratios must be finite and > 0",
-                            h_ratio_ptrs[i][row - h_offsets[i]], (long long)i, (long long)(row - h_offsets[i]));
-            }
-            HCU(cudaMemcpyAsync(A + o_rat + (size_t)r0 * 8, dst, (size_t)(r1 - r0) * 8, cudaMemcpyHostToDevice, p->copy_stream));
-            HCU(cudaEventRecord(p->ring_ev[r], p->copy_stream));
-            p->ring_used[r] = true;
-        }
-        // one event behind the last ratio slice (the ratio slices themselves record only their ring events)
-        while (p->slice_ev.size() <= (size_t)slot) {
-            cudaEvent_t ev;
-            HCU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            p->slice_ev.push_back(ev);
-        }
-        HCU(cudaEventRecord(p->slice_ev[slot], p->copy_stream));
-        HCU(cudaStreamWaitEvent(st, p->slice_ev[slot], 0));
-    }
-    p->h2d_bytes = (int64_t)obs_bytes_total + (use_ratios ? total * 8 : 0);
+    HOK(d.upload_obs(h_obs_ptrs, nptr, obs_bytes, K));
+    if (use_ratios) HOK(d.upload_ratios(h_ratio_ptrs));
+    p->h2d_bytes = total * K * obs_bytes + (use_ratios ? total * 8 : 0);
     tr.mark("h2d+emission", true);
 
     // Two attempts at most.  The first runs the stages with deferred verification (option "defer":
     // no stall of the stream after each stage to read the repair count); the counts are looked at
     // once everything has arrived.  If a speculated chunk boundary failed -- rare -- the trellis and
-    // the download run again with the synchronous verify / repair loop.
+    // the download run again with the synchronous verify / repair loop.  (After a refusal the context
+    // leaves "defer" off for its next calls: see tehmm_ctx_check.)
     struct DeferGuard { tehmm_ctx *c; ~DeferGuard() { tehmm_ctx_set_option(c, "defer", 0); } } defer_guard{c};
-    double *pin_lp = nullptr;
-    int rc = TEHMM_OK;
-    // (after a refusal the next calls go straight to the synchronous loop: a refused attempt costs the
-    //  trellis twice, and a model / batch that needed repairs tends to need them again)
-    int attempt = 0;
-    if (p->defer_skip > 0) { p->defer_skip -= 1; attempt = 1; }
-    for (; attempt < 2; ++attempt) {
+    const double *pin_lp = nullptr;
+    for (int attempt = 0; attempt < 2; ++attempt) {
         HOK(tehmm_ctx_set_option(c, "defer", attempt == 0 ? 1 : 0));
-        // ---- the trellis
-        if (!piecewise) HOK(tehmm_run_emission(c, prec, nullptr, em_log, em_lin, (double *)(A + o_rowmax)));
-        if (both) {
-            // forward + backward(MAP) first: their states travel and are widened while the Viterbi kernels run
-            HOK(tehmm_run_forward(c, prec, A + o_lc, (double *)(A + o_rowmax), nullptr, A + o_lb, d_lp2, A + o_scratch));
-            HOK(tehmm_run_backward(c, prec, TEHMM_BWD_MAP | TEHMM_BWD_RENORM_EPS, A + o_lc, A + o_lb, nullptr, nullptr,
-                                   d_states2, d_sc, nullptr, A + o_scratch));
-        } else if (viterbi) {
-            HOK(tehmm_run_viterbi(c, prec, A + o_la, (const double *)(A + o_rowmax), nullptr, d_rat, A + o_lb, d_states, nullptr, d_lp, A + o_scratch));
-        } else {
-            HOK(tehmm_run_forward(c, prec, A + o_la, (double *)(A + o_rowmax), nullptr, A + o_lb, d_lp, A + o_scratch));
-            HOK(tehmm_run_backward(c, prec, TEHMM_BWD_MAP | TEHMM_BWD_RENORM_EPS, A + o_la, A + o_lb, nullptr, nullptr,
-                                   d_states, d_sc, nullptr, A + o_scratch));
-        }
-
+        HOK(d.run_trellis());
         tr.mark("trellis", true);
-        // ---- device -> host: one byte per step over PCIe, widened by the host's cores
-        const size_t out_bytes = (both ? 2 : 1) * up256((size_t)total) + (size_t)nseq * 32;
-        if (p->pin_out_bytes < out_bytes) {
-            HCU(cudaStreamSynchronize(st));
-            if (p->pin_out) cudaFreeHost(p->pin_out);
-            p->pin_out = nullptr; p->pin_out_bytes = 0;
-            HCU(cudaMallocHost((void **)&p->pin_out, out_bytes + out_bytes / 8));
-            p->pin_out_bytes = out_bytes + out_bytes / 8;
-        }
-        pin_lp = (double *)(p->pin_out + (both ? 2 : 1) * up256((size_t)total));
-        if (!both) HCU(cudaMemcpyAsync(pin_lp, d_lp, (size_t)nseq * 32, cudaMemcpyDeviceToHost, st));
-        if (gpu_widen && !both) {
-            int64_t *d_s64 = (int64_t *)(A + o_s64);
-            HOK(tehmm_widen_states(c, d_states, d_s64, total));
-            HCU(cudaMemcpyAsync(h_states, d_s64, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
-            HCU(cudaStreamSynchronize(st));
-            tr.mark("d2h(int64)", false);
-            rc = TEHMM_OK;
-            if (attempt == 0) {
-                int64_t unverified = 0;
-                HOK(tehmm_ctx_set_option(c, "defer", 0));
-                HOK(tehmm_ctx_check(c, &unverified));
-                if (unverified == 0) { p->defer_penalty /= 2; break; }
-                p->redone += 1;
-                p->defer_penalty = std::min(256, std::max(4, 2 * p->defer_penalty));
-                p->defer_skip = p->defer_penalty;
-            }
-            continue;
-        }
-        // slices, so that the widening of slice i overlaps the transfer of slice i+1
-        const int nsl = (int)std::min<int64_t>(8, (total + (1 << 20) - 1) >> 20);
-        const int64_t per_sl = ((total + nsl - 1) / nsl + 63) & ~(int64_t)63;
-        while ((int)p->slice_ev.size() < 2 * nsl) {        // the upload's events are long complete: reuse them
-            cudaEvent_t ev;
-            HCU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            p->slice_ev.push_back(ev);
-        }
-        const std::vector<cudaEvent_t> &evs = p->slice_ev;
-        // queue the copies of one path (`which` picks the half of the pinned buffer and of the events)
-        auto queue_copies = [&](const uint8_t *d_src, int which, cudaStream_t cs) -> int {
-            for (int i = 0; i < nsl; ++i) {
-                const int64_t a = (int64_t)i * per_sl, n = std::min(per_sl, total - a);
-                if (n > 0) HCU(cudaMemcpyAsync(p->pin_out + which * up256((size_t)total) + a, d_src + a, (size_t)n, cudaMemcpyDeviceToHost, cs));
-                HCU(cudaEventRecord(evs[which * nsl + i], cs));
-            }
-            return TEHMM_OK;
-        };
-        auto widen_slices = [&](int64_t *h_dst, int which) {
-            for (int i = 0; i < nsl; ++i) {
-                const int64_t a = (int64_t)i * per_sl, n = std::min(per_sl, total - a);
-                cudaError_t e = cudaEventSynchronize(evs[which * nsl + i]);
-                if (e != cudaSuccess) { rc = herr(TEHMM_ECUDA, "decode failed: %s", cudaGetErrorString(e)); continue; }
-                if (n <= 0 || rc != TEHMM_OK) continue;
-                const int64_t per = ((n + nth - 1) / nth + 63) & ~(int64_t)63;
-                const uint8_t *src = p->pin_out + which * up256((size_t)total) + a;
-                int64_t *dst = h_dst + a;
-                p->pool->parallel_for(nth, [&](int t) {
-                    const int64_t b0 = (int64_t)t * per;
-                    if (b0 < n) widen_u8_i64(src + b0, dst + b0, std::min(per, n - b0));
-                });
-            }
-        };
-        rc = TEHMM_OK;
-        if (both) {
-            // the MAP path leaves on the copy stream behind the backward pass; the Viterbi stage is queued on
-            // the compute stream meanwhile, and the host widens the MAP path while those kernels run
-            HCU(cudaEventRecord(p->both_ev, st));
-            HCU(cudaStreamWaitEvent(p->copy_stream, p->both_ev, 0));
-            HOK(queue_copies(d_states2, 1, p->copy_stream));
-            HOK(tehmm_run_viterbi(c, prec, A + o_la, (const double *)(A + o_rowmax), nullptr, d_rat, A + o_lb, d_states, nullptr, d_lp, A + o_scratch));
-            HCU(cudaMemcpyAsync(pin_lp, d_lp, (size_t)nseq * 32, cudaMemcpyDeviceToHost, st));
-            HOK(queue_copies(d_states, 0, st));
-            widen_slices(h_states_map, 1);
-            widen_slices(h_states, 0);
-        } else {
-            HOK(queue_copies(d_states, 0, st));
-            widen_slices(h_states, 0);
-        }
-        if (rc != TEHMM_OK) return rc;
-        HCU(cudaStreamSynchronize(st));
+        HOK(d.download(h_states, h_states_map, &pin_lp));
         tr.mark("d2h+widen", false);
         if (attempt == 0) {
             int64_t unverified = 0;
             HOK(tehmm_ctx_set_option(c, "defer", 0));
             HOK(tehmm_ctx_check(c, &unverified));
-            if (unverified == 0) { p->defer_penalty /= 2; break; }
-            p->redone += 1;
-            p->defer_penalty = std::min(256, std::max(4, 2 * p->defer_penalty));
-            p->defer_skip = p->defer_penalty;
+            if (unverified == 0) break;
         }
     }
     memcpy(h_logprob, pin_lp, (size_t)nseq * 8);
     if (h_score) memcpy(h_score, pin_lp + nseq, (size_t)nseq * 8);
     if (both) memcpy(h_fwd_logprob, pin_lp + 2 * nseq, (size_t)nseq * 8);
-    p->d2h_bytes = (gpu_widen && !both ? (int64_t)total * 8 : (both ? 2 : 1) * (int64_t)total) + nseq * (both ? 32 : 16);
+    p->d2h_bytes = (both ? 2 : 1) * total + nseq * (both ? 32 : 16);
     return TEHMM_OK;
 }
 

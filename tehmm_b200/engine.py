@@ -67,51 +67,14 @@ class _ResultPool(object):
     def __init__(self):
         self._free = []
         self._lock = threading.Lock()
-        self._registered = {}            # id(block) -> address: page-locked with cudaHostRegister
-
-    # With TEHMM_PIN_RESULTS=1 (or TEHMM_WIDEN=gpu) blocks are page-locked (cudaHostRegister) so that
-    # tehmm_decode_host can let the DMA engine write the int64 path straight into the result (device-side
-    # widening, csrc/host.cu) instead of widening on the host's cores.  Off by default: measured slower
-    # (profiles/r02_notes_e2e.md).  Registration costs milliseconds per block, paid once: blocks are recycled.
-    @staticmethod
-    def _address(block):
-        c = ctypes.c_char.from_buffer(block)
-        try:
-            return ctypes.addressof(c)
-        finally:
-            del c                        # drop the extra buffer export at once
-
-    def _register(self, block):
-        if os.environ.get("TEHMM_PIN_RESULTS", "0") != "1" and os.environ.get("TEHMM_WIDEN") != "gpu":
-            return
-        try:
-            torch = _torch()
-            if not torch.cuda.is_available():
-                return
-            addr = self._address(block)
-            rc = torch.cuda.cudart().cudaHostRegister(addr, len(block), 0)
-            if int(rc) == 0:
-                self._registered[id(block)] = addr
-        except Exception:
-            pass
-
-    def _unregister(self, block):
-        addr = self._registered.pop(id(block), None)
-        if addr is not None:
-            try:
-                _torch().cuda.cudart().cudaHostUnregister(addr)
-            except Exception:
-                pass
 
     def _put(self, block):
+        # over the cap the block is simply not kept: it is unmapped when the dying array releases
+        # its buffer export (closing it here would raise: the export is still counted in a finalizer)
         with self._lock:
             held = sum(len(b) for b in self._free)
             if len(self._free) < self.MAX_FREE and held + len(block) <= self.MAX_FREE_BYTES:
                 self._free.append(block)
-                return
-        # over the cap: the block is simply not kept -- it is unmapped when the dying array releases
-        # its buffer export (closing it here would raise: the export is still counted in a finalizer)
-        self._unregister(block)
 
     def empty_int64(self, n):
         nbytes = max(8, int(n) * 8)
@@ -130,7 +93,6 @@ class _ResultPool(object):
                 block.madvise(mmap.MADV_HUGEPAGE)
             except (AttributeError, OSError, ValueError):
                 pass
-            self._register(block)
         arr = np.frombuffer(block, dtype=np.int64, count=int(n))
         weakref.finalize(arr, self._put, block)
         return arr
@@ -191,18 +153,7 @@ class Engine(object):
         torch = self.torch
         self._bind_stream()
         self.batch_token = None
-        arrays = [as_obs_array(o) for o in obs_list]
-        assert len(arrays) > 0
-        K = arrays[0].shape[1]
-        for a in arrays:
-            assert a.shape[1] == K, "all sequences must have the same number of tracks"
-        dt = arrays[0].dtype
-        if any(a.dtype != dt for a in arrays):
-            dt = np.dtype(np.int32)
-            arrays = [a.astype(np.int32) for a in arrays]
-        lens = np.array([a.shape[0] for a in arrays], dtype=np.int64)
-        offsets = np.zeros(len(arrays) + 1, dtype=np.int64)
-        np.cumsum(lens, out=offsets[1:])
+        arrays, dt, offsets, _ = self._host_arrays(obs_list)
         host = arrays[0] if len(arrays) == 1 else np.concatenate(arrays, axis=0)
         if dt == np.uint16:   # torch has no full uint16 support everywhere: move raw bytes
             d_obs = torch.from_numpy(host.view(np.uint8).reshape(-1)).to(self.device)
@@ -220,7 +171,8 @@ class Engine(object):
 
     @staticmethod
     def _host_arrays(obs_list):
-        """observation matrices of a host-buffer call: (arrays, dtype, offsets int64[nseq+1], void* table)"""
+        """observation matrices of a batch, converted and checked: (arrays, dtype, offsets int64[nseq+1],
+        void* table for the host-buffer calls)"""
         arrays = [as_obs_array(o) for o in obs_list]
         assert len(arrays) > 0
         K = arrays[0].shape[1]

@@ -65,6 +65,7 @@ def test_decode_host_equals_device_path_large():
     pinned = torch.from_numpy(obs).pin_memory().numpy()
     for first in (obs, pinned):
         lp, _, st = eng.decode_host([first, obs2], _lib.DECODE_VITERBI)
+        assert eng.d2h_bytes == T + 200_003 + 32
         assert_array_equal(lp, lp_d)
         assert_array_equal(st[0], st_d[0])
         assert_array_equal(st[1], st_d[1])
@@ -103,39 +104,11 @@ def test_decode_host_wide_model_equals_device_path(nseq):
         assert_array_equal(ms[i], out["map_states"][i])
 
 
-def test_device_side_widening_into_the_registered_result(monkeypatch):
-    """TEHMM_WIDEN=gpu: the int64 path is written by the DMA engine straight into the (page-locked) result
-    array of the Python layer's pool -- no host thread touches it; same states as the host-widening route."""
-    from tehmm_b200 import _lib, synth
-    m = synth.make_model(N=30, seed=0)
-    obs, _ = synth.sample_obs(m, 700_001, seed=5)
-    eng = _engine()
-    eng.upload_model(m["log_start"], m["log_trans"], m["table"], 1.0, m["widths"])
-    monkeypatch.setenv("TEHMM_WIDEN", "host")
-    lp_h, _, st_h = eng.decode_host([obs], _lib.DECODE_VITERBI)
-    assert eng.d2h_bytes == 700_001 + 16
-    monkeypatch.setenv("TEHMM_WIDEN", "gpu")
-    from tehmm_b200 import engine as engine_mod
-    del st_h
-    engine_mod._result_pool._free[:] = []           # blocks are page-locked when they are created
-    lp_g, _, st_g = eng.decode_host([obs], _lib.DECODE_VITERBI)
-    assert eng.d2h_bytes == 8 * 700_001 + 16, "the result pool's blocks must be page-locked for the device-side route"
-    assert_array_equal(lp_g, lp_h)
-    st_g_copy = st_g[0].copy()
-    assert st_g[0].dtype == np.int64
-    _, sc_g, ms_g = eng.decode_host([obs], _lib.DECODE_MAP)
-    monkeypatch.setenv("TEHMM_WIDEN", "host")
-    _, sc_h, ms_h = eng.decode_host([obs], _lib.DECODE_MAP)
-    assert_array_equal(ms_g[0], ms_h[0])
-    assert_array_equal(sc_g, sc_h)
-    _, _, st_h2 = eng.decode_host([obs], _lib.DECODE_VITERBI)
-    assert_array_equal(st_g_copy, st_h2[0])
-
-
 def test_decode_both_equals_the_two_calls():
     """one upload, one emission pass, both decodings: bit-identical to decode(viterbi) and decode(map)"""
     from tehmm_b200 import synth
     from tehmm_b200.emission import IndependentMultinomialEmissionModel
+    from tehmm_b200.engine import get_engine
     from tehmm_b200.hmm import MultitrackHmm
     m = synth.make_model(N=30, seed=0)
     obs = [synth.sample_obs(m, T, seed=20 + i)[0] for i, T in enumerate([1_200_003, 17, 300_000, 1])]
@@ -151,6 +124,7 @@ def test_decode_both_equals_the_two_calls():
         assert_array_equal(vst, st)
         assert_array_equal(mst, ms)
         assert vst.dtype == np.int64 and mst.dtype == np.int64
+    assert get_engine(0).d2h_bytes == 2 * sum(len(o) for o in obs) + 32 * len(obs)
     assert hv.getLastLogProb() is not None
 
 
@@ -232,7 +206,7 @@ def test_deferred_verification_falls_back_to_the_repair_loop(oracle):
     eng.ctx.set_option("warmup", 1)
     try:
         eng.upload_model(m["log_start"], m["log_trans"], m["table"], 1.0, m["widths"])
-        eng.ctx._defer_skip = 0
+        eng.ctx.set_option("defer_skip", 0)
         bad0 = eng.ctx.stat("deferred_bad")
         lp, _, states = eng.decode_host(seqs, _lib.DECODE_VITERBI, precision="f64")
         flp, score, mstates = eng.decode_host(seqs, _lib.DECODE_MAP, precision="f64")
@@ -246,7 +220,7 @@ def test_deferred_verification_falls_back_to_the_repair_loop(oracle):
             assert flp[i] == pytest.approx(ref["logprob"], rel=1e-10)
         # engine passes (fp32 production kernels): optimistic attempt, refused, repaired
         eng.upload_batch(seqs)
-        eng.ctx._defer_skip = 0
+        eng.ctx.set_option("defer_skip", 0)
         bad1 = eng.ctx.stat("deferred_bad")
         out = eng.posteriors(renorm_eps=False, want_map=True, want_post=False, precision="f32")
         vlp, vst = eng.viterbi(precision="f32")
@@ -260,8 +234,8 @@ def test_deferred_verification_falls_back_to_the_repair_loop(oracle):
                                   m["log_start"], m["log_trans"])
         assert st["obs"].sum() == pytest.approx(sum(lens) * m["K"], rel=1e-5)
         # a healthy warm-up: the optimistic attempt stands (once the back-off after a refusal is over)
-        assert eng.ctx._defer_skip > 0
-        eng.ctx._defer_skip = 0
+        assert eng.ctx.stat("defer_skip") > 0
+        eng.ctx.set_option("defer_skip", 0)
         eng.ctx.set_option("warmup", 0)
         eng.upload_batch(seqs)
         bad2 = eng.ctx.stat("deferred_bad")
