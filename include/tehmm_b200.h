@@ -423,6 +423,38 @@ int tehmm_scores_to_bed(int fd, const char *chrom, int64_t start, const double *
 /* convert on the device before a D2H copy */
 int tehmm_convert_lattice(tehmm_ctx *ctx, int prec, const void *d_in, double *d_out, int64_t n);
 
+/* ------------------------------------------------- windows of sequences longer than device memory
+ * (DESIGN.md section 11, csrc/window.cu).  A batch can be one time window of longer sequences: a
+ * sequence of the batch may continue one that began before the window, or go on after it.
+ * tehmm_set_boundary gives such sequences their boundary vectors (host arrays, copied; sequence
+ * indices increasing, every vector finite, >= 0 and not zero; n = 0: none).  tehmm_set_batch
+ * clears them, and so does a call with n_entry = n_exit = 0: without vectors every pass is
+ * exactly what it was.
+ *   entry (h_entry_vec[k*N ..]): the forward vector of the step before the sequence's first row,
+ *     normalised here to sum 1.  tehmm_run_forward's first step is then (v A) .* b instead of
+ *     pi .* b, and its log-likelihood is the increment log P(x_a..x_{b-1} | x_{<a}); the first
+ *     row adds nothing to the start counts and tehmm_ratio_diag_counts gives it its segment
+ *     ratio's diagonal count.  With entry vectors set, segment ratios must be folded
+ *     (tehmm_fold_ratios): tehmm_run_backward(TRANS) with d_ratios returns TEHMM_EINVAL.
+ *   exit (h_exit_vec[k*N ..]): b .* beta of the step after the sequence's last row, any positive
+ *     scale.  tehmm_run_backward then ends the sequence with beta = A u instead of the constant
+ *     row (the reference's log(1/N)); the statistics keep the reference's 1/N factor.  It scales
+ *     the last rows of d_alpha and d_blin for the duration of the call and puts them back.
+ * tehmm_forward_row: row `row` of a forward lattice, normalised to sum 1, into h_out[N]: the entry
+ *   vector of the window that continues after that row.
+ * tehmm_cut_pair: the transition pair across a cut, from h_v (the entry vector of the window to the
+ *   right of the cut) and d_post_row (that window's first posterior row, lattice precision, not
+ *   renormalised): adds (1/N) v_i A_ij u_j / sum(v A u) to d_trans[i*N + j] (N x N float64 on the
+ *   device, may be NULL) with u = gamma ./ (v A) (0 where v A is 0), and writes u to h_u[N]: the
+ *   exit vector of the window to the left.  Synchronises the stream.
+ * tehmm_convert_rows: a (rows, LD) lattice to (rows, N) float64 on the device; renorm = 1 applies
+ *   the TEHMM_BWD_RENORM_EPS renormalisation to the stored posteriors as the backward pass does. */
+int tehmm_set_boundary(tehmm_ctx *ctx, int64_t n_entry, const int64_t *h_entry_seq, const double *h_entry_vec,
+                       int64_t n_exit, const int64_t *h_exit_seq, const double *h_exit_vec);
+int tehmm_forward_row(tehmm_ctx *ctx, int prec, const void *d_alpha, int64_t row, double *h_out);
+int tehmm_cut_pair(tehmm_ctx *ctx, int prec, const double *h_v, const void *d_post_row, double *d_trans, double *h_u);
+int tehmm_convert_rows(tehmm_ctx *ctx, int prec, const void *d_in, int64_t rows, int renorm, double *d_out);
+
 #ifdef __cplusplus
 }
 #endif

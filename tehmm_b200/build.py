@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libtehmm_b200.so")
-UNITS = ["api", "strict", "emission", "forward", "backward", "viterbi", "stats", "tile", "host", "umma", "fallback", "tracks", "ratios", "supervised"]
+UNITS = ["api", "strict", "emission", "forward", "backward", "viterbi", "stats", "tile", "host", "umma", "fallback", "tracks", "ratios", "supervised", "window"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",
           "-Xptxas", "-v"]

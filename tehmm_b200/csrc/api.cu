@@ -50,6 +50,10 @@ cudaError_t tehmm_launch_transfer_ops(cudaStream_t, const TehmmModelDev &, const
 cudaError_t tehmm_launch_ratio_fold(cudaStream_t, const TehmmModelDev &, int64_t, int, const double *, void *, double *, int);
 cudaError_t tehmm_launch_ratio_diag(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const double *, const void *, double *, double *, int);
 cudaError_t tehmm_launch_chain(cudaStream_t, const TehmmModelDev &, int, int, int, const int64_t *, const int64_t *, int64_t, const void *, const double *, const void *, void *);
+cudaError_t tehmm_launch_entry(cudaStream_t, const TehmmBatchDev &, int, int, int64_t, const int64_t *, const double *, void *, int *);
+cudaError_t tehmm_launch_exit(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, int64_t, const int64_t *, const double *, void *, void *, void *, int);
+cudaError_t tehmm_launch_cut_pair(cudaStream_t, const TehmmModelDev &, int, const double *, const void *, double *, double *);
+cudaError_t tehmm_launch_convert_rows(cudaStream_t, int, int, int, const void *, int64_t, int, double *, int);
 
 // ---------------------------------------------------------------- errors
 static thread_local std::string g_err;
@@ -140,6 +144,15 @@ struct tehmm_ctx {
     int64_t seq_flag_n = 0;
     int64_t max_tiles_per_chunk = 1;
     int64_t fine_len = 0;         // steps per chunk of the fine partition
+    // boundary conditions of the current batch (tehmm_set_boundary, window.cu; cleared by tehmm_set_batch):
+    // blob = cont[nseq] | entry_seq[n_entry] | entry_vec[n_entry][NP] | exit_seq[n_exit] | exit_vec[n_exit][NP]
+    //        | the rows exit_kernel saves (n_exit x 2 x LD elements of float64 size)
+    int64_t n_entry = 0, n_exit = 0;
+    void *bnd_blob = nullptr;
+    size_t bnd_blob_bytes = 0;
+    const int64_t *d_entry_seq = nullptr, *d_exit_seq = nullptr;
+    const double *d_entry_vec = nullptr, *d_exit_vec = nullptr;
+    void *d_exit_save = nullptr;
 };
 
 extern "C" {
@@ -184,6 +197,7 @@ int tehmm_ctx_destroy(tehmm_ctx *c)
     tehmm_hostpipe_release(c);
     if (c->model_blob) cudaFree(c->model_blob);
     if (c->batch_blob) cudaFree(c->batch_blob);
+    if (c->bnd_blob) cudaFree(c->bnd_blob);
     if (c->d_seq_flag) cudaFree(c->d_seq_flag);
     if (c->h_nbad) cudaFreeHost(c->h_nbad);
     if (c->h_pending) cudaFreeHost(c->h_pending);
@@ -755,6 +769,8 @@ int tehmm_set_batch(tehmm_ctx *c, const void *d_obs, int obs_bytes, int64_t nseq
     CU(cudaSetDevice(c->device));
     const int64_t total = h_offsets[nseq];
     if (total <= 0) return fail(TEHMM_EINVAL, "empty batch");
+    c->n_entry = c->n_exit = 0;               // a new batch starts without boundary vectors
+    c->b.cont = c->bf.cont = nullptr;
     {   // the same batch shape at the same address again (a stream of decode calls): keep the partition
         std::vector<int64_t> key(h_offsets, h_offsets + nseq + 1);
         key.push_back((int64_t)(uintptr_t)d_obs); key.push_back(obs_bytes);
@@ -836,6 +852,7 @@ int tehmm_set_batch(tehmm_ctx *c, const void *d_obs, int obs_bytes, int64_t nseq
     b.seq_off = (const int64_t *)(d + o_off); b.seq_chunk0 = (const int64_t *)(d + o_sc);
     b.chunks = (const TehmmChunk *)(d + o_ch);
     b.warmup = (int)(c->opt_warmup > 0 ? c->opt_warmup : 64);
+    b.cont = nullptr;
     c->bf = b;
     c->bf.nchunks = nfchunks;
     c->bf.seq_chunk0 = (const int64_t *)(d + o_fsc);
@@ -1241,6 +1258,13 @@ static int repair_loop(tehmm_ctx *c, cudaStream_t st, const TehmmBatchDev &PB, i
     CU(launch(0));
     tk_end(c, timer[kind]);
     c->launches += 1;
+    if (kind == 0 && c->n_entry > 0) {
+        // continued sequences (tehmm_set_boundary): their first chunks are exact from the entry vectors, run
+        // like repaired chunks; the verification below then checks the chunks after them as usual
+        CU(tehmm_launch_entry(st, PB, prec, c->m.NP, c->n_entry, c->d_entry_seq, c->d_entry_vec, sv, bad));
+        CU(launch(1));
+        c->launches += 2;
+    }
     const bool umma = umma_used && *umma_used;
     double tol = tolerance(prec, log_space);
     const int64_t max_pass = c->opt_max_repair > 0 ? c->opt_max_repair : PB.nchunks + 1;
@@ -1330,6 +1354,10 @@ int tehmm_run_backward(tehmm_ctx *c, int prec, int flags, const void *d_blin, co
     if ((flags & TEHMM_BWD_POSTERIORS) && !d_post) return fail(TEHMM_EINVAL, "POSTERIORS needs d_post");
     if ((flags & TEHMM_BWD_MAP) && (!d_map_states || !d_map_score)) return fail(TEHMM_EINVAL, "MAP needs d_map_states and d_map_score");
     if ((flags & TEHMM_BWD_TRANS) && !d_start_trans) return fail(TEHMM_EINVAL, "TRANS needs d_start_trans");
+    // the in-kernel diagonal count of unfolded ratios treats every sequence's first row as a start; a continued
+    // sequence's first row is not one: such batches fold the ratios and count them with tehmm_ratio_diag_counts
+    if ((flags & TEHMM_BWD_TRANS) && d_ratios && c->n_entry > 0)
+        return fail(TEHMM_EINVAL, "TRANS with unfolded segment ratios and entry vectors: fold the ratios (tehmm_fold_ratios) and use tehmm_ratio_diag_counts");
     const Scratch s = carve(c, prec);
     char *w = (char *)d_scratch;
     void *sv = w + s.start_vec, *ev = w + s.end_vec;
@@ -1347,6 +1375,33 @@ int tehmm_run_backward(tehmm_ctx *c, int prec, int flags, const void *d_blin, co
     // first pass on the fine partition; repairs stay with the one-chunk-per-warp kernel on the same partition
     const bool wide_umma = use_umma(c, prec, d_ratios) && !(flags & TEHMM_BWD_TRANS);
     const TehmmBatchDev &PB = (tile || wide_umma) ? c->bf : c->b;
+    // exit vectors: the last rows of alpha and blin are scaled by A u until the end of the call (window.cu); the
+    // guard queues their restore on every way out, so a failing launch below never leaves the caller's lattices changed
+    struct ExitRows {
+        tehmm_ctx *c = nullptr;
+        cudaStream_t st;
+        int prec;
+        void *alpha, *blin;
+        cudaError_t restore()
+        {
+            tehmm_ctx *cc = c;
+            c = nullptr;
+            if (!cc) return cudaSuccess;
+            cc->launches += 1;
+            return tehmm_launch_exit(st, cc->m, cc->b, prec, cc->n_exit, cc->d_exit_seq, cc->d_exit_vec, alpha, blin, cc->d_exit_save, 1);
+        }
+        ~ExitRows() { restore(); }
+    } exit_rows;
+    if (c->n_exit > 0) {
+        CU(tehmm_launch_exit(st, c->m, c->b, prec, c->n_exit, c->d_exit_seq, c->d_exit_vec, const_cast<void *>(d_alpha),
+                             const_cast<void *>(d_blin), c->d_exit_save, 0));
+        c->launches += 1;
+        exit_rows.c = c;
+        exit_rows.st = st;
+        exit_rows.prec = prec;
+        exit_rows.alpha = const_cast<void *>(d_alpha);
+        exit_rows.blin = const_cast<void *>(d_blin);
+    }
     bool umma_used = false;
     auto launch = [&](int mode) -> cudaError_t {
         if (wide_umma && tehmm_backward_umma_ok(c->m, PB, flags, mode, c->fine_len)) {
@@ -1371,6 +1426,7 @@ int tehmm_run_backward(tehmm_ctx *c, int prec, int flags, const void *d_blin, co
         tk_end(c, TK_XI);
         c->launches += 2;
     }
+    CU(exit_rows.restore());
     return TEHMM_OK;
 }
 
@@ -1487,6 +1543,123 @@ int tehmm_path_score(tehmm_ctx *c, const uint8_t *d_states, const double *d_rati
     double *sp = (double *)((char *)d_scratch + s.part_a);
     CU(tehmm_launch_rescore(st, c->m, c->bf, d_states, d_ratios_emission, d_ratios_dp, sp, d_logprob, lo, hi));
     c->launches += 2;
+    return TEHMM_OK;
+}
+
+// ---------------------------------------------------------------- windows of longer sequences (window.cu)
+static int check_vectors(const char *what, int64_t n, const int64_t *seq, const double *vec, int64_t nseq, int N,
+                         const std::vector<int64_t> &off)
+{
+    for (int64_t k = 0; k < n; ++k) {
+        if (seq[k] < 0 || seq[k] >= nseq) return fail(TEHMM_EINVAL, "%s %lld: sequence %lld outside [0,%lld)", what, (long long)k, (long long)seq[k], (long long)nseq);
+        if (k > 0 && seq[k] <= seq[k - 1]) return fail(TEHMM_EINVAL, "%s sequences must be increasing", what);
+        if (off[seq[k] + 1] <= off[seq[k]]) return fail(TEHMM_EINVAL, "%s %lld: sequence %lld is empty", what, (long long)k, (long long)seq[k]);
+        double sum = 0.0;
+        for (int j = 0; j < N; ++j) {
+            const double x = vec[k * N + j];
+            if (!(x >= 0.0) || !std::isfinite(x)) return fail(TEHMM_EINVAL, "%s %lld: component %d is %g (must be finite and >= 0)", what, (long long)k, j, x);
+            sum += x;
+        }
+        if (!(sum > 0.0)) return fail(TEHMM_EINVAL, "%s %lld: the vector is zero", what, (long long)k);
+    }
+    return 0;
+}
+
+int tehmm_set_boundary(tehmm_ctx *c, int64_t n_entry, const int64_t *h_entry_seq, const double *h_entry_vec,
+                       int64_t n_exit, const int64_t *h_exit_seq, const double *h_exit_vec)
+{
+    if (!c) return fail(TEHMM_EINVAL, "ctx is NULL");
+    if (!c->has_model) return fail(TEHMM_ESTATE, "tehmm_set_model has not been called");
+    if (!c->has_batch) return fail(TEHMM_ESTATE, "tehmm_set_batch has not been called");
+    if (n_entry < 0 || n_exit < 0 || (n_entry > 0 && (!h_entry_seq || !h_entry_vec)) || (n_exit > 0 && (!h_exit_seq || !h_exit_vec)))
+        return fail(TEHMM_EINVAL, "bad argument");
+    CU(cudaSetDevice(c->device));
+    const int64_t nseq = c->b.nseq;
+    const int N = c->m.N, NP = c->m.NP;
+    const std::vector<int64_t> off(c->batch_key.begin(), c->batch_key.begin() + nseq + 1);
+    if (check_vectors("entry", n_entry, h_entry_seq, h_entry_vec, nseq, N, off)) return TEHMM_EINVAL;
+    if (check_vectors("exit", n_exit, h_exit_seq, h_exit_vec, nseq, N, off)) return TEHMM_EINVAL;
+    CU(cudaStreamSynchronize(c->stream));     // the passes queued so far read the vectors being replaced
+    c->n_entry = c->n_exit = 0;
+    c->b.cont = c->bf.cont = nullptr;
+    if (n_entry == 0 && n_exit == 0) return TEHMM_OK;
+    size_t o_cont = 0, o_es = align_up((size_t)nseq), o_ev = align_up(o_es + (size_t)n_entry * 8);
+    size_t o_xs = align_up(o_ev + (size_t)n_entry * NP * 8), o_xv = align_up(o_xs + (size_t)n_exit * 8);
+    size_t o_save = align_up(o_xv + (size_t)n_exit * NP * 8), bytes = align_up(o_save + (size_t)n_exit * 2 * c->m.LD * 8);
+    std::vector<unsigned char> h(bytes, 0);
+    for (int64_t k = 0; k < n_entry; ++k) {
+        h[o_cont + h_entry_seq[k]] = 1;
+        ((int64_t *)&h[o_es])[k] = h_entry_seq[k];
+        double sum = 0.0;                     // sum 1: the first chunk's log-likelihood is the increment
+        for (int j = 0; j < N; ++j) sum += h_entry_vec[k * N + j];
+        for (int j = 0; j < N; ++j) ((double *)&h[o_ev])[k * NP + j] = h_entry_vec[k * N + j] / sum;
+    }
+    for (int64_t k = 0; k < n_exit; ++k) {
+        ((int64_t *)&h[o_xs])[k] = h_exit_seq[k];
+        double mx = 0.0;                      // any scale: brought to a maximum of 1
+        for (int j = 0; j < N; ++j) mx = std::max(mx, h_exit_vec[k * N + j]);
+        for (int j = 0; j < N; ++j) ((double *)&h[o_xv])[k * NP + j] = h_exit_vec[k * N + j] / mx;
+    }
+    if (bytes > c->bnd_blob_bytes) {
+        if (c->bnd_blob) { cudaFree(c->bnd_blob); c->bnd_blob = nullptr; c->bnd_blob_bytes = 0; }
+        CU(cudaMalloc(&c->bnd_blob, bytes));
+        c->bnd_blob_bytes = bytes;
+    }
+    CU(cudaMemcpy(c->bnd_blob, h.data(), bytes, cudaMemcpyHostToDevice));
+    unsigned char *d = (unsigned char *)c->bnd_blob;
+    c->n_entry = n_entry;
+    c->n_exit = n_exit;
+    c->d_entry_seq = (const int64_t *)(d + o_es);
+    c->d_entry_vec = (const double *)(d + o_ev);
+    c->d_exit_seq = (const int64_t *)(d + o_xs);
+    c->d_exit_vec = (const double *)(d + o_xv);
+    c->d_exit_save = d + o_save;
+    if (n_entry > 0) c->b.cont = c->bf.cont = (const uint8_t *)(d + o_cont);
+    return TEHMM_OK;
+}
+
+int tehmm_forward_row(tehmm_ctx *c, int prec, const void *d_alpha, int64_t row, double *h_out)
+{
+    RUN_PROLOGUE();
+    if (!d_alpha || !h_out) return fail(TEHMM_EINVAL, "NULL argument");
+    if (row < 0 || row >= c->b.total) return fail(TEHMM_EINVAL, "row %lld outside the batch", (long long)row);
+    const int N = c->m.N, LD = c->m.LD;
+    const size_t ts = prec == TEHMM_F32 ? 4 : 8;
+    std::vector<unsigned char> raw((size_t)LD * ts);
+    CU(cudaMemcpyAsync(raw.data(), (const char *)d_alpha + (size_t)row * LD * ts, raw.size(), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    double sum = 0.0;
+    for (int j = 0; j < N; ++j) {
+        h_out[j] = prec == TEHMM_F32 ? (double)((const float *)raw.data())[j] : ((const double *)raw.data())[j];
+        sum += h_out[j];
+    }
+    if (!(sum > 0.0) || !std::isfinite(sum)) return fail(TEHMM_ESTATE, "forward row %lld sums to %g", (long long)row, sum);
+    for (int j = 0; j < N; ++j) h_out[j] /= sum;
+    return TEHMM_OK;
+}
+
+int tehmm_cut_pair(tehmm_ctx *c, int prec, const double *h_v, const void *d_post_row, double *d_trans, double *h_u)
+{
+    RUN_PROLOGUE();
+    if (!h_v || !d_post_row || !h_u) return fail(TEHMM_EINVAL, "NULL argument");
+    const int N = c->m.N;
+    DevBuf dv;
+    CU(dv.alloc((size_t)2 * N * 8));
+    CU(cudaMemcpyAsync(dv.p, h_v, (size_t)N * 8, cudaMemcpyHostToDevice, st));
+    CU(tehmm_launch_cut_pair(st, c->m, prec, dv.as<double>(), d_post_row, d_trans, dv.as<double>() + N));
+    c->launches += 1;
+    CU(cudaMemcpyAsync(h_u, dv.as<double>() + N, (size_t)N * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return TEHMM_OK;
+}
+
+int tehmm_convert_rows(tehmm_ctx *c, int prec, const void *d_in, int64_t rows, int renorm, double *d_out)
+{
+    RUN_PROLOGUE();
+    if (!d_in || !d_out || rows < 0) return fail(TEHMM_EINVAL, "bad argument");
+    if (rows == 0) return TEHMM_OK;
+    CU(tehmm_launch_convert_rows(st, prec, c->m.N, c->m.LD, d_in, rows, renorm, d_out, c->sms));
+    c->launches += 1;
     return TEHMM_OK;
 }
 

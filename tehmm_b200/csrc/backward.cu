@@ -368,7 +368,7 @@ __global__ void trans_reduce_kernel(TehmmModelDev m, TehmmBatchDev b, const T *_
     if (e < N) {
         double acc = 0.0;
         for (int64_t s = 0; s < b.nseq; ++s)
-            if (b.seq_off[s + 1] > b.seq_off[s]) acc += (double)gamma0[s * NP + e];
+            if (b.seq_off[s + 1] > b.seq_off[s] && tehmm_is_start(b, s)) acc += (double)gamma0[s * NP + e];
         start_trans[e] += acc;
     }
     if (e < N * N) {

@@ -72,7 +72,14 @@ struct TehmmBatchDev {
     const int64_t *seq_chunk0;   // [nseq+1] first chunk of each sequence
     const TehmmChunk *chunks;    // [nchunks]
     int warmup;
+    // [nseq] 1 where the sequence continues one that began before this batch (tehmm_set_boundary:
+    // its first row is not a start, so it adds nothing to the start counts), or NULL: none does
+    const uint8_t *cont;
 };
+__device__ __forceinline__ bool tehmm_is_start(const TehmmBatchDev &b, int64_t seq)
+{
+    return b.cont == nullptr || b.cont[seq] == 0;
+}
 
 __device__ __forceinline__ long tehmm_load_sym(const void *obs, int obs_bytes, int64_t idx)
 {

@@ -62,10 +62,11 @@ __global__ void ratio_diag_kernel(TehmmModelDev m, TehmmBatchDev b, const double
     for (int64_t c = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; c < b.nchunks; c += ((int64_t)gridDim.x * blockDim.x) >> 5) {
         const TehmmChunk ch = b.chunks[c];
         double acc[2] = {0.0, 0.0};
+        const int64_t s0 = tehmm_is_start(b, ch.seq) ? ch.s0 : -1;     // a continued sequence has a transition into its first row
         for (int64_t t4 = ch.t0; t4 < ch.t1; t4 += 4) {
             double r[4];                 // four rows in flight: the walk is latency bound
 #pragma unroll
-            for (int q = 0; q < 4; ++q) r[q] = t4 + q < ch.t1 && t4 + q != ch.s0 ? ratios[t4 + q] : 0.0;
+            for (int q = 0; q < 4; ++q) r[q] = t4 + q < ch.t1 && t4 + q != s0 ? ratios[t4 + q] : 0.0;
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 if (!(r[q] > 1.0)) continue;

@@ -372,7 +372,9 @@ fwd_tile_kernel(TehmmModelDev m, TehmmBatchDev b, const float *__restrict__ blin
                 const TehmmChunk ch = b.chunks[c];
                 const int64_t dist = ch.t0 - ch.s0;
                 pred[r] = dist > 0;
-                if (dist == 0) { ks[r] = W; first[r] = true; }
+                // mode 1 takes a sequence's first chunk only when the sequence continues one before the batch
+                // (tehmm_set_boundary): it starts from the entry vector in start_vec like any repaired chunk
+                if (dist == 0 && mode == 0) { ks[r] = W; first[r] = true; }
                 else if (mode == 1) ks[r] = W;                       // from the true vector at t0-1
                 else if (dist <= W) { ks[r] = W - (int)dist; first[r] = true; }
                 else ks[r] = 0;                                      // speculate from a flat vector
@@ -1021,7 +1023,7 @@ __global__ void xi_reduce_kernel(TehmmModelDev m, TehmmBatchDev b, const double 
     if (e < N) {
         double acc = 0.0;
         for (int64_t s = 0; s < b.nseq; ++s)
-            if (b.seq_off[s + 1] > b.seq_off[s]) acc += (double)gamma0[s * 32 + e];
+            if (b.seq_off[s + 1] > b.seq_off[s] && tehmm_is_start(b, s)) acc += (double)gamma0[s * 32 + e];
         start_trans[e] += acc;
     }
     if (e < N * N) {

@@ -101,6 +101,29 @@ class _ResultPool(object):
 _result_pool = _ResultPool()
 
 
+def plan_windows(total, bytes_per_step, budget_bytes, max_window_steps=None, fit_bytes_per_step=None,
+                 min_window_steps=4096):
+    """Cuts of the concatenated time axis [0, total) into windows of
+    cap = min(max_window_steps, budget_bytes // bytes_per_step) rows, the last one
+    shorter: int64 array [0, cap, 2 cap, ..., total].  None when the whole batch fits
+    (no cap given and total * fit_bytes_per_step <= budget_bytes, fit_bytes_per_step
+    being what the unwindowed path holds per step, bytes_per_step by default): the
+    unwindowed path.  MemoryError when the memory left would force windows shorter than
+    min_window_steps: a run of millions of tiny windows would crawl instead of failing."""
+    total = int(total)
+    fit = bytes_per_step if fit_bytes_per_step is None else fit_bytes_per_step
+    if max_window_steps is None and total * int(fit) <= int(budget_bytes):
+        return None
+    cap = int(budget_bytes) // max(1, int(bytes_per_step))
+    want = total if max_window_steps is None else max(1, int(max_window_steps))
+    if cap < min(want, int(min_window_steps)):
+        raise MemoryError("windowed forward-backward: %d bytes of device memory left hold %d steps of %d bytes, "
+                          "fewer than the %d-step minimum window" % (int(budget_bytes), max(0, cap),
+                                                                    int(bytes_per_step), int(min_window_steps)))
+    cap = max(1, min(cap, want))
+    return np.append(np.arange(0, total, cap, dtype=np.int64), np.int64(total))
+
+
 class Engine(object):
     """One per Context.  Holds nothing of the model between calls except what
     upload_model() put on the device."""
@@ -115,6 +138,7 @@ class Engine(object):
         self.N = self.K = self.S = None
         self.batch_token = None        # set by fit(): the resident batch is reused across EM iterations
         self.batch_ratios = None
+        self._fitted = 0               # bytes per call of the batch _plan last let run unwindowed (0: ask again)
 
     # ------------------------------------------------------------ plumbing
     def _bind_stream(self):
@@ -153,6 +177,7 @@ class Engine(object):
         torch = self.torch
         self._bind_stream()
         self.batch_token = None
+        self._fitted = 0
         arrays, dt, offsets, _ = self._host_arrays(obs_list)
         host = arrays[0] if len(arrays) == 1 else np.concatenate(arrays, axis=0)
         if dt == np.uint16:   # torch has no full uint16 support everywhere: move raw bytes
@@ -210,6 +235,7 @@ class Engine(object):
         Returns (logprob float64[nseq], score float64[nseq] (MAP only), [int64 states])."""
         self._bind_stream()
         self.batch_token = None
+        self._fitted = 0
         prec, _ = self._prec(precision)
         arrays, dt, offsets, ptrs = self._host_arrays(obs_list)
         keep, rptrs = self._host_ratios(ratios, offsets)
@@ -241,6 +267,7 @@ class Engine(object):
         (viterbi logprob[nseq], [viterbi states], map score[nseq], [map states], forward logprob[nseq])."""
         self._bind_stream()
         self.batch_token = None
+        self._fitted = 0
         prec, _ = self._prec(precision)
         arrays, dt, offsets, ptrs = self._host_arrays(obs_list)
         keep, rptrs = self._host_ratios(ratios, offsets)
@@ -270,6 +297,7 @@ class Engine(object):
         """Batch already resident on the device (bench / multi-call reuse)."""
         self._bind_stream()
         self.batch_token = None
+        self._fitted = 0
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         self._keep["obs"] = d_obs
         self._keep["offsets"] = offsets
@@ -499,10 +527,16 @@ class Engine(object):
         return logprob.cpu().numpy()
 
     def posteriors(self, ratios_em=None, ratios_dp=None, renorm_eps=True, want_map=False,
-                   want_post=True, precision=None):
-        """score_samples / _decode_map for the batch (basehmm.py:238-273,332-359)."""
+                   want_post=True, precision=None, max_window_steps=None):
+        """score_samples / _decode_map for the batch (basehmm.py:238-273,332-359).
+        Posteriors without MAP states run in time windows when their lattices do not fit in free
+        device memory, or when max_window_steps caps the window length (as in estep)."""
         prec, tdt = self._prec(precision)
         d_re, d_rd = self.upload_ratios(ratios_em), self.upload_ratios(ratios_dp)
+        assert max_window_steps is None or (want_post and not want_map), "windows serve posteriors without MAP states"
+        cuts = self._plan(prec, 3, 8 * self.N, max_window_steps) if want_post and not want_map else None
+        if cuts is not None:
+            return self._posteriors_windows(cuts, prec, tdt, d_re, d_rd, renorm_eps)
         _, blin, rowmax = self.run_emission(prec, tdt, d_re, False, True)
         d_rd = self.fold_ratios(prec, d_rd, blin, rowmax)
         flags = (_lib.BWD_POSTERIORS if want_post else 0) | (_lib.BWD_MAP if want_map else 0) | \
@@ -604,19 +638,28 @@ class Engine(object):
         return res
 
     def estep(self, ratios=None, want_start=True, want_trans=True, want_obs=True,
-              precision=None, device_result=False, seq_slots=None, stats_S=None):
+              precision=None, device_result=False, seq_slots=None, stats_S=None, max_window_steps=None):
         """One E-step over the batch (basehmm.py:507-522 + hmm.py:545-574).
         Returns the packed float64 device tensor
             [sum logprob | nseq | start N | trans N*N | obs K*N*S | per-sequence logprob]
         (ready for ONE all-reduce) or, by default, a dict of host arrays.
         seq_slots = (n_total, indices): where this batch's sequences sit in the
-        job-wide per-sequence tail (other ranks fill the other slots)."""
+        job-wide per-sequence tail (other ranks fill the other slots).
+        When the batch's lattices do not fit in free device memory -- or windows of at most
+        max_window_steps rows are asked for -- the time axis is cut into windows and each is
+        run exactly from the boundary vectors of its neighbours (DESIGN.md section 11)."""
         torch = self.torch
         prec, tdt = self._prec(precision)
         N, K = self.N, self.K
         S = self.stats_S = int(stats_S) if stats_S else self.S    # width of the caller's obsStats
         n_total, slots = seq_slots if seq_slots is not None else (self.nseq, list(range(self.nseq)))
         d_r = ratios if (ratios is None or torch.is_tensor(ratios)) else self.upload_ratios(ratios)
+        # the unwindowed path holds blin and alpha, and the posteriors when it needs them (as its flags below)
+        fit_lattices = 3 if want_obs or (d_r is not None and (want_start or want_trans)) else 2
+        cuts = self._plan(prec, fit_lattices, 0, max_window_steps)
+        if cuts is not None:
+            packed = self._estep_windows(cuts, prec, tdt, d_r, want_start or want_trans, want_obs, S, n_total, slots)
+            return packed if device_result else self.unpack_stats(packed.cpu().numpy())
         _, blin, rowmax = self.run_emission(prec, tdt, d_r, False, True)
         self.fold_ratios(prec, d_r, blin, rowmax)          # forward / backward below run without ratios
         base = 2 + N + N * N + K * N * S
@@ -646,6 +689,158 @@ class Engine(object):
         if device_result:
             return packed
         return self.unpack_stats(packed.cpu().numpy())
+
+    # ------------------------------------------------------------ time windows (DESIGN.md section 11)
+    def _plan(self, prec, fit_lattices, extra, max_window_steps):
+        """window cuts of the current batch, or None for the unwindowed path.  Bytes per step:
+        `fit_lattices` (total, LD) lattices for the unwindowed path, three for a window (its
+        posteriors feed the pair across the cut), rowmax and `extra` (a float64 posterior row on
+        its way to the host); the budget is the device's free memory plus what torch holds
+        unused, less a margin for the scratch, the model and the partition."""
+        torch = self.torch
+        ts = 4 if prec == _lib.F32 else 8
+        per_step = lambda lattices: lattices * self.LD * ts + 8 + extra
+        need = self.total * per_step(fit_lattices)
+        if max_window_steps is None and need <= self._fitted:
+            # a batch this size just ran unwindowed (an EM loop): the memory queries below cost ~0.1 ms each
+            return None
+        cached = torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        free, _ = torch.cuda.mem_get_info(self.device)
+        budget = max(0, int((free + cached) * 0.9) - (256 << 20))
+        cuts = plan_windows(self.total, per_step(3), budget, max_window_steps, fit_bytes_per_step=per_step(fit_lattices))
+        if cuts is None:
+            self._fitted = need
+        return cuts
+
+    def _set_window(self, w0, w1, entry, exit_vec):
+        """describe rows [w0, w1) of the resident batch to the library: the pieces of the sequences that
+        overlap it, with the entry vector (dict: cut -> vector) of a piece that continues a sequence and
+        the exit vector of one that goes on.  Returns (sequence index of each piece, piece offsets)."""
+        off = self._win_offsets
+        seqs = np.arange(np.searchsorted(off[1:], w0, side="right"), np.searchsorted(off[:-1], w1, side="left"))
+        lo, hi = np.maximum(off[seqs], w0), np.minimum(off[seqs + 1], w1)
+        seqs = seqs[hi > lo]
+        lo, hi = np.maximum(off[seqs], w0), np.minimum(off[seqs + 1], w1)
+        sub = np.concatenate([[0], np.cumsum(hi - lo)]).astype(np.int64)
+        d_obs = self._keep["obs"]
+        base = d_obs.data_ptr() + int(w0) * self.K * self.obs_bytes
+        _lib.check(self.lib.tehmm_set_batch(self.ctx.handle, ctypes.c_void_p(base), self.obs_bytes, len(seqs),
+                                            _lib.ptr(sub)))
+        self.total, self.nseq = int(w1 - w0), len(seqs)
+        self._keep["offsets"] = sub
+        ent = np.zeros(1, dtype=np.int64) if off[seqs[0]] < w0 else None
+        # (the forward sweep runs a window without the exit vector it does not need)
+        ext = np.array([len(seqs) - 1], dtype=np.int64) if off[seqs[-1] + 1] > w1 and exit_vec is not None else None
+        ev = np.ascontiguousarray(entry[w0], dtype=np.float64) if ent is not None else None
+        xv = np.ascontiguousarray(exit_vec, dtype=np.float64) if ext is not None else None
+        if ent is not None or ext is not None:
+            _lib.check(self.lib.tehmm_set_boundary(self.ctx.handle, 0 if ent is None else 1, _lib.ptr(ent), _lib.ptr(ev),
+                                                   0 if ext is None else 1, _lib.ptr(ext), _lib.ptr(xv)))
+        return seqs, sub
+
+    def _windows(self, cuts, prec, tdt, d_em, d_fold, body):
+        """Checkpointed forward-backward over the windows [cuts[w], cuts[w+1]).  Forward, left to right,
+        over the windows that end inside a sequence, keeping only the normalised forward vector at each
+        such cut; then right to left, body(w0, w1, pieces' sequences, blin, rowmax, the window's folded
+        ratios) per window, which runs forward (from the saved vector) and backward (ending on the vector
+        the window to its right handed back) and returns the window's raw posterior lattice.  Its first
+        row and the saved vector give the pair across the cut and the exit vector of the window to the
+        left (tehmm_cut_pair).  d_em: ratios of the emission, d_fold: ratios folded into blin."""
+        off = self._win_offsets = self._keep["offsets"]
+        total, nseq = self.total, self.nseq
+        inner = set(int(x) for x in cuts[1:-1] if not np.isin(x, off))      # cuts inside a sequence
+        entry = {}
+        try:
+            for w in range(len(cuts) - 2):
+                w0, w1 = int(cuts[w]), int(cuts[w + 1])
+                if w1 not in inner:
+                    continue
+                self._set_window(w0, w1, entry, None)
+                _, blin, rowmax = self.run_emission(prec, tdt, None if d_em is None else d_em[w0:w1], False, True)
+                self.fold_ratios(prec, None if d_fold is None else d_fold[w0:w1], blin, rowmax)
+                alpha, _ = self.ctx.optimistic(lambda: self.run_forward(prec, tdt, blin, rowmax, None))
+                v = np.empty(self.N, dtype=np.float64)
+                _lib.check(self.lib.tehmm_forward_row(self.ctx.handle, prec, self._p(alpha), w1 - w0 - 1, _lib.ptr(v)))
+                entry[w1] = v
+                del alpha, blin, rowmax
+            u = None
+            for w in range(len(cuts) - 2, -1, -1):
+                w0, w1 = int(cuts[w]), int(cuts[w + 1])
+                seqs, sub = self._set_window(w0, w1, entry, u)
+                dr = None if d_fold is None else d_fold[w0:w1]
+                _, blin, rowmax = self.run_emission(prec, tdt, None if d_em is None else d_em[w0:w1], False, True)
+                self.fold_ratios(prec, dr, blin, rowmax)
+                post = body(w0, w1, seqs, blin, rowmax, dr)
+                u = None
+                if w0 in inner:
+                    u = np.empty(self.N, dtype=np.float64)
+                    trans = self._win_trans
+                    _lib.check(self.lib.tehmm_cut_pair(self.ctx.handle, prec, _lib.ptr(entry[w0]), self._p(post),
+                                                       self._p(trans), _lib.ptr(u)))
+                del post, blin, rowmax
+        finally:
+            self._keep["offsets"] = off
+            self.total, self.nseq = total, nseq
+            _lib.check(self.lib.tehmm_set_batch(self.ctx.handle, self._p(self._keep["obs"]), self.obs_bytes,
+                                                len(off) - 1, _lib.ptr(off)))
+
+    def _estep_windows(self, cuts, prec, tdt, d_r, want_trans, want_obs, S, n_total, slots):
+        torch = self.torch
+        N, K = self.N, self.K
+        base = 2 + N + N * N + K * N * S
+        packed = torch.zeros(base + n_total, dtype=torch.float64, device=self.device)
+        lp = torch.zeros(self.nseq, dtype=torch.float64, device=self.device)
+        flags = _lib.BWD_POSTERIORS | (_lib.BWD_TRANS if want_trans else 0)   # row 0 of the posteriors feeds the cut pair
+        self._win_trans = packed[2 + N:2 + N + N * N] if want_trans else None
+
+        def body(w0, w1, seqs, blin, rowmax, dr):
+            def stages():
+                alpha, logprob = self.run_forward(prec, tdt, blin, rowmax, None)
+                part = torch.zeros(base, dtype=torch.float64, device=self.device)
+                post, _, _ = self.run_backward(prec, tdt, flags, blin, alpha, None,
+                                               start_trans=part[2:2 + N + N * N] if want_trans else None)
+                if dr is not None and want_trans:
+                    _lib.check(self.lib.tehmm_ratio_diag_counts(self.ctx.handle, prec, self._p(post), self._p(dr),
+                                                                self._p(part[2:2 + N + N * N]), self._p(self.scratch(prec))))
+                if want_obs:
+                    self.run_emission_stats(prec, post, dr, part[2 + N + N * N:base], S)
+                return part, logprob, post
+            part, logprob, post = self.ctx.optimistic(stages)
+            packed[2:base] += part[2:base]
+            lp.index_add_(0, torch.as_tensor(seqs, dtype=torch.int64, device=self.device), logprob)
+            return post
+
+        self._windows(cuts, prec, tdt, d_r, d_r, body)
+        self._win_trans = None
+        packed[0] = lp.sum()
+        packed[1] = float(self.nseq)
+        packed[base:].index_copy_(0, torch.as_tensor(slots, dtype=torch.int64, device=self.device), lp)
+        return packed
+
+    def _posteriors_windows(self, cuts, prec, tdt, d_re, d_rd, renorm_eps):
+        torch = self.torch
+        N = self.N
+        host = np.empty((self.total, N), dtype=np.float64)
+        lp = torch.zeros(self.nseq, dtype=torch.float64, device=self.device)
+        self._win_trans = None
+        # the cut needs the posteriors before renormalisation: the backward pass leaves them raw and the
+        # conversion to float64 applies TEHMM_BWD_RENORM_EPS exactly as the backward kernels do
+
+        def body(w0, w1, seqs, blin, rowmax, dr):
+            def stages():
+                alpha, logprob = self.run_forward(prec, tdt, blin, rowmax, None)
+                post, _, _ = self.run_backward(prec, tdt, _lib.BWD_POSTERIORS, blin, alpha, None)
+                return logprob, post
+            logprob, post = self.ctx.optimistic(stages)
+            lp.index_add_(0, torch.as_tensor(seqs, dtype=torch.int64, device=self.device), logprob)
+            out = self.empty((w1 - w0) * N, torch.float64)
+            _lib.check(self.lib.tehmm_convert_rows(self.ctx.handle, prec, self._p(post), w1 - w0,
+                                                   1 if renorm_eps else 0, self._p(out)))
+            host[w0:w1] = self.to_host(out).reshape(w1 - w0, N)
+            return post
+
+        self._windows(cuts, prec, tdt, d_re, d_rd, body)
+        return {"logprob": lp.cpu().numpy(), "post": self.split(host)}
 
     def unpack_stats(self, host):
         N, K, S = self.N, self.K, getattr(self, "stats_S", self.S)
