@@ -257,7 +257,10 @@ int tehmm_run_emission_stats(tehmm_ctx *ctx, int prec, const void *d_post,
  * d_lattice: workspace of tehmm_viterbi_workspace_bytes() for the delta lattice.
  * d_ratios_emission: the ratios the emission was computed with (only used by
  * the re-score); d_ratios_dp: the ratios the DP applies (basehmm.py:327 vs
- * hmm.py:674 use different ones).                                            */
+ * hmm.py:674 use different ones).  A batch that is one time window of longer
+ * sequences takes its entry delta rows and exit states from
+ * tehmm_set_viterbi_boundary (below); d_logprob is then not the path score of
+ * the pieces that have them.                                                  */
 int64_t tehmm_viterbi_workspace_bytes(tehmm_ctx *ctx, int prec);
 int tehmm_run_viterbi(tehmm_ctx *ctx, int prec, const void *d_elog, const double *d_rowmax,
                       const double *d_ratios_emission, const double *d_ratios_dp,
@@ -278,7 +281,12 @@ int tehmm_run_viterbi(tehmm_ctx *ctx, int prec, const void *d_elog, const double
  * No segment ratios (tehmm_decode_host_ratios below takes them).  The library owns everything in between: a grow-only
  * device arena, pinned staging rings and a thread pool (TEHMM_HOST_THREADS,
  * default min(16, cores)) that stages pageable input and widens the uint8
- * states that crossed PCIe.  Blocks until the outputs are complete.          */
+ * states that crossed PCIe.  Blocks until the outputs are complete.
+ * TEHMM_ENOMEM: the arena (the batch's lattices: three of (total, LD) in
+ * TEHMM_DECODE_BOTH mode) does not fit in device memory; nothing was written
+ * and no arena is kept.  Decode such a batch in time windows with the calls
+ * below (tehmm_set_viterbi_boundary, tehmm_set_boundary; Engine.decode_host
+ * does).                                                                       */
 #define TEHMM_DECODE_VITERBI 0
 #define TEHMM_DECODE_MAP 1
 #define TEHMM_DECODE_BOTH 2
@@ -448,7 +456,25 @@ int tehmm_convert_lattice(tehmm_ctx *ctx, int prec, const void *d_in, double *d_
  *   device, may be NULL) with u = gamma ./ (v A) (0 where v A is 0), and writes u to h_u[N]: the
  *   exit vector of the window to the left.  Synchronises the stream.
  * tehmm_convert_rows: a (rows, LD) lattice to (rows, N) float64 on the device; renorm = 1 applies
- *   the TEHMM_BWD_RENORM_EPS renormalisation to the stored posteriors as the backward pass does. */
+ *   the TEHMM_BWD_RENORM_EPS renormalisation to the stored posteriors as the backward pass does.
+ * tehmm_set_viterbi_boundary: the same two boundary conditions for tehmm_run_viterbi (host arrays,
+ *   copied; sequence indices increasing; n = 0: none; cleared by tehmm_set_batch and by a call with
+ *   n_entry = n_exit = 0; independent of tehmm_set_boundary).
+ *   entry (h_entry_delta[k*N ..], log space, any finite shift, -inf allowed but not all -inf, no NaN or
+ *     +inf): the Viterbi delta of the step before the sequence's first row -- a row of the delta
+ *     lattice as stored.  The first row is then an ordinary transition step from it (with the
+ *     from-state-0 segment-ratio term at the row's own DP ratio), not log_start.
+ *   exit (h_exit_state[k] in [0, N), h_exit_ratio[k] the DP ratio of the row after the cut: NULL or
+ *     < 0 = none, else finite and > 0): the traceback of the sequence's last row starts from
+ *     argmax_i (delta_last[i] + A'(i, s)), lowest i on ties, A' the traceback's transition term at
+ *     that ratio, instead of argmax_i delta_last[i]: the path then joins the one after the cut as
+ *     the traceback of the whole sequence would.
+ *   With Viterbi boundaries set, d_logprob of tehmm_run_viterbi is not a path score of the pieces
+ *   that have them (the DP's value and the re-score both count the continued first row as a
+ *   start); score the joined path with tehmm_path_score over the whole sequences instead.          */
+int tehmm_set_viterbi_boundary(tehmm_ctx *ctx, int64_t n_entry, const int64_t *h_entry_seq,
+                               const double *h_entry_delta, int64_t n_exit, const int64_t *h_exit_seq,
+                               const int32_t *h_exit_state, const double *h_exit_ratio);
 int tehmm_set_boundary(tehmm_ctx *ctx, int64_t n_entry, const int64_t *h_entry_seq, const double *h_entry_vec,
                        int64_t n_exit, const int64_t *h_exit_seq, const double *h_exit_vec);
 int tehmm_forward_row(tehmm_ctx *ctx, int prec, const void *d_alpha, int64_t row, double *h_out);

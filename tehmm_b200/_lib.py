@@ -89,6 +89,7 @@ SIGNATURES = {
     "tehmm_scores_to_bed": (_c_int, [_c_int, ctypes.c_char_p, _c_i64, _c_void, _c_i64, _c_void, _c_void, _c_i64]),
     "tehmm_convert_lattice": (_c_int, [_c_void, _c_int, _c_void, _c_void, _c_i64]),
     "tehmm_set_boundary": (_c_int, [_c_void, _c_i64, _c_void, _c_void, _c_i64, _c_void, _c_void]),
+    "tehmm_set_viterbi_boundary": (_c_int, [_c_void, _c_i64, _c_void, _c_void, _c_i64, _c_void, _c_void, _c_void]),
     "tehmm_forward_row": (_c_int, [_c_void, _c_int, _c_void, _c_i64, _c_void]),
     "tehmm_cut_pair": (_c_int, [_c_void, _c_int, _c_void, _c_void, _c_void, _c_void]),
     "tehmm_convert_rows": (_c_int, [_c_void, _c_int, _c_void, _c_i64, _c_int, _c_void]),

@@ -51,6 +51,7 @@ cudaError_t tehmm_launch_ratio_fold(cudaStream_t, const TehmmModelDev &, int64_t
 cudaError_t tehmm_launch_ratio_diag(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const double *, const void *, double *, double *, int);
 cudaError_t tehmm_launch_chain(cudaStream_t, const TehmmModelDev &, int, int, int, const int64_t *, const int64_t *, int64_t, const void *, const double *, const void *, void *);
 cudaError_t tehmm_launch_entry(cudaStream_t, const TehmmBatchDev &, int, int, int64_t, const int64_t *, const double *, void *, int *);
+cudaError_t tehmm_launch_vit_exit(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, const void *, int64_t, const int64_t *, const int32_t *, const double *, uint8_t *, uint8_t *, int *);
 cudaError_t tehmm_launch_exit(cudaStream_t, const TehmmModelDev &, const TehmmBatchDev &, int, int64_t, const int64_t *, const double *, void *, void *, void *, int);
 cudaError_t tehmm_launch_cut_pair(cudaStream_t, const TehmmModelDev &, int, const double *, const void *, double *, double *);
 cudaError_t tehmm_launch_convert_rows(cudaStream_t, int, int, int, const void *, int64_t, int, double *, int);
@@ -153,6 +154,14 @@ struct tehmm_ctx {
     const int64_t *d_entry_seq = nullptr, *d_exit_seq = nullptr;
     const double *d_entry_vec = nullptr, *d_exit_vec = nullptr;
     void *d_exit_save = nullptr;
+    // Viterbi boundary conditions (tehmm_set_viterbi_boundary; cleared by tehmm_set_batch):
+    // vbnd_blob = entry_seq[n_ventry] | entry_delta[n_ventry][NP] | exit_seq[n_vexit] | exit_state[n_vexit] | exit_ratio[n_vexit]
+    int64_t n_ventry = 0, n_vexit = 0;
+    void *vbnd_blob = nullptr;
+    size_t vbnd_blob_bytes = 0;
+    const int64_t *d_ventry_seq = nullptr, *d_vexit_seq = nullptr;
+    const double *d_ventry_vec = nullptr, *d_vexit_ratio = nullptr;
+    const int32_t *d_vexit_state = nullptr;
 };
 
 extern "C" {
@@ -198,6 +207,7 @@ int tehmm_ctx_destroy(tehmm_ctx *c)
     if (c->model_blob) cudaFree(c->model_blob);
     if (c->batch_blob) cudaFree(c->batch_blob);
     if (c->bnd_blob) cudaFree(c->bnd_blob);
+    if (c->vbnd_blob) cudaFree(c->vbnd_blob);
     if (c->d_seq_flag) cudaFree(c->d_seq_flag);
     if (c->h_nbad) cudaFreeHost(c->h_nbad);
     if (c->h_pending) cudaFreeHost(c->h_pending);
@@ -770,6 +780,7 @@ int tehmm_set_batch(tehmm_ctx *c, const void *d_obs, int obs_bytes, int64_t nseq
     const int64_t total = h_offsets[nseq];
     if (total <= 0) return fail(TEHMM_EINVAL, "empty batch");
     c->n_entry = c->n_exit = 0;               // a new batch starts without boundary vectors
+    c->n_ventry = c->n_vexit = 0;
     c->b.cont = c->bf.cont = nullptr;
     {   // the same batch shape at the same address again (a stream of decode calls): keep the partition
         std::vector<int64_t> key(h_offsets, h_offsets + nseq + 1);
@@ -1258,10 +1269,13 @@ static int repair_loop(tehmm_ctx *c, cudaStream_t st, const TehmmBatchDev &PB, i
     CU(launch(0));
     tk_end(c, timer[kind]);
     c->launches += 1;
-    if (kind == 0 && c->n_entry > 0) {
-        // continued sequences (tehmm_set_boundary): their first chunks are exact from the entry vectors, run
-        // like repaired chunks; the verification below then checks the chunks after them as usual
-        CU(tehmm_launch_entry(st, PB, prec, c->m.NP, c->n_entry, c->d_entry_seq, c->d_entry_vec, sv, bad));
+    const int64_t n_entry = kind == 0 ? c->n_entry : kind == 2 ? c->n_ventry : 0;
+    if (n_entry > 0) {
+        // continued sequences (tehmm_set_boundary / tehmm_set_viterbi_boundary): their first chunks are exact
+        // from the entry vectors, run like repaired chunks; the verification below then checks the chunks after
+        // them as usual (a first chunk is never flagged, so the exact fallback chains from its end vector)
+        CU(tehmm_launch_entry(st, PB, prec, c->m.NP, n_entry, kind == 0 ? c->d_entry_seq : c->d_ventry_seq,
+                              kind == 0 ? c->d_entry_vec : c->d_ventry_vec, sv, bad));
         CU(launch(1));
         c->launches += 2;
     }
@@ -1503,6 +1517,15 @@ int tehmm_run_viterbi(tehmm_ctx *c, int prec, const void *d_elog, const double *
     CU(tehmm_launch_traceback(st, c->m, TBP, prec, d_lattice, d_ratios_dp, d_states, d_states64, spec_end, pred, forced, bad, 0, tb_grid));
     tk_end(c, TK_TRACEBACK);
     c->launches += 1;
+    if (c->n_vexit > 0) {
+        // exit states (tehmm_set_viterbi_boundary): the last chunks of those sequences are walked again from
+        // the forced state of their last row before the verification, which then checks the chunks to their
+        // left against that walk; the exact fallback takes their end state as known (spec_end)
+        CU(tehmm_launch_vit_exit(st, c->m, TBP, prec, d_lattice, c->n_vexit, c->d_vexit_seq, c->d_vexit_state,
+                                 c->d_vexit_ratio, spec_end, forced, bad));
+        CU(tehmm_launch_traceback(st, c->m, TBP, prec, d_lattice, d_ratios_dp, d_states, d_states64, spec_end, pred, forced, bad, 1, tb_grid));
+        c->launches += 2;
+    }
     int64_t tb_reach = 8;
     for (int64_t pass = 0;; ++pass) {
         CU(tehmm_launch_tb_verify(st, TBP, spec_end, pred, forced, bad, nbad));
@@ -1547,13 +1570,21 @@ int tehmm_path_score(tehmm_ctx *c, const uint8_t *d_states, const double *d_rati
 }
 
 // ---------------------------------------------------------------- windows of longer sequences (window.cu)
-static int check_vectors(const char *what, int64_t n, const int64_t *seq, const double *vec, int64_t nseq, int N,
-                         const std::vector<int64_t> &off)
+static int check_seqs(const char *what, int64_t n, const int64_t *seq, int64_t nseq, const std::vector<int64_t> &off)
 {
     for (int64_t k = 0; k < n; ++k) {
         if (seq[k] < 0 || seq[k] >= nseq) return fail(TEHMM_EINVAL, "%s %lld: sequence %lld outside [0,%lld)", what, (long long)k, (long long)seq[k], (long long)nseq);
         if (k > 0 && seq[k] <= seq[k - 1]) return fail(TEHMM_EINVAL, "%s sequences must be increasing", what);
         if (off[seq[k] + 1] <= off[seq[k]]) return fail(TEHMM_EINVAL, "%s %lld: sequence %lld is empty", what, (long long)k, (long long)seq[k]);
+    }
+    return 0;
+}
+
+static int check_vectors(const char *what, int64_t n, const int64_t *seq, const double *vec, int64_t nseq, int N,
+                         const std::vector<int64_t> &off)
+{
+    if (check_seqs(what, n, seq, nseq, off)) return TEHMM_EINVAL;
+    for (int64_t k = 0; k < n; ++k) {
         double sum = 0.0;
         for (int j = 0; j < N; ++j) {
             const double x = vec[k * N + j];
@@ -1615,6 +1646,72 @@ int tehmm_set_boundary(tehmm_ctx *c, int64_t n_entry, const int64_t *h_entry_seq
     c->d_exit_vec = (const double *)(d + o_xv);
     c->d_exit_save = d + o_save;
     if (n_entry > 0) c->b.cont = c->bf.cont = (const uint8_t *)(d + o_cont);
+    return TEHMM_OK;
+}
+
+int tehmm_set_viterbi_boundary(tehmm_ctx *c, int64_t n_entry, const int64_t *h_entry_seq, const double *h_entry_delta,
+                               int64_t n_exit, const int64_t *h_exit_seq, const int32_t *h_exit_state,
+                               const double *h_exit_ratio)
+{
+    if (!c) return fail(TEHMM_EINVAL, "ctx is NULL");
+    if (!c->has_model) return fail(TEHMM_ESTATE, "tehmm_set_model has not been called");
+    if (!c->has_batch) return fail(TEHMM_ESTATE, "tehmm_set_batch has not been called");
+    if (n_entry < 0 || n_exit < 0 || (n_entry > 0 && (!h_entry_seq || !h_entry_delta)) ||
+        (n_exit > 0 && (!h_exit_seq || !h_exit_state)))
+        return fail(TEHMM_EINVAL, "bad argument");
+    CU(cudaSetDevice(c->device));
+    const int64_t nseq = c->b.nseq;
+    const int N = c->m.N, NP = c->m.NP;
+    const std::vector<int64_t> off(c->batch_key.begin(), c->batch_key.begin() + nseq + 1);
+    if (check_seqs("entry", n_entry, h_entry_seq, nseq, off) || check_seqs("exit", n_exit, h_exit_seq, nseq, off))
+        return TEHMM_EINVAL;
+    for (int64_t k = 0; k < n_entry; ++k) {
+        double mx = -INFINITY;
+        for (int j = 0; j < N; ++j) {
+            const double x = h_entry_delta[k * N + j];
+            if (std::isnan(x) || x == INFINITY) return fail(TEHMM_EINVAL, "entry %lld: component %d is %g (must be finite or -inf)", (long long)k, j, x);
+            mx = std::max(mx, x);
+        }
+        if (!(mx > -INFINITY)) return fail(TEHMM_EINVAL, "entry %lld: every component is -inf", (long long)k);
+    }
+    for (int64_t k = 0; k < n_exit; ++k) {
+        if (h_exit_state[k] < 0 || h_exit_state[k] >= N) return fail(TEHMM_EINVAL, "exit %lld: state %d outside [0,%d)", (long long)k, (int)h_exit_state[k], N);
+        const double r = h_exit_ratio ? h_exit_ratio[k] : -1.0;
+        if (r >= 0.0 && !(r > 0.0 && std::isfinite(r))) return fail(TEHMM_EINVAL, "exit %lld: ratio %g (must be finite and > 0, or < 0 for none)", (long long)k, r);
+        if (std::isnan(r)) return fail(TEHMM_EINVAL, "exit %lld: ratio is NaN", (long long)k);
+    }
+    CU(cudaStreamSynchronize(c->stream));     // the passes queued so far read the vectors being replaced
+    c->n_ventry = c->n_vexit = 0;
+    if (n_entry == 0 && n_exit == 0) return TEHMM_OK;
+    const size_t o_es = 0, o_ev = align_up(o_es + (size_t)n_entry * 8), o_xs = align_up(o_ev + (size_t)n_entry * NP * 8);
+    const size_t o_xst = align_up(o_xs + (size_t)n_exit * 8), o_xr = align_up(o_xst + (size_t)n_exit * 4);
+    const size_t bytes = align_up(o_xr + (size_t)n_exit * 8);
+    std::vector<unsigned char> h(bytes, 0);
+    for (int64_t k = 0; k < n_entry; ++k) {
+        ((int64_t *)&h[o_es])[k] = h_entry_seq[k];
+        double mx = -INFINITY;                // brought to a maximum of 0, as the DP keeps its rows; padding -inf
+        for (int j = 0; j < N; ++j) mx = std::max(mx, h_entry_delta[k * N + j]);
+        for (int j = 0; j < NP; ++j) ((double *)&h[o_ev])[k * NP + j] = j < N ? h_entry_delta[k * N + j] - mx : -INFINITY;
+    }
+    for (int64_t k = 0; k < n_exit; ++k) {
+        ((int64_t *)&h[o_xs])[k] = h_exit_seq[k];
+        ((int32_t *)&h[o_xst])[k] = h_exit_state[k];
+        ((double *)&h[o_xr])[k] = h_exit_ratio && h_exit_ratio[k] > 0.0 ? h_exit_ratio[k] : -1.0;
+    }
+    if (bytes > c->vbnd_blob_bytes) {
+        if (c->vbnd_blob) { cudaFree(c->vbnd_blob); c->vbnd_blob = nullptr; c->vbnd_blob_bytes = 0; }
+        CU(cudaMalloc(&c->vbnd_blob, bytes));
+        c->vbnd_blob_bytes = bytes;
+    }
+    CU(cudaMemcpy(c->vbnd_blob, h.data(), bytes, cudaMemcpyHostToDevice));
+    unsigned char *d = (unsigned char *)c->vbnd_blob;
+    c->n_ventry = n_entry;
+    c->n_vexit = n_exit;
+    c->d_ventry_seq = (const int64_t *)(d + o_es);
+    c->d_ventry_vec = (const double *)(d + o_ev);
+    c->d_vexit_seq = (const int64_t *)(d + o_xs);
+    c->d_vexit_state = (const int32_t *)(d + o_xst);
+    c->d_vexit_ratio = (const double *)(d + o_xr);
     return TEHMM_OK;
 }
 

@@ -320,7 +320,15 @@ struct Decode {
             HCU(cudaStreamSynchronize(st));
             if (p->arena) { cudaFree(p->arena); p->arena = nullptr; p->arena_bytes = 0; }
             const size_t want = need + need / 8;
-            HCU(cudaMalloc(&p->arena, want));
+            const cudaError_t e = cudaMalloc(&p->arena, want);
+            if (e == cudaErrorMemoryAllocation) {
+                // the batch's lattices do not fit: the caller can decode it in time windows (Engine.decode_host)
+                cudaGetLastError();
+                p->arena = nullptr;
+                return herr(TEHMM_ENOMEM, "the decode arena (%zu bytes for %lld steps) does not fit in device memory",
+                            want, (long long)total);
+            }
+            HCU(e);
             p->arena_bytes = want;
             return TEHMM_OK;
         };

@@ -10,6 +10,11 @@
 //     backward kernel changes and their hot loops stay as they are.
 //   the transition pair across a cut: (1/N) v_i A_ij u_j / sum(v A u), with u = gamma ./ (v A) from the
 //     first posterior row after the cut (cut_pair_kernel; also returns u, the left window's exit vector).
+//
+// Viterbi (tehmm_set_viterbi_boundary): the entry delta goes through entry_kernel and the DP's repair mode
+// like the forward entry vector; the exit state s of the row after the cut fixes the state of the last row,
+// argmax_i (delta_last[i] + A'(i, s)) -- one more step of the traceback walk, with its operands
+// (vit_exit_kernel) -- and the last chunk is walked again from it (forced end, as a repaired chunk).
 #include "scan.cuh"
 
 // start_vec[first chunk of seq[k]] = v[k] (lattice precision), bad[that chunk] = 1 (bad zeroed before)
@@ -118,6 +123,74 @@ __global__ void convert_rows_kernel(int N, int LD, const T *__restrict__ in, int
         if (renorm) gv = (T)(((double)gv + eps32) * renorm_inv);
         out[e] = (double)gv;
     }
+}
+
+// The traceback's step from state s at the row after the cut back to the last row, with the operands of
+// vit_traceback4_kernel (fp32: log A clamped to <= 0 in float, arg-max = smallest bit pattern, lowest state on
+// ties) and of vit_traceback_kernel's back() (float64: strict '>' from state 0 up).  r < 0: no segment ratio.
+__device__ int vit_exit_argmax(const TehmmModelDev &m, const float *d, int s, double rd)
+{
+    const int NP = m.NP;
+    const float r = (float)rd;
+    unsigned best = 0xffffffffu;
+    int arg = 0;
+    for (int i = 0; i < NP; ++i) {
+        float a = fminf((float)m.cut_trans[(int64_t)i * NP + s], 0.f);
+        if (i == 0 && r >= 0.f) {
+            const float dgs = fminf((float)m.cut_trans[(int64_t)s * NP + s], 0.f);
+            const float a00 = (float)m.cut_trans[0];
+            float extra0 = dgs > -INFINITY ? (r > 1.f ? dgs : dgs * r) : 0.f;
+            if (s == 0 && a00 > -INFINITY) extra0 -= a00;
+            a += extra0;
+        }
+        const unsigned bits = __float_as_uint(d[i] + a);
+        if (bits < best) { best = bits; arg = i; }
+    }
+    return arg;
+}
+__device__ int vit_exit_argmax(const TehmmModelDev &m, const double *d, int s, double r)
+{
+    const int NP = m.NP, N = m.N;
+    double best = -INFINITY;
+    int arg = 0;
+    for (int i = 0; i < NP; ++i) {
+        double cand = (i < N ? d[i] : -INFINITY) + m.cut_trans[(int64_t)i * NP + s];
+        if (i == 0 && r >= 0.0) {
+            const double dgs = m.cut_trans[(int64_t)s * NP + s], a00 = m.cut_trans[0];
+            const double common = r > 1.0 ? dgs * (r - 1.0) : 0.0;
+            double extra0 = dgs > -INFINITY ? dgs * r - common : 0.0;
+            if (s == 0 && a00 > -INFINITY) extra0 -= a00;
+            cand += extra0;
+        }
+        if (i == 0 || cand > best) { best = cand; arg = i; }
+    }
+    return arg;
+}
+
+// one thread per exit sequence: forced[last chunk] = spec_end[last chunk] = the state of its last row, bad = 1
+template <typename T>
+__global__ void vit_exit_kernel(TehmmModelDev m, TehmmBatchDev b, const T *__restrict__ lattice, int64_t n,
+                                const int64_t *__restrict__ seq, const int32_t *__restrict__ state,
+                                const double *__restrict__ ratio, uint8_t *__restrict__ spec_end,
+                                uint8_t *__restrict__ forced, int *__restrict__ bad)
+{
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const int64_t q = seq[k];
+    const int st = vit_exit_argmax(m, lattice + (b.seq_off[q + 1] - 1) * m.LD, state[k], ratio[k]);
+    const int64_t c = b.seq_chunk0[q + 1] - 1;
+    forced[c] = spec_end[c] = (uint8_t)st;
+    bad[c] = 1;
+}
+
+cudaError_t tehmm_launch_vit_exit(cudaStream_t st, const TehmmModelDev &m, const TehmmBatchDev &b, int prec,
+                                  const void *lattice, int64_t n, const int64_t *seq, const int32_t *state,
+                                  const double *ratio, uint8_t *spec_end, uint8_t *forced, int *bad)
+{
+    const int grid = (int)((n + 127) / 128);
+    if (prec == TEHMM_F32) vit_exit_kernel<float><<<grid, 128, 0, st>>>(m, b, (const float *)lattice, n, seq, state, ratio, spec_end, forced, bad);
+    else vit_exit_kernel<double><<<grid, 128, 0, st>>>(m, b, (const double *)lattice, n, seq, state, ratio, spec_end, forced, bad);
+    return cudaGetLastError();
 }
 
 cudaError_t tehmm_launch_entry(cudaStream_t st, const TehmmBatchDev &b, int prec, int NP, int64_t n,

@@ -226,13 +226,18 @@ class Engine(object):
                 "sequence %d: %d segment ratios for %d observations" % (i, r.shape[0], offsets[i + 1] - offsets[i])
         return keep, (ctypes.c_void_p * n)(*[None if r is None else r.ctypes.data for r in keep])
 
-    def decode_host(self, obs_list, algorithm, precision=None, ratios=None):
+    def decode_host(self, obs_list, algorithm, precision=None, ratios=None, max_window_steps=None):
         """The whole decode call with host buffers on both sides, in the library
         (tehmm_decode_host: pinned staging + worker threads in, uint8 states over PCIe and
         widened to the reference's int64 out).  ratios: None, or per sequence an array of
         segment ratios or None (tehmm_decode_host_ratios); the Viterbi DP takes them, the
         emission and MAP decoding do not, as in the reference's decode.
+        When the library's arena does not fit in device memory (TEHMM_ENOMEM), or windows of at
+        most max_window_steps rows are asked for, the batch is uploaded and decoded in time windows
+        (Engine.viterbi / Engine.posteriors, DESIGN.md section 11) with the same results.
         Returns (logprob float64[nseq], score float64[nseq] (MAP only), [int64 states])."""
+        if max_window_steps is not None:
+            return self._decode_windows(obs_list, (algorithm,), precision, ratios, max_window_steps)
         self._bind_stream()
         self.batch_token = None
         self._fitted = 0
@@ -245,13 +250,16 @@ class Engine(object):
         logprob = np.empty(n, dtype=np.float64)
         score = np.empty(n, dtype=np.float64)
         if rptrs is None:
-            _lib.check(self.lib.tehmm_decode_host(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets),
-                                                  int(algorithm), prec, _lib.ptr(states), _lib.ptr(logprob),
-                                                  _lib.ptr(score)))
+            rc = self.lib.tehmm_decode_host(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets),
+                                            int(algorithm), prec, _lib.ptr(states), _lib.ptr(logprob), _lib.ptr(score))
         else:
-            _lib.check(self.lib.tehmm_decode_host_ratios(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets),
-                                                         rptrs, int(algorithm), prec, _lib.ptr(states),
-                                                         _lib.ptr(logprob), _lib.ptr(score)))
+            rc = self.lib.tehmm_decode_host_ratios(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets),
+                                                   rptrs, int(algorithm), prec, _lib.ptr(states),
+                                                   _lib.ptr(logprob), _lib.ptr(score))
+        if rc == _lib.TEHMM_ENOMEM:
+            del keep, states
+            return self._decode_windows(obs_list, (algorithm,), precision, ratios, None)
+        _lib.check(rc)
         del keep
         self._keep.pop("obs", None)            # the batch now points into the library's arena
         self._keep["offsets"] = offsets
@@ -260,11 +268,16 @@ class Engine(object):
         self.d2h_bytes = int(self.lib.tehmm_decode_host_bytes(self.ctx.handle, 1))
         return logprob, score, [states[offsets[i]:offsets[i + 1]] for i in range(n)]
 
-    def decode_host_both(self, obs_list, precision=None, ratios=None):
+    def decode_host_both(self, obs_list, precision=None, ratios=None, max_window_steps=None):
         """Viterbi AND posterior (MAP) decoding of the same observations in one call
         (tehmm_decode_host_both): one upload, one emission pass.  ratios as for decode_host:
-        the Viterbi path takes them, the MAP path and the forward log-likelihood do not.  Returns
-        (viterbi logprob[nseq], [viterbi states], map score[nseq], [map states], forward logprob[nseq])."""
+        the Viterbi path takes them, the MAP path and the forward log-likelihood do not.  In time
+        windows as decode_host (TEHMM_ENOMEM or max_window_steps), the two decodings one after the
+        other.  Returns (viterbi logprob[nseq], [viterbi states], map score[nseq], [map states],
+        forward logprob[nseq])."""
+        if max_window_steps is not None:
+            return self._decode_windows(obs_list, (_lib.DECODE_VITERBI, _lib.DECODE_MAP), precision, ratios,
+                                        max_window_steps)
         self._bind_stream()
         self.batch_token = None
         self._fitted = 0
@@ -276,14 +289,17 @@ class Engine(object):
         vst, mst = _result_pool.empty_int64(total), _result_pool.empty_int64(total)
         vlp, msc, flp = (np.empty(n, dtype=np.float64) for _ in range(3))
         if rptrs is None:
-            _lib.check(self.lib.tehmm_decode_host_both(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets), prec,
-                                                       _lib.ptr(vst), _lib.ptr(vlp), _lib.ptr(mst), _lib.ptr(msc),
-                                                       _lib.ptr(flp)))
+            rc = self.lib.tehmm_decode_host_both(self.ctx.handle, ptrs, n, dt.itemsize, n, _lib.ptr(offsets), prec,
+                                                 _lib.ptr(vst), _lib.ptr(vlp), _lib.ptr(mst), _lib.ptr(msc),
+                                                 _lib.ptr(flp))
         else:
-            _lib.check(self.lib.tehmm_decode_host_both_ratios(self.ctx.handle, ptrs, n, dt.itemsize, n,
-                                                              _lib.ptr(offsets), rptrs, prec, _lib.ptr(vst),
-                                                              _lib.ptr(vlp), _lib.ptr(mst), _lib.ptr(msc),
-                                                              _lib.ptr(flp)))
+            rc = self.lib.tehmm_decode_host_both_ratios(self.ctx.handle, ptrs, n, dt.itemsize, n,
+                                                        _lib.ptr(offsets), rptrs, prec, _lib.ptr(vst),
+                                                        _lib.ptr(vlp), _lib.ptr(mst), _lib.ptr(msc), _lib.ptr(flp))
+        if rc == _lib.TEHMM_ENOMEM:
+            del keep, vst, mst
+            return self._decode_windows(obs_list, (_lib.DECODE_VITERBI, _lib.DECODE_MAP), precision, ratios, None)
+        _lib.check(rc)
         del keep
         self._keep.pop("obs", None)
         self._keep["offsets"] = offsets
@@ -292,6 +308,42 @@ class Engine(object):
         self.d2h_bytes = int(self.lib.tehmm_decode_host_bytes(self.ctx.handle, 1))
         cut = lambda st: [st[offsets[i]:offsets[i + 1]] for i in range(n)]
         return vlp, cut(vst), msc, cut(mst), flp
+
+    def _decode_windows(self, obs_list, algorithms, precision, ratios, max_window_steps):
+        """decode_host (one algorithm) / decode_host_both (Viterbi, then MAP) of a batch whose decode
+        arena does not fit: the observations resident on the device, each decoding in time windows
+        (max_window_steps None: as free memory allows).  Ratios as the host call takes them: a sequence
+        without ratios gets the plain Viterbi recursion (-1.0 on the device), and MAP ignores them."""
+        offsets = self.upload_batch(obs_list)
+        n = len(offsets) - 1
+        d_rd = None
+        if ratios is not None and any(r is not None for r in ratios):
+            self._host_ratios(ratios, offsets)                    # (checks the lengths)
+            host = np.full(self.total, -1.0)
+            for i, r in enumerate(ratios):
+                if r is not None:
+                    r = np.asarray(r, dtype=np.float64).reshape(-1)
+                    if not np.all(np.isfinite(r) & (r > 0)):
+                        raise AssertionError("sequence %d: segment ratios must be finite and > 0" % i)
+                    host[offsets[i]:offsets[i + 1]] = r
+            d_rd = self.torch.from_numpy(host).to(self.device)
+        out = []
+        d2h = 0
+        for alg in algorithms:
+            if alg == _lib.DECODE_VITERBI:
+                lp, st = self._viterbi(precision, None, d_rd, max_window_steps)
+                out.append((lp, np.full(n, np.nan), st))
+                d2h += self.total
+            else:
+                r = self.posteriors(renorm_eps=True, want_map=True, want_post=False, precision=precision,
+                                    max_window_steps=max_window_steps)
+                out.append((r["logprob"], r["map_score"], r["map_states"]))
+                d2h += self.total
+        self.d2h_bytes = d2h + 16 * n * len(algorithms)
+        if len(algorithms) == 1:
+            return out[0]
+        (vlp, _, vst), (flp, msc, mst) = out
+        return vlp, vst, msc, mst, flp
 
     def use_device_batch(self, d_obs, obs_bytes, offsets):
         """Batch already resident on the device (bench / multi-call reuse)."""
@@ -476,9 +528,11 @@ class Engine(object):
         _lib.check(self.lib.tehmm_run_emission_stats(self.ctx.handle, prec, self._p(post), self._p(d_ratios),
                                                      self._p(obs_stats), int(stats_S), self._p(sc)))
 
-    def run_viterbi(self, prec, elog, d_ratios_em, d_ratios_dp, want64=True, rowmax=None):
+    def run_viterbi(self, prec, elog, d_ratios_em, d_ratios_dp, want64=True, rowmax=None, lattice=None):
+        """lattice: the delta lattice workspace (tehmm_viterbi_workspace_bytes), when the caller reads it after"""
         torch = self.torch
-        bp = self.empty(int(self.lib.tehmm_viterbi_workspace_bytes(self.ctx.handle, prec)), torch.uint8)
+        bp = lattice if lattice is not None else \
+            self.empty(int(self.lib.tehmm_viterbi_workspace_bytes(self.ctx.handle, prec)), torch.uint8)
         states = self.empty(self.total, torch.uint8)
         states64 = self.empty(self.total, torch.int64) if want64 else None
         logprob = self.empty(self.nseq, torch.float64)
@@ -529,14 +583,15 @@ class Engine(object):
     def posteriors(self, ratios_em=None, ratios_dp=None, renorm_eps=True, want_map=False,
                    want_post=True, precision=None, max_window_steps=None):
         """score_samples / _decode_map for the batch (basehmm.py:238-273,332-359).
-        Posteriors without MAP states run in time windows when their lattices do not fit in free
+        Posteriors and MAP states run in time windows when their lattices do not fit in free
         device memory, or when max_window_steps caps the window length (as in estep)."""
         prec, tdt = self._prec(precision)
         d_re, d_rd = self.upload_ratios(ratios_em), self.upload_ratios(ratios_dp)
-        assert max_window_steps is None or (want_post and not want_map), "windows serve posteriors without MAP states"
-        cuts = self._plan(prec, 3, 8 * self.N, max_window_steps) if want_post and not want_map else None
+        # the unwindowed path holds blin, alpha and the posteriors it returns, the MAP states, the rows for the host
+        cuts = self._plan(prec, 3 if want_post else 2, (8 * self.N if want_post else 0) + (1 if want_map else 0),
+                          max_window_steps)
         if cuts is not None:
-            return self._posteriors_windows(cuts, prec, tdt, d_re, d_rd, renorm_eps)
+            return self._posteriors_windows(cuts, prec, tdt, d_re, d_rd, renorm_eps, want_post, want_map)
         _, blin, rowmax = self.run_emission(prec, tdt, d_re, False, True)
         d_rd = self.fold_ratios(prec, d_rd, blin, rowmax)
         flags = (_lib.BWD_POSTERIORS if want_post else 0) | (_lib.BWD_MAP if want_map else 0) | \
@@ -554,10 +609,18 @@ class Engine(object):
             out["map_score"] = mscore.cpu().numpy()
         return out
 
-    def viterbi(self, ratios_em=None, ratios_dp=None, precision=None):
-        """decode(algorithm='viterbi') for the batch (basehmm.py:301-330, hmm.py:668-676)."""
+    def viterbi(self, ratios_em=None, ratios_dp=None, precision=None, max_window_steps=None):
+        """decode(algorithm='viterbi') for the batch (basehmm.py:301-330, hmm.py:668-676).
+        In time windows when the emission and delta lattices do not fit in free device memory, or
+        when max_window_steps caps the window length (DESIGN.md section 11)."""
+        return self._viterbi(precision, self.upload_ratios(ratios_em), self.upload_ratios(ratios_dp), max_window_steps)
+
+    def _viterbi(self, precision, d_re, d_rd, max_window_steps):
         prec, tdt = self._prec(precision)
-        d_re, d_rd = self.upload_ratios(ratios_em), self.upload_ratios(ratios_dp)
+        # the unwindowed path holds elog, the delta lattice and the uint8 states
+        cuts = self._plan(prec, 2, 1, max_window_steps, win_lattices=2)
+        if cuts is not None:
+            return self._viterbi_windows(cuts, prec, tdt, d_re, d_rd)
         elog, _, rowmax = self.run_emission(prec, tdt, d_re, True, False)
         states, _, logprob = self.ctx.optimistic(
             lambda: self.run_viterbi(prec, elog, d_re, d_rd, want64=False, rowmax=rowmax))
@@ -691,11 +754,12 @@ class Engine(object):
         return self.unpack_stats(packed.cpu().numpy())
 
     # ------------------------------------------------------------ time windows (DESIGN.md section 11)
-    def _plan(self, prec, fit_lattices, extra, max_window_steps):
+    def _plan(self, prec, fit_lattices, extra, max_window_steps, win_lattices=3):
         """window cuts of the current batch, or None for the unwindowed path.  Bytes per step:
-        `fit_lattices` (total, LD) lattices for the unwindowed path, three for a window (its
-        posteriors feed the pair across the cut), rowmax and `extra` (a float64 posterior row on
-        its way to the host); the budget is the device's free memory plus what torch holds
+        `fit_lattices` (total, LD) lattices for the unwindowed path, `win_lattices` for a window
+        (three for forward-backward: its posteriors feed the pair across the cut; two for Viterbi:
+        emission and delta), rowmax and `extra` (a float64 posterior row on its way to the host,
+        the uint8 states); the budget is the device's free memory plus what torch holds
         unused, less a margin for the scratch, the model and the partition."""
         torch = self.torch
         ts = 4 if prec == _lib.F32 else 8
@@ -707,15 +771,18 @@ class Engine(object):
         cached = torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
         free, _ = torch.cuda.mem_get_info(self.device)
         budget = max(0, int((free + cached) * 0.9) - (256 << 20))
-        cuts = plan_windows(self.total, per_step(3), budget, max_window_steps, fit_bytes_per_step=per_step(fit_lattices))
+        cuts = plan_windows(self.total, per_step(win_lattices), budget, max_window_steps,
+                            fit_bytes_per_step=per_step(fit_lattices))
         if cuts is None:
             self._fitted = need
         return cuts
 
-    def _set_window(self, w0, w1, entry, exit_vec):
+    def _set_window(self, w0, w1, entry, exit_vec, viterbi=False):
         """describe rows [w0, w1) of the resident batch to the library: the pieces of the sequences that
         overlap it, with the entry vector (dict: cut -> vector) of a piece that continues a sequence and
-        the exit vector of one that goes on.  Returns (sequence index of each piece, piece offsets)."""
+        the exit vector of one that goes on.  viterbi: the Viterbi DP's boundary instead
+        (tehmm_set_viterbi_boundary): entry[cut] the delta row before the cut, exit_vec = (state of
+        the row after the cut, its DP ratio or -1).  Returns (sequence index of each piece, piece offsets)."""
         off = self._win_offsets
         seqs = np.arange(np.searchsorted(off[1:], w0, side="right"), np.searchsorted(off[:-1], w1, side="left"))
         lo, hi = np.maximum(off[seqs], w0), np.minimum(off[seqs + 1], w1)
@@ -732,6 +799,14 @@ class Engine(object):
         # (the forward sweep runs a window without the exit vector it does not need)
         ext = np.array([len(seqs) - 1], dtype=np.int64) if off[seqs[-1] + 1] > w1 and exit_vec is not None else None
         ev = np.ascontiguousarray(entry[w0], dtype=np.float64) if ent is not None else None
+        if viterbi:
+            xs = np.array([exit_vec[0]], dtype=np.int32) if ext is not None else None
+            xr = np.array([exit_vec[1]], dtype=np.float64) if ext is not None else None
+            if ent is not None or ext is not None:
+                _lib.check(self.lib.tehmm_set_viterbi_boundary(self.ctx.handle, 0 if ent is None else 1, _lib.ptr(ent),
+                                                               _lib.ptr(ev), 0 if ext is None else 1, _lib.ptr(ext),
+                                                               _lib.ptr(xs), _lib.ptr(xr)))
+            return seqs, sub
         xv = np.ascontiguousarray(exit_vec, dtype=np.float64) if ext is not None else None
         if ent is not None or ext is not None:
             _lib.check(self.lib.tehmm_set_boundary(self.ctx.handle, 0 if ent is None else 1, _lib.ptr(ent), _lib.ptr(ev),
@@ -779,10 +854,61 @@ class Engine(object):
                                                        self._p(trans), _lib.ptr(u)))
                 del post, blin, rowmax
         finally:
-            self._keep["offsets"] = off
-            self.total, self.nseq = total, nseq
-            _lib.check(self.lib.tehmm_set_batch(self.ctx.handle, self._p(self._keep["obs"]), self.obs_bytes,
-                                                len(off) - 1, _lib.ptr(off)))
+            self._whole_batch(off, total, nseq)
+
+    def _whole_batch(self, off, total, nseq):
+        """the resident batch described to the library again after its windows"""
+        self._keep["offsets"] = off
+        self.total, self.nseq = total, nseq
+        _lib.check(self.lib.tehmm_set_batch(self.ctx.handle, self._p(self._keep["obs"]), self.obs_bytes,
+                                            len(off) - 1, _lib.ptr(off)))
+
+    def _viterbi_windows(self, cuts, prec, tdt, d_re, d_rd):
+        """Viterbi over the windows [cuts[w], cuts[w+1]) (DESIGN.md section 11).  Left to right over the
+        windows that end inside a sequence: emission and DP from the delta row handed on by the window to
+        the left, keeping only the delta row before each such cut.  Then right to left: emission, DP
+        from that row and traceback from the state the window to the right chose at the cut, into the
+        batch's uint8 states.  The joined paths are scored once over the whole batch."""
+        torch = self.torch
+        off = self._win_offsets = self._keep["offsets"]
+        total, nseq = self.total, self.nseq
+        inner = set(int(x) for x in cuts[1:-1] if not np.isin(x, off))      # cuts inside a sequence
+        states = self.empty(total, torch.uint8)
+        entry = {}
+
+        def window(w0, w1, exit_state):
+            self._set_window(w0, w1, entry, exit_state, viterbi=True)
+            dre = None if d_re is None else d_re[w0:w1]
+            drd = None if d_rd is None else d_rd[w0:w1]
+            elog, _, rowmax = self.run_emission(prec, tdt, dre, True, False)
+            lattice = self.empty(int(self.lib.tehmm_viterbi_workspace_bytes(self.ctx.handle, prec)), torch.uint8)
+            st, _, _ = self.ctx.optimistic(
+                lambda: self.run_viterbi(prec, elog, dre, drd, want64=False, rowmax=rowmax, lattice=lattice))
+            return st, lattice
+
+        try:
+            for w in range(len(cuts) - 2):
+                w0, w1 = int(cuts[w]), int(cuts[w + 1])
+                if w1 not in inner:
+                    continue
+                _, lattice = window(w0, w1, None)
+                entry[w1] = lattice.view(tdt)[(w1 - w0 - 1) * self.LD:(w1 - w0 - 1) * self.LD + self.N].double().cpu().numpy()
+                del lattice
+            nxt = None
+            for w in range(len(cuts) - 2, -1, -1):
+                w0, w1 = int(cuts[w]), int(cuts[w + 1])
+                st, lattice = window(w0, w1, nxt if w1 in inner else None)
+                del lattice
+                states[w0:w1].copy_(st)
+                nxt = None
+                if w0 in inner:
+                    nxt = (int(st[0].item()), float(d_rd[w0].item()) if d_rd is not None else -1.0)
+        finally:
+            self._whole_batch(off, total, nseq)
+        logprob = self.empty(nseq, torch.float64)
+        _lib.check(self.lib.tehmm_path_score(self.ctx.handle, self._p(states), self._p(d_re), self._p(d_rd), 0, total,
+                                             self._p(logprob), self._p(self.scratch(prec))))
+        return logprob.cpu().numpy(), self.split(self.states_to_host(states))
 
     def _estep_windows(self, cuts, prec, tdt, d_r, want_trans, want_obs, S, n_total, slots):
         torch = self.torch
@@ -817,30 +943,49 @@ class Engine(object):
         packed[base:].index_copy_(0, torch.as_tensor(slots, dtype=torch.int64, device=self.device), lp)
         return packed
 
-    def _posteriors_windows(self, cuts, prec, tdt, d_re, d_rd, renorm_eps):
+    def _posteriors_windows(self, cuts, prec, tdt, d_re, d_rd, renorm_eps, want_post=True, want_map=False):
         torch = self.torch
         N = self.N
-        host = np.empty((self.total, N), dtype=np.float64)
+        host = np.empty((self.total, N), dtype=np.float64) if want_post else None
+        mstates = self.empty(self.total, torch.uint8) if want_map else None
         lp = torch.zeros(self.nseq, dtype=torch.float64, device=self.device)
+        msc = torch.zeros(self.nseq, dtype=torch.float64, device=self.device)
         self._win_trans = None
         # the cut needs the posteriors before renormalisation: the backward pass leaves them raw and the
-        # conversion to float64 applies TEHMM_BWD_RENORM_EPS exactly as the backward kernels do
+        # conversion to float64 applies TEHMM_BWD_RENORM_EPS exactly as the backward kernels do.  The MAP
+        # arg-max is over the raw values in every kernel, and the renormalised MAP score is affine in the
+        # raw one: sum_t (best_t + eps32) / (1 + N eps32), applied below to the whole sequence.
+        flags = _lib.BWD_POSTERIORS | (_lib.BWD_MAP if want_map else 0)
 
         def body(w0, w1, seqs, blin, rowmax, dr):
             def stages():
                 alpha, logprob = self.run_forward(prec, tdt, blin, rowmax, None)
-                post, _, _ = self.run_backward(prec, tdt, _lib.BWD_POSTERIORS, blin, alpha, None)
-                return logprob, post
-            logprob, post = self.ctx.optimistic(stages)
-            lp.index_add_(0, torch.as_tensor(seqs, dtype=torch.int64, device=self.device), logprob)
-            out = self.empty((w1 - w0) * N, torch.float64)
-            _lib.check(self.lib.tehmm_convert_rows(self.ctx.handle, prec, self._p(post), w1 - w0,
-                                                   1 if renorm_eps else 0, self._p(out)))
-            host[w0:w1] = self.to_host(out).reshape(w1 - w0, N)
+                return (logprob,) + self.run_backward(prec, tdt, flags, blin, alpha, None)
+            logprob, post, ms, sc = self.ctx.optimistic(stages)
+            idx = torch.as_tensor(seqs, dtype=torch.int64, device=self.device)
+            lp.index_add_(0, idx, logprob)
+            if want_map:
+                msc.index_add_(0, idx, sc)
+                mstates[w0:w1].copy_(ms)
+            if want_post:
+                out = self.empty((w1 - w0) * N, torch.float64)
+                _lib.check(self.lib.tehmm_convert_rows(self.ctx.handle, prec, self._p(post), w1 - w0,
+                                                       1 if renorm_eps else 0, self._p(out)))
+                host[w0:w1] = self.to_host(out).reshape(w1 - w0, N)
             return post
 
         self._windows(cuts, prec, tdt, d_re, d_rd, body)
-        return {"logprob": lp.cpu().numpy(), "post": self.split(host)}
+        out = {"logprob": lp.cpu().numpy()}
+        if want_post:
+            out["post"] = self.split(host)
+        if want_map:
+            score = msc.cpu().numpy()
+            if renorm_eps:
+                eps32 = 1.1920928955078125e-07
+                score = (score + np.diff(self._keep["offsets"]) * eps32) * (1.0 / (1.0 + N * eps32))
+            out["map_score"] = score
+            out["map_states"] = self.split(self.states_to_host(mstates))
+        return out
 
     def unpack_stats(self, host):
         N, K, S = self.N, self.K, getattr(self, "stats_S", self.S)
